@@ -12,6 +12,7 @@ measures the loop; `--steps 1000` times complete volumes.  Sampling shards the b
 ranks with no communication (scaling = "weak": per-GPU batch fixed).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+                  [--dump-outputs DIR]
   torchrun ... bench.py --gpus N ...            (one rank per GPU; rank 0 prints ONE JSON line)
 
 --impl reference times the reference's own algorithm for the same path on the host CPU cores
@@ -531,7 +532,9 @@ def run_ours(args, rank, world, local_rank):
             sampler.start()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(K):
+        for i in range(K):
+            if i and i % T_STEPS == 0:   # the trajectory reached t = 0: the next volume starts at T - 1
+                prog.t_in.fill_(T_STEPS - 1)
             graph.replay()
         e1.record()
         torch.cuda.synchronize(dev)
@@ -539,6 +542,7 @@ def run_ours(args, rank, world, local_rank):
         barrier()
         clocks = sampler.stop() if rank == 0 else None
         finite = bool(torch.isfinite(prog.x_in).all().item())
+        x_last = prog.x_in.cpu() if args.dump_outputs and rank == 0 else None   # x_{t-1} of step K
 
         # ---- end to end through the public API with host buffers, every step ---------------
         # Every step's input comes from pinned host memory and every step's result goes back to
@@ -736,7 +740,26 @@ def run_ours(args, rank, world, local_rank):
         line["gpu_comparator"] = comparator
     if train is not None:
         line["train"] = train
+    if x_last is not None:
+        dump_outputs(args.dump_outputs, {"x_prev": x_last})
     print(json.dumps(line), flush=True)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays) -> None:
+    """--dump-outputs: every array as <out_dir>/<name>.npy in float32, for comparing two builds
+    output for output.  Over DUMP_LIMIT_BYTES in all, only the leading samples (dim 0) that fit
+    are written."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.numel() for a in arrays.values()) * 4
+    for name, a in arrays.items():
+        a = a.detach().float()
+        if total > DUMP_LIMIT_BYTES:
+            a = a[:max(1, a.shape[0] * DUMP_LIMIT_BYTES // total)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 def run_train(args, rank, world, local_rank):
@@ -883,7 +906,15 @@ def main():
     ap.add_argument("--torch-ddp", action="store_true", help="train mode, N > 1: torch DDP instead of the "
                     "overlapped bucketed all-reduce (parallel.DistributedDataParallel)")
     ap.add_argument("--per-op", default="", help="write per-GEMM timings (CUDA events) to this file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="sample mode: after the timed steps write rank 0's x_{t-1} of the last timed "
+                         "step as DIR/x_prev.npy (float32, [batch, 3, 40, 48, 40]; inputs are seeded, "
+                         "so two builds can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.mode != "sample" or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the sampling workload (--mode sample --impl ours)")
 
     if args.batch <= 0:
         args.batch = {"sample": 16, "train": 8, "vae": 1}[args.mode]

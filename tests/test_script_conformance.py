@@ -1,9 +1,9 @@
-"""Static drop-in check against the reference's OWN driver scripts (build container only: needs
-/root/reference; skipped on the GPU box).  The scripts cannot be executed here (they import mlflow,
-perun, nibabel and build datasets at import time -- SURVEY.md 8c), so their source is parsed
-instead: every name they import from the hot-path modules must exist in the overlay package, and
-every constructor / method call they make on those classes must bind to the drop-in's signature
-with the same positional and keyword arguments.  (Executing the scripts needs a GPU next to the
+"""Static drop-in check against the reference's OWN driver scripts (the checks that parse them need
+a reference checkout named by MRI_REFERENCE_DIR and skip without one).  The scripts cannot be
+executed here (they import mlflow, perun, nibabel and build datasets at import time -- SURVEY.md
+8c), so their source is parsed instead: every name they import from the hot-path modules must
+exist in the overlay package, and every constructor / method call they make on those classes
+must bind to the drop-in's signature with the same positional and keyword arguments.  (Executing the scripts needs a GPU next to the
 reference: tools/run_reference_scripts.py / tests/test_gpu_scripts.py, logs under profiles/r04*.)"""
 import ast
 import contextlib
@@ -14,8 +14,8 @@ import os
 
 import pytest
 
-REF = "/root/reference/model_scripts"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="/root/reference only exists in the build container")
+REF = os.path.join(os.environ.get("MRI_REFERENCE_DIR") or "/nonexistent", "model_scripts")
+needs_reference = pytest.mark.skipif(not os.path.isdir(REF), reason="needs a reference checkout (MRI_REFERENCE_DIR)")
 
 HOT_MODULES = {"unet", "unet_attention", "diffusion", "vae"}
 SCRIPTS = {
@@ -51,6 +51,7 @@ def bind_ok(fn, n_pos, kw_names, drop_self=True):
         return False
 
 
+@needs_reference
 @pytest.mark.parametrize("pkg", sorted(SCRIPTS))
 def test_imports_and_calls_of_reference_scripts_bind_to_the_drop_in(pkg):
     checked_imports = checked_ctor = checked_methods = 0
@@ -123,6 +124,7 @@ def test_attributes_read_by_the_scripts_exist():
     assert u3.in_channels == 3 and list(u3.chs) == [16, 32]
 
 
+@needs_reference
 def test_ddp_calls_of_the_training_script_bind_to_the_overlapped_wrapper():
     """ddpm_3d_ldm/train.py wraps the UNet as `DDP(unet, device_ids=[local_rank],
     output_device=local_rank, find_unused_parameters=False)` and later unwraps `.module`: every such
