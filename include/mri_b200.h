@@ -282,6 +282,19 @@ int mri_ddpm_step(const float* x, const void* eps, int eps_nhwc_ldc, int channel
 int mri_ddim_step(const float* x, const void* eps, int eps_nhwc_ldc, int channels,
                   const int64_t* t, const int64_t* t_prev, const float* alphas_cumprod, float* out,
                   int samples, int64_t per_sample, void* stream);
+/* mri_dpmpp_step: one DPM-Solver++(2M) step (not in the reference).  coef: device fp32 [rows][5]
+ * table of (s, r, A, B, C) rows (schedules.dpmpp_2m_table); k: device int64 row index (nullptr:
+ * row 0).  With that row, per element:
+ *     x0 = (x - s*eps)*r ;  out = (A*x + B*x0) + C*(x0 - x0_prev) ;  x0_prev = x0
+ * fp32, that association, no FMA contraction; the C term is not evaluated when C == 0, so
+ * x0_prev is not read on a first-order row (it may hold NaN there).  x0_prev is fp32 in x's
+ * layout; eps as for mri_ddim_step (ldc >= channels).  x and out may alias. */
+int mri_dpmpp_step(const float* x, const void* eps, int eps_nhwc_ldc, int channels,
+                   float* x0_prev, const float* coef, const int64_t* k, float* out, int samples,
+                   int64_t per_sample, void* stream);
+/* mri_step_table_advance: k[0] += 1, then t[b] = ts[min(k[0], rows - 1)] for b < n, in one
+ * launch (race-free for any n) -- the bookkeeping between two replays of a DPM-Solver++ step. */
+int mri_step_table_advance(int64_t* t, int n, int64_t* k, const int64_t* ts, int rows, void* stream);
 int mri_minsnr_loss(const float* pred, const float* noise, const int64_t* t, const float* snr,
                     float gamma, float* per_sample_out, float* loss_out, int samples,
                     int64_t per_sample, void* stream);
@@ -313,14 +326,17 @@ int mri_rng_seed(uint64_t* rng, uint64_t seed, uint64_t offset, void* stream);
  * Y[q + off(tap)][tap * cout + co], rounded to bf16 exactly as mri_tap_gather stores it, and
  *   mode 0: x <- DDPM update with z drawn in the kernel (ATen mapping over the whole state tensor),
  *   mode 1: x <- DDIM update (t_prev, alphas_cumprod),
- *   mode 2: eps only (eps_out bf16 [positions][ldo] required; otherwise optional).
+ *   mode 2: eps only (eps_out bf16 [positions][ldo] required; otherwise optional),
+ *   mode 3: x <- DPM-Solver++(2M) update of mri_dpmpp_step (x0_prev, coef, k; bf16-rounded eps).
  * x is the fp32 NC[D]HW sampler state [samples][cout][D][H][W], updated in place; 3^ndim taps,
- * ndim 2 (D = 1) or 3, cout 1..4.  The predicted noise never goes to HBM in modes 0 / 1. */
+ * ndim 2 (D = 1) or 3, cout 1..4.  The predicted noise never goes to HBM in modes 0 / 1 / 3.
+ * Arguments a mode does not use may be null. */
 int mri_tap_gather_step(const void* y, const float* bias, int samples, int D, int H, int W, int ndim,
                         int cout, int ldy, float* x, void* eps_out, int ldo, int mode,
                         const uint64_t* rng, const int64_t* t, const int64_t* t_prev,
                         const float* betas, const float* sqrt_1mac, const float* sqrt_recip_alphas,
-                        const float* post_var, const float* alphas_cumprod, void* stream);
+                        const float* post_var, const float* alphas_cumprod, float* x0_prev,
+                        const float* coef, const int64_t* k, void* stream);
 int mri_randn_offset_increment(int64_t numel, uint64_t* increment_out);
 int mri_randn(float* out, int64_t numel, const uint64_t* rng, void* stream);
 int mri_q_sample_rng(const float* x0, const uint64_t* rng, const int64_t* t, const float* sqrt_ac,

@@ -145,6 +145,8 @@ SIGNATURES = {
     "mri_q_sample": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _vp]),
     "mri_ddpm_step": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _vp]),
     "mri_ddim_step": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _i, _i64, _vp]),
+    "mri_dpmpp_step": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _i, _i64, _vp]),
+    "mri_step_table_advance": (_i, [_vp, _i, _vp, _vp, _i, _vp]),
     "mri_minsnr_loss": (_i, [_vp, _vp, _vp, _vp, _f, _vp, _vp, _i, _i64, _vp]),
     "mri_add_i64": (_i, [_vp, _i, _i64, _vp]),
     "mri_randn_offset_increment": (_i, [_i64, C.POINTER(C.c_uint64)]),
@@ -154,7 +156,7 @@ SIGNATURES = {
     "mri_ddpm_step_rng": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _vp]),
     "mri_step_advance": (_i, [_vp, _vp, _i, _i64, _vp, _u64, _vp]),
     "mri_tap_gather_step": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp, _vp,
-                                 _vp, _vp, _vp, _vp, _vp, _vp]),
+                                 _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mri_wgrad_launch": (_i, [C.POINTER(MriWgradArgs), _vp]),
     "mri_gn_bwd_reduce": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _i, _i, _i, _f, _i, _vp]),
     "mri_gn_bwd_apply": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _i, _i, _i, _f,

@@ -312,13 +312,90 @@ ddim_step_kernel(const float* x, const void* eps, int ldc, int channels, const i
       one);
 }
 
+// One DPM-Solver++(2M) step with coefficient row (s, r, A, B, C) (schedules.dpmpp_2m_table):
+//   x0 = (x - s*eps)*r ; out = (A*x + B*x0) + C*(x0 - x0_prev) ; x0_prev <- x0
+// The C term is skipped when C == 0, so x0_prev is never read on a first-order row (it may hold
+// anything there, NaN included).
+struct DpmRow {
+  float s, r, A, B, C;
+};
+__device__ __forceinline__ DpmRow dpm_row(const float* coef, const int64_t* k) {
+  const float* c = coef + 5 * (k != nullptr ? *k : 0);
+  return DpmRow{c[0], c[1], c[2], c[3], c[4]};
+}
+__device__ __forceinline__ float dpm_update(const DpmRow& c, float x, float e, float x0p, float& x0) {
+  x0 = __fmul_rn(__fsub_rn(x, __fmul_rn(c.s, e)), c.r);
+  const float o = __fadd_rn(__fmul_rn(c.A, x), __fmul_rn(c.B, x0));
+  return c.C != 0.f ? __fadd_rn(o, __fmul_rn(c.C, __fsub_rn(x0, x0p))) : o;
+}
+
+// x / out may alias; x0_prev is the solver's [samples][per_sample] fp32 state
+__global__ void __launch_bounds__(256)
+dpmpp_step_kernel(const float* x, const void* eps, int ldc, int channels, float* x0_prev,
+                  const float* coef, const int64_t* k, float* out, long long per_sample,
+                  long long numel, long long Tt, int n_iter) {
+  const long long spatial = per_sample / (channels > 0 ? channels : 1);
+  const DpmRow c = dpm_row(coef, k);
+  const bool second = c.C != 0.f;
+  const bool al = aligned16(x) && aligned16(out) && aligned16(x0_prev);
+  const bool eps_al = ldc == 0 && aligned16(eps);
+  auto one = [&](long long e, float) {
+    const long long n = e / per_sample;
+    const float ev = load_eps(eps, ldc, spatial, per_sample, n, e - n * per_sample);
+    float x0;
+    out[e] = dpm_update(c, x[e], ev, second ? x0_prev[e] : 0.f, x0);
+    x0_prev[e] = x0;
+  };
+  element_loop<false>(numel, Tt, n_iter, nullptr, nullptr,
+      [&](long long e0, const float (&)[4]) {
+        const long long n = e0 / per_sample;
+        const long long j = e0 - n * per_sample;
+        const bool same = (j + 3 < per_sample) && (ldc == 0 || (j % spatial) + 3 < spatial);
+        if (!same) {
+#pragma unroll
+          for (int m = 0; m < 4; ++m) one(e0 + m, 0.f);
+          return;
+        }
+        float xv[4], ev[4], pv[4] = {0.f, 0.f, 0.f, 0.f}, o[4], x0[4];
+        load4(x + e0, al, xv);
+        if (second) load4(x0_prev + e0, al, pv);
+        if (ldc == 0) {
+          load4(reinterpret_cast<const float*>(eps) + e0, eps_al, ev);
+        } else {
+          const long long ch = j / spatial;
+          const long long s = j - ch * spatial;
+          const __nv_bfloat16* ep =
+              reinterpret_cast<const __nv_bfloat16*>(eps) + (n * spatial + s) * ldc + ch;
+#pragma unroll
+          for (int m = 0; m < 4; ++m) ev[m] = __bfloat162float(ep[(long long)m * ldc]);
+        }
+#pragma unroll
+        for (int m = 0; m < 4; ++m) o[m] = dpm_update(c, xv[m], ev[m], pv[m], x0[m]);
+        store4(out + e0, al, o);
+        store4(x0_prev + e0, al, x0);
+      },
+      one);
+}
+
+// k += 1, then t[b] = ts[min(k, rows - 1)] for b < n.  One block: every thread reads the old k
+// before thread 0 writes the new one, for any n.
+__global__ void __launch_bounds__(256)
+step_table_advance_kernel(int64_t* t, int n, int64_t* k, const int64_t* ts, int rows) {
+  const int64_t kn = *k + 1;
+  __syncthreads();
+  if (threadIdx.x == 0) *k = kn;
+  const int64_t v = ts[kn < rows ? kn : rows - 1];
+  for (int b = threadIdx.x; b < n; b += blockDim.x) t[b] = v;
+}
+
 // ------------------------------------------------------------------------------------------
 // Thin output convolution finished INSIDE the reverse step.  The k^d convolution with 1..4 output
 // channels (out_conv) is computed as one GEMM over all taps, Y[q][tap * cout + co] = W[tap][co] . a[q]
 // (the activation is read once); this kernel sums the shifted taps -- eps[q][co] = bias[co] +
 // sum_tap Y[q + off(tap)][tap][co], in the same order and with the same bf16 rounding of the result
-// as mri_tap_gather -- and applies the DDPM (noise drawn in-kernel, ATen mapping) or DDIM update to
-// the fp32 NC[D]HW sampler state in place, so the predicted noise never goes to HBM.
+// as mri_tap_gather -- and applies the DDPM (noise drawn in-kernel, ATen mapping), DDIM or
+// DPM-Solver++(2M) update to the fp32 NC[D]HW sampler state in place, so the predicted noise never
+// goes to HBM.
 // One CTA = a tile of (TD x TH x TW) output positions; the Y rows of the tile plus a one-voxel halo
 // are staged in shared memory (odd word pitch: conflict-free), one thread per output position.
 // ------------------------------------------------------------------------------------------
@@ -331,7 +408,10 @@ struct FusedStepArgs {
   const int64_t* t;
   const int64_t* t_prev;    // DDIM
   const float *betas, *sqrt_1mac, *sqrt_recip_alphas, *post_var, *alphas_cumprod;
-  int samples, D, H, W, ndim, cout, ldy, ldo, mode;  // mode 0: DDPM, 1: DDIM, 2: eps only
+  float* x0_prev;           // DPM-Solver++: solver state, coefficient table, device row index
+  const float* coef;
+  const int64_t* k;
+  int samples, D, H, W, ndim, cout, ldy, ldo, mode;  // 0: DDPM, 1: DDIM, 2: eps only, 3: DPM-Solver++
   int TD, TH, TW, pitch_w;  // tile and shared-memory row pitch in 32-bit words
   long long Tt;             // ATen launch geometry of a randn over the whole state
 };
@@ -475,6 +555,11 @@ tap_gather_step_kernel(const FusedStepArgs a) {
       const float2 bm = (ii < 2) ? box_muller(rr.x, rr.y) : box_muller(rr.z, rr.w);
       const float z = (ii & 1) ? bm.y : bm.x;
       a.x[idx] = __fadd_rn(__fmul_rn(c1, __fsub_rn(xv, __fmul_rn(q_c, e))), __fmul_rn(wn, z));
+    } else if (a.mode == 3) {
+      const DpmRow c = dpm_row(a.coef, a.k);
+      float x0;
+      a.x[idx] = dpm_update(c, xv, e, c.C != 0.f ? a.x0_prev[idx] : 0.f, x0);
+      a.x0_prev[idx] = x0;
     } else {
       const float x0 = __fdiv_rn(__fsub_rn(xv, __fmul_rn(s1m_t, e)), denom);
       a.x[idx] = __fadd_rn(__fmul_rn(sqrt_a_p, x0), __fmul_rn(s1m_p, e));
@@ -680,6 +765,32 @@ extern "C" int mri_ddim_step(const float* x, const void* eps, int eps_nhwc_ldc, 
   return check_launch("ddim_step_kernel");
 }
 
+extern "C" int mri_dpmpp_step(const float* x, const void* eps, int eps_nhwc_ldc, int channels,
+                              float* x0_prev, const float* coef, const int64_t* k, float* out,
+                              int samples, int64_t per_sample, void* stream) {
+  if (samples < 1 || per_sample < 1) return set_error(-2, "mri_dpmpp_step: empty input");
+  if (x == nullptr || eps == nullptr || x0_prev == nullptr || coef == nullptr || out == nullptr)
+    return set_error(-2, "mri_dpmpp_step: null x / eps / x0_prev / coef / out");
+  if (eps_nhwc_ldc != 0 && (channels < 1 || per_sample % channels != 0 || eps_nhwc_ldc < channels))
+    return set_error(-2, "mri_dpmpp_step: per_sample must be channels * spatial, ldc >= channels");
+  const long long numel = (long long)samples * per_sample;
+  int rc = device_props();
+  if (rc) return rc;
+  const AtenGrid g = aten_grid(numel);
+  dpmpp_step_kernel<<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
+      x, eps, eps_nhwc_ldc, channels, x0_prev, coef, k, out, per_sample, numel, g.Tt, g.n_iter);
+  return check_launch("dpmpp_step_kernel");
+}
+
+extern "C" int mri_step_table_advance(int64_t* t, int n, int64_t* k, const int64_t* ts, int rows,
+                                      void* stream) {
+  if (n < 1) return 0;
+  if (t == nullptr || k == nullptr || ts == nullptr || rows < 1)
+    return set_error(-2, "mri_step_table_advance: null t / k / ts or rows < 1");
+  step_table_advance_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(t, n, k, ts, rows);
+  return check_launch("step_table_advance_kernel");
+}
+
 extern "C" int mri_rng_seed(uint64_t* rng, uint64_t seed, uint64_t offset, void* stream) {
   if (rng == nullptr) return set_error(-2, "mri_rng_seed: null state");
   if (offset % 4 != 0) return set_error(-2, "mri_rng_seed: philox offset must be a multiple of 4");
@@ -721,14 +832,18 @@ extern "C" int mri_tap_gather_step(const void* y, const float* bias, int samples
                                    int mode, const uint64_t* rng, const int64_t* t,
                                    const int64_t* t_prev, const float* betas, const float* sqrt_1mac,
                                    const float* sqrt_recip_alphas, const float* post_var,
-                                   const float* alphas_cumprod, void* stream) {
+                                   const float* alphas_cumprod, float* x0_prev, const float* coef,
+                                   const int64_t* k, void* stream) {
   if (ndim != 2 && ndim != 3) return set_error(-2, "mri_tap_gather_step: ndim must be 2 or 3");
   if (cout < 1 || cout > 4) return set_error(-2, "mri_tap_gather_step: 1..4 output channels");
   const int taps = ndim == 3 ? 27 : 9;
   if (ldy % 2 != 0 || taps * cout > ldy) return set_error(-2, "mri_tap_gather_step: bad Y row layout");
   if (samples < 1 || D < 1 || H < 1 || W < 1) return set_error(-2, "mri_tap_gather_step: empty input");
   if (ndim == 2 && D != 1) return set_error(-2, "mri_tap_gather_step: 2-D problems have D = 1");
-  if (mode < 0 || mode > 2) return set_error(-2, "mri_tap_gather_step: mode 0 (DDPM) / 1 (DDIM) / 2 (eps only)");
+  if (mode < 0 || mode > 3)
+    return set_error(-2, "mri_tap_gather_step: mode 0 (DDPM) / 1 (DDIM) / 2 (eps only) / 3 (DPM-Solver++)");
+  if (mode == 3 && (x0_prev == nullptr || coef == nullptr || x == nullptr))
+    return set_error(-2, "mri_tap_gather_step: DPM-Solver++ mode needs x, x0_prev and coef");
   if (mode == 0 && (rng == nullptr || t == nullptr || betas == nullptr || sqrt_1mac == nullptr ||
                     sqrt_recip_alphas == nullptr || post_var == nullptr || x == nullptr))
     return set_error(-2, "mri_tap_gather_step: DDPM mode needs x, rng, t and the four schedule tables");
@@ -751,6 +866,9 @@ extern "C" int mri_tap_gather_step(const void* y, const float* bias, int samples
   a.sqrt_recip_alphas = sqrt_recip_alphas;
   a.post_var = post_var;
   a.alphas_cumprod = alphas_cumprod;
+  a.x0_prev = x0_prev;
+  a.coef = coef;
+  a.k = k;
   a.samples = samples; a.D = D; a.H = H; a.W = W; a.ndim = ndim; a.cout = cout; a.ldy = ldy; a.ldo = ldo;
   a.mode = mode;
   a.TD = ndim == 3 ? 4 : 1;

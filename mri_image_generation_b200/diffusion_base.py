@@ -4,6 +4,7 @@ The three public classes (model_scripts/*/diffusion.py) differ only in schedule,
 model arguments (z_pos, context) and the loss; everything that touches the GPU is here:
   - q_sample / p_sample / DDIM arithmetic: one fused fp32 kernel each (mri_q_sample,
     mri_ddpm_step, mri_ddim_step), bit-exact w.r.t. the reference's eager association order;
+    DPM-Solver++(2M) (not in the reference): mri_dpmpp_step over a host-built coefficient table;
   - the reverse loop: when the denoiser is one of this package's UNets, one CUDA graph holds a
     whole reverse step (time embedding, UNet, fused update with the noise drawn INSIDE the
     kernel, t -= 1) and is replayed T times.  The kernels draw Philox4x32-10 + Box-Muller
@@ -21,7 +22,7 @@ from typing import Callable, Dict, Optional, Tuple
 import torch
 import torch.nn as nn
 
-from . import _lib, ops
+from . import _lib, ops, schedules
 from .modules import EngineModule
 
 
@@ -153,6 +154,48 @@ class DiffusionBase(nn.Module):
                                  t.to(pred.device).long().contiguous(),
                                  snr if snr is not None else self.betas, float(gamma))
 
+    # ------------------------------------------------------------------ DPM-Solver++(2M)
+    def _dpmpp_table(self, start_t, num_steps) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(ts, coef) of schedules.dpmpp_2m_table for num_steps UNet calls from start_t to sigma = 0."""
+        T, s, M = self.timesteps, int(start_t), int(num_steps)
+        if not 1 <= M <= s <= T - 1:
+            raise ValueError(f"DPM-Solver++ needs 1 <= num_steps <= start_t <= {T - 1} "
+                             f"(got num_steps={M}, start_t={s})")
+        return schedules.dpmpp_2m_table(self.alphas_cumprod, schedules.dpmpp_timesteps(s, M))
+
+    def _sample_dpmpp(self, img, table, prog, eps_fn: Callable) -> torch.Tensor:
+        """Run the solver over `table` from x = img.  prog: a UNetProgram whose conditioning inputs
+        the caller has set (replayed step graph), or None: eager, eps = eps_fn(x, t) per step.
+        Returns the fp32 x0 estimate."""
+        _require_cuda(img, "sample_dpmpp")
+        ts, coef = table
+        if prog is not None:
+            return self._reverse_loop(prog, img.float(), int(ts[0]), ts.numel(), "dpmpp", table=table)
+        dev = img.device
+        with torch.cuda.device(dev):
+            coef = coef.to(dev)
+            x = img.float().contiguous().clone()
+            x0_prev = torch.empty_like(x)
+            for i, t in enumerate(ts.tolist()):
+                tt = torch.full((x.shape[0],), t, device=dev, dtype=torch.long)
+                eps = eps_fn(x, tt)
+                ops.dpmpp_step(x, eps.float().contiguous(), x0_prev, coef[i], None, x)
+        return x
+
+    def _dpmpp_buffers(self, prog, rows: int) -> Dict[str, torch.Tensor]:
+        """The program's solver state: table (>= T rows, so that one captured graph serves every
+        num_steps and start_t), row index k and x0_prev."""
+        bufs = prog.__dict__.get("_dpmpp_bufs")
+        if bufs is None or bufs["ts"].numel() < rows:
+            dev, n = prog.x_in.device, max(rows, self.timesteps)
+            bufs = dict(coef=torch.zeros(n, 5, dtype=torch.float32, device=dev),
+                        ts=torch.zeros(n, dtype=torch.int64, device=dev),
+                        k=torch.zeros(1, dtype=torch.int64, device=dev),
+                        x0_prev=torch.zeros_like(prog.x_in))
+            prog.__dict__["_dpmpp_bufs"] = bufs
+            prog.__dict__.get("_step_graphs", {}).pop("dpmpp", None)  # captured on the old buffers
+        return bufs
+
     # ------------------------------------------------------------------ graph-replayed loops
     def _engine_model(self) -> Optional[EngineModule]:
         m = self.model
@@ -206,14 +249,17 @@ class DiffusionBase(nn.Module):
 
     def _reverse_loop(self, prog, img: torch.Tensor, start_t: int, n_steps: int, mode: str,
                       use_graph: bool = True, t_vec: Optional[torch.Tensor] = None,
-                      stride: int = 1) -> torch.Tensor:
+                      stride: int = 1, table=None) -> torch.Tensor:
         """Run n_steps reverse steps (i = start_t, start_t - stride, ...) on `prog` (a UNetProgram
-        whose x_in is the sampler state).  mode: 'ddpm' | 'ddim' (t_prev = max(t - stride, 0))."""
+        whose x_in is the sampler state).  mode: 'ddpm' | 'ddim' (t_prev = max(t - stride, 0)) |
+        'dpmpp' (table = (ts, coef) of schedules.dpmpp_2m_table, n_steps = its rows)."""
         dev = img.device
         with torch.cuda.device(dev):
-            return self._reverse_loop_on(prog, img, start_t, n_steps, mode, use_graph, t_vec, stride)
+            return self._reverse_loop_on(prog, img, start_t, n_steps, mode, use_graph, t_vec, stride,
+                                         table)
 
-    def _reverse_loop_on(self, prog, img, start_t, n_steps, mode, use_graph, t_vec, stride):
+    def _reverse_loop_on(self, prog, img, start_t, n_steps, mode, use_graph, t_vec, stride,
+                         table=None):
         dev = img.device
         if prog.params_changed():
             prog.do_refresh()
@@ -230,6 +276,12 @@ class DiffusionBase(nn.Module):
 
         fused = (getattr(prog, "fused_head", None) is not None and not prog.training
                  and os.environ.get("MRI_FUSED_STEP", "1") != "0")
+        if mode == "dpmpp":
+            # the graph reads its row of the table through the device index k: it bakes in no
+            # timestep, so changing num_steps or start_t only rewrites the table
+            dpm = self._dpmpp_buffers(prog, n_steps)
+            kbuf, xp, rows = dpm["k"], dpm["x0_prev"], dpm["ts"].numel()
+            kbuf.zero_()   # a valid row for the warm-up launch of a capture
 
         def one_step():
             if fused:  # out_conv's tap sum + the update in one kernel: eps never goes to HBM
@@ -239,6 +291,9 @@ class DiffusionBase(nn.Module):
                                         sqrt_recip_alphas=self.sqrt_recip_alphas,
                                         post_var=self.posterior_variance)
                     ops.step_advance(prog.t_in, -1, rng=rng, rng_increment=inc)
+                elif mode == "dpmpp":
+                    prog.run_fused_step(3, x0_prev=xp, coef=dpm["coef"], k=kbuf)
+                    ops.step_table_advance(prog.t_in, kbuf, dpm["ts"], rows)
                 else:
                     prog.run_fused_step(1, t=prog.t_in, t_prev=tprev, alphas_cumprod=self.alphas_cumprod)
                     ops.step_advance(prog.t_in, -stride, t_prev=tprev)
@@ -249,6 +304,10 @@ class DiffusionBase(nn.Module):
                                   self.sqrt_one_minus_alphas_cumprod, self.sqrt_recip_alphas,
                                   self.posterior_variance, prog.x_in, eps_nhwc_ldc=ldc, channels=C)
                 ops.step_advance(prog.t_in, -1, rng=rng, rng_increment=inc)
+            elif mode == "dpmpp":
+                ops.dpmpp_step(prog.x_in, prog.eps_nhwc, xp, dpm["coef"], kbuf, prog.x_in,
+                               eps_nhwc_ldc=ldc, channels=C)
+                ops.step_table_advance(prog.t_in, kbuf, dpm["ts"], rows)
             else:
                 ops.ddim_step(prog.x_in, prog.eps_nhwc, prog.t_in, tprev, self.alphas_cumprod,
                               prog.x_in, eps_nhwc_ldc=ldc, channels=C)
@@ -263,6 +322,13 @@ class DiffusionBase(nn.Module):
         else:
             prog.t_in.fill_(start_t)
         tprev.fill_(max(start_t - stride, 0))
+        if mode == "dpmpp":   # undo the warm-up launches of a capture and load this call's table
+            ts, coef = table
+            M = ts.numel()
+            dpm["coef"][:M].copy_(coef)
+            dpm["ts"][:M].copy_(ts)
+            dpm["ts"][M:].fill_(int(ts[-1]))
+            kbuf.zero_()
         off = rng.load() if mode == "ddpm" else 0
         for _ in range(n_steps):
             if graph is not None:

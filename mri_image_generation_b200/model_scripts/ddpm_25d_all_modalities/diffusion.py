@@ -57,3 +57,26 @@ class GaussianDiffusion(_GD2):
         return self.p_sample_loop(
             (batch_size, self.channels, self.image_size, self.image_size), z_pos=z_pos,
             context=context)
+
+    @torch.no_grad()
+    def sample_dpmpp(self, batch_size=16, z_pos=0.5, context=None, num_steps=20):
+        """Few-step sampler (not in the reference): x_T drawn as sample() draws it, then
+        DPM-Solver++(2M) with `num_steps` UNet calls from t = T - 1 to sigma = 0 (returns x0)."""
+        table = self._dpmpp_table(self.timesteps - 1, num_steps)
+        device = self.betas.device
+        shape = (batch_size, self.channels, self.image_size, self.image_size)
+        img = self._randn(shape, device)
+        z_pos = self._z_tensor(z_pos, batch_size, device)
+        if context is not None:
+            context = context.to(device)
+        eng = self._engine_model()
+        prog = None
+        if eng is not None:
+            _require_cuda(img, "sample_dpmpp")
+            cc = 0 if context is None else context.shape[1]
+            prog = eng.program(batch_size, shape[2:], shape[1], cc)
+            prog.z_in.copy_(z_pos.reshape(-1, 1))
+            if context is not None:
+                prog.ctx_in.copy_(context)
+        return self._sample_dpmpp(img, table, prog,
+                                  lambda x, t: self.model(x, t, z_pos, context=context))

@@ -86,3 +86,20 @@ class GaussianDiffusion(DiffusionBase):
         """diffusion.py:157-166."""
         return self.p_sample_loop(
             (batch_size, self.channels, self.image_size, self.image_size), z_pos=z_pos)
+
+    @torch.no_grad()
+    def sample_dpmpp(self, batch_size=16, z_pos=0.5, num_steps=20):
+        """Few-step sampler (not in the reference): x_T drawn as sample() draws it, then
+        DPM-Solver++(2M) with `num_steps` UNet calls from t = T - 1 to sigma = 0 (returns x0)."""
+        table = self._dpmpp_table(self.timesteps - 1, num_steps)
+        device = self.betas.device
+        shape = (batch_size, self.channels, self.image_size, self.image_size)
+        img = self._randn(shape, device)
+        z_pos = self._z_tensor(z_pos, batch_size, device)
+        eng = self._engine_model()
+        prog = None
+        if eng is not None:
+            _require_cuda(img, "sample_dpmpp")
+            prog = eng.program(batch_size, shape[2:], shape[1], 0)
+            prog.z_in.copy_(z_pos.reshape(-1, 1))
+        return self._sample_dpmpp(img, table, prog, lambda x, t: self.model(x, t, z_pos))

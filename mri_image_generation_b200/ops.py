@@ -139,6 +139,26 @@ def ddim_step(x, eps, t, t_prev, alphas_cumprod, out, eps_nhwc_ldc: int = 0,
                "mri_ddim_step")
 
 
+def dpmpp_step(x, eps, x0_prev, coef, k, out, eps_nhwc_ldc: int = 0, channels: int = 0) -> None:
+    """One DPM-Solver++(2M) step with row k (device int64 tensor, or None for row 0) of the fp32
+    [rows][5] table of schedules.dpmpp_2m_table; x0_prev (x's shape, fp32) is read on
+    second-order rows and overwritten with this step's x0.  x and out may alias."""
+    _chk_contig(x, eps, x0_prev, coef, out)
+    assert x0_prev.dtype == coef.dtype == torch.float32 and x0_prev.numel() == x.numel()
+    assert k is None or k.dtype == torch.int64
+    n = x.shape[0]
+    _lib.check(_lib.load().mri_dpmpp_step(_p(x), _p(eps), eps_nhwc_ldc, channels, _p(x0_prev),
+                                          _p(coef), _p(k), _p(out), n, x.numel() // n, _s()),
+               "mri_dpmpp_step")
+
+
+def step_table_advance(t: torch.Tensor, k: torch.Tensor, ts: torch.Tensor, rows: int) -> None:
+    """k += 1, then t[:] = ts[min(k, rows - 1)] (one launch, stream-ordered)."""
+    assert t.dtype == k.dtype == ts.dtype == torch.int64 and 1 <= rows <= ts.numel()
+    _lib.check(_lib.load().mri_step_table_advance(_p(t), t.numel(), _p(k), _p(ts), int(rows), _s()),
+               "mri_step_table_advance")
+
+
 def minsnr_loss(pred, noise, t, snr, gamma: float, per_sample_out, loss_out) -> None:
     _chk_contig(pred, noise)
     n = pred.shape[0]
@@ -220,14 +240,17 @@ def ddpm_step_rng(x, eps, rng: DeviceRng, t, betas, sqrt_1mac, sqrt_recip_alphas
 
 def tap_gather_step(y, bias, samples, D, H, W, ndim, cout, ldy, x, mode: int, rng=None, t=None,
                     t_prev=None, betas=None, sqrt_1mac=None, sqrt_recip_alphas=None, post_var=None,
-                    alphas_cumprod=None, eps_out=None, ldo: int = 0) -> None:
+                    alphas_cumprod=None, eps_out=None, ldo: int = 0, x0_prev=None, coef=None,
+                    k=None) -> None:
     """Finish the thin out_conv (sum of shifted tap products) and apply the reverse-step update to
-    the sampler state x in place: mode 0 DDPM (noise drawn in-kernel), 1 DDIM, 2 eps only."""
-    _chk_contig(y, x, eps_out)
+    the sampler state x in place: mode 0 DDPM (noise drawn in-kernel), 1 DDIM, 2 eps only,
+    3 DPM-Solver++(2M) (x0_prev, coef row k: see dpmpp_step)."""
+    _chk_contig(y, x, eps_out, x0_prev, coef)
     _lib.check(_lib.load().mri_tap_gather_step(
         _p(y), _p(bias), samples, D, H, W, ndim, cout, ldy, _p(x), _p(eps_out), ldo, mode,
         _p(rng.state) if rng is not None else None, _p(t), _p(t_prev), _p(betas), _p(sqrt_1mac),
-        _p(sqrt_recip_alphas), _p(post_var), _p(alphas_cumprod), _s()), "mri_tap_gather_step")
+        _p(sqrt_recip_alphas), _p(post_var), _p(alphas_cumprod), _p(x0_prev), _p(coef), _p(k),
+        _s()), "mri_tap_gather_step")
 
 
 def step_advance(t: torch.Tensor, delta: int, t_prev=None, rng: Optional[DeviceRng] = None,

@@ -38,9 +38,10 @@ def _world() -> Tuple[int, int]:
 
 def sample_sharded(diffusion, total_batch: int, *sample_args, base_seed: int = 1234,
                    gather: bool = True, per_sample_kwargs: Optional[dict] = None,
-                   **sample_kwargs) -> Optional[torch.Tensor]:
+                   method: str = "sample", **sample_kwargs) -> Optional[torch.Tensor]:
     """Generate `total_batch` samples across all ranks: rank r runs
-    diffusion.sample(its share, *sample_args, **sample_kwargs) under seed base_seed + r.
+    getattr(diffusion, method)(its share, *sample_args, **sample_kwargs) under seed
+    base_seed + r (method="sample_dpmpp", num_steps=20: the few-step sampler).
 
     per_sample_kwargs: tensors with a leading dim of total_batch (e.g. z_pos of the 155 slices of
     a pseudo-3D brain, slice_cond_2d_ddpm/show_model.py:179-185) that are sliced per rank.
@@ -56,7 +57,7 @@ def sample_sharded(diffusion, total_batch: int, *sample_args, base_seed: int = 1
     local = None
     if hi > lo:
         torch.manual_seed(base_seed + rank)
-        local = diffusion.sample(hi - lo, *sample_args, **kw)
+        local = getattr(diffusion, method)(hi - lo, *sample_args, **kw)
     if not gather or world == 1:
         return local
     return gather_to_rank0(local, total_batch)

@@ -46,3 +46,55 @@ def make_buffers(betas: torch.Tensor, with_snr: bool) -> "OrderedDict[str, torch
     out["posterior_variance"] = posterior_variance
     out["posterior_log_variance_clipped"] = torch.log(torch.clamp(posterior_variance, min=1e-20))
     return out
+
+
+def dpmpp_timesteps(start_t: int, num_steps: int) -> list:
+    """The points DPM-Solver++(2M) visits: round(linspace(start_t, 0, M + 1))[:-1] in integer
+    arithmetic (halves round up), then -1 for sigma = 0.  With start_t = T - 1 this is the
+    "linspace" timestep spacing of diffusers' multistep scheduler.  Needs 1 <= M <= start_t, which
+    keeps the UNet timesteps distinct and >= 1."""
+    M, s = int(num_steps), int(start_t)
+    if not 1 <= M <= s:
+        raise ValueError(f"need 1 <= num_steps <= start_t (got num_steps={M}, start_t={s})")
+    return [(2 * s * (M - i) + M) // (2 * M) for i in range(M)] + [-1]
+
+
+def dpmpp_2m_table(alphas_cumprod: torch.Tensor, timesteps):
+    """DPM-Solver++(2M) (data prediction, midpoint second-order form) over the visited points
+    t_0 > t_1 > ... > t_M; a final -1 means sigma = 0.  Returns (ts, coef): the M timesteps the
+    UNet is evaluated at (int64) and one fp32 row (s, r, A, B, C) per step, for the update
+
+        x0 = (x - s * eps) * r ;  x <- (A * x + B * x0) + C * (x0 - x0_prev)
+
+    computed in fp64 from the fp32 alphas_cumprod and rounded once.  Row 0 is first order (C = 0);
+    a step to sigma = 0 is first order and returns x0 (A, B, C = 0, 1, 0)."""
+    ac = [float(v) for v in alphas_cumprod.detach().cpu().double().tolist()]
+    T = len(ac)
+    ts = [int(v) for v in timesteps]
+    if len(ts) < 2:
+        raise ValueError("DPM-Solver++ needs at least two timesteps")
+    for i, t in enumerate(ts):
+        if not (0 <= t <= T - 1 or (t == -1 and i == len(ts) - 1)):
+            raise ValueError(f"timestep {t} outside [0, {T - 1}] (only the last may be -1)")
+    if any(a <= b for a, b in zip(ts, ts[1:])):
+        raise ValueError(f"timesteps must be strictly decreasing: {ts}")
+    M = len(ts) - 1
+    alpha = [math.sqrt(ac[t]) if t >= 0 else 1.0 for t in ts]
+    sigma = [math.sqrt(1.0 - ac[t]) if t >= 0 else 0.0 for t in ts]
+    lam = [math.log(alpha[i]) - math.log(sigma[i]) if ts[i] >= 0 else math.inf for i in range(M + 1)]
+    rows = []
+    for i in range(M):
+        s, r = sigma[i], 1.0 / alpha[i]
+        if ts[i + 1] < 0:
+            rows.append((s, r, 0.0, 1.0, 0.0))
+            continue
+        h = lam[i + 1] - lam[i]
+        phi = math.expm1(-h)
+        A, B = sigma[i + 1] / sigma[i], -alpha[i + 1] * phi
+        C = 0.0
+        if i > 0:
+            rho = (lam[i] - lam[i - 1]) / h
+            C = -0.5 * alpha[i + 1] * phi / rho
+        rows.append((s, r, A, B, C))
+    return (torch.tensor(ts[:M], dtype=torch.int64),
+            torch.tensor(rows, dtype=torch.float64).to(torch.float32))
