@@ -295,6 +295,18 @@ int mri_dpmpp_step(const float* x, const void* eps, int eps_nhwc_ldc, int channe
 /* mri_step_table_advance: k[0] += 1, then t[b] = ts[min(k[0], rows - 1)] for b < n, in one
  * launch (race-free for any n) -- the bookkeeping between two replays of a DPM-Solver++ step. */
 int mri_step_table_advance(int64_t* t, int n, int64_t* k, const int64_t* ts, int rows, void* stream);
+/* mri_inpaint_merge: inpainting by replacement (not in the reference), in place per element:
+ *     x = mask ? x : (tau < 0 ? known : sqrt_ac[tau]*known + sqrt_1mac[tau]*z),  tau = t[n] + t_delta
+ * with mri_q_sample's operations.  mask: one uint8 per element (nonzero = regenerate), known fp32,
+ * both in x's layout.  z comes from `noise` (fp32, x's layout) or, with rng, from Philox under the
+ * ATen mapping at generator offset rng[1] + rng_skip (rng_skip a multiple of 4): the
+ * torch.randn_like that follows a draw which advanced the offset by rng_skip.  Exactly one of
+ * noise / rng.  Values of known where mask != 0 and of x where mask == 0 never reach the output
+ * (selected, not blended: NaN there is harmless); both buffers must still be readable in full. */
+int mri_inpaint_merge(float* x, const float* known, const uint8_t* mask, const float* noise,
+                      const uint64_t* rng, uint64_t rng_skip, const int64_t* t, int64_t t_delta,
+                      const float* sqrt_ac, const float* sqrt_1mac, int samples, int64_t per_sample,
+                      void* stream);
 int mri_minsnr_loss(const float* pred, const float* noise, const int64_t* t, const float* snr,
                     float gamma, float* per_sample_out, float* loss_out, int samples,
                     int64_t per_sample, void* stream);

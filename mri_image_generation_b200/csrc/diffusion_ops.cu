@@ -126,17 +126,19 @@ __device__ __forceinline__ float load_eps(const void* eps, int ldc, long long sp
 // The element loop shared by the kernels below.  MODE_RNG: z comes from Philox (ATen mapping);
 // otherwise from `noise` (may be null when F ignores z).  F(e, z) handles ONE element; the
 // loop hands it four consecutive elements at a time, so the compiler keeps 16-byte accesses where
-// F's loads / stores are expressed through the Vec4 helpers.
+// F's loads / stores are expressed through the Vec4 helpers.  ctr_skip: Philox counters skipped
+// past the generator offset (a later draw of the same size: its offset increment / 4).
 template <bool RNG, class F4, class F1>
 __device__ __forceinline__ void element_loop(long long numel, long long Tt, int n_iter,
-                                             const uint64_t* rng, const float* noise, F4 f4, F1 f1) {
+                                             const uint64_t* rng, const float* noise, F4 f4, F1 f1,
+                                             uint64_t ctr_skip = 0) {
   const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long j0 = 4 * k;
   if (j0 >= Tt) return;
   uint64_t seed = 0, ctr0 = 0;
   if (RNG) {
     seed = rng[0];
-    ctr0 = rng[1] >> 2;
+    ctr0 = (rng[1] >> 2) + ctr_skip;
   }
   const bool n_al = (reinterpret_cast<uintptr_t>(noise) & 15) == 0;
   for (int it = 0; it < n_iter; ++it) {
@@ -386,6 +388,47 @@ step_table_advance_kernel(int64_t* t, int n, int64_t* k, const int64_t* ts, int 
   if (threadIdx.x == 0) *k = kn;
   const int64_t v = ts[kn < rows ? kn : rows - 1];
   for (int b = threadIdx.x; b < n; b += blockDim.x) t[b] = v;
+}
+
+// Inpainting by replacement, in place: x <- where(mask, x, kn) with, per sample, tau = t + t_delta
+// and kn = known (tau < 0) or sqrt_ac[tau]*known + sqrt_1mac[tau]*z (q_sample_kernel's operations).
+// Select, never blend: values of known where mask != 0 and of x where mask == 0 never reach the
+// output, NaN included (the 16-byte path still loads all four of both); a four-element group with
+// every mask byte set is not touched.
+template <bool RNG>
+__global__ void __launch_bounds__(256)
+inpaint_merge_kernel(float* x, const float* known, const uint8_t* mask, const float* noise,
+                     const uint64_t* rng, uint64_t ctr_skip, const int64_t* t, long long t_delta,
+                     const float* sqrt_ac, const float* sqrt_1mac, long long per_sample,
+                     long long numel, long long Tt, int n_iter) {
+  const bool al = aligned16(x) && aligned16(known) && (reinterpret_cast<uintptr_t>(mask) & 3) == 0;
+  auto kn = [&](long long tau, float k0, float z) {
+    return tau < 0 ? k0 : __fadd_rn(__fmul_rn(__ldg(sqrt_ac + tau), k0), __fmul_rn(__ldg(sqrt_1mac + tau), z));
+  };
+  auto one = [&](long long e, float z) {
+    if (mask[e] != 0) return;
+    x[e] = kn(t[e / per_sample] + t_delta, known[e], z);
+  };
+  element_loop<RNG>(numel, Tt, n_iter, rng, noise,
+      [&](long long e0, const float (&z)[4]) {
+        const long long n = e0 / per_sample;
+        if (!al || (e0 + 3) / per_sample != n) {
+#pragma unroll
+          for (int m = 0; m < 4; ++m) one(e0 + m, z[m]);
+          return;
+        }
+        const uchar4 mk = *reinterpret_cast<const uchar4*>(mask + e0);
+        const bool keep[4] = {mk.x != 0, mk.y != 0, mk.z != 0, mk.w != 0};
+        if (keep[0] && keep[1] && keep[2] && keep[3]) return;
+        const long long tau = t[n] + t_delta;
+        float xv[4], kv[4];
+        load4(x + e0, true, xv);
+        load4(known + e0, true, kv);
+#pragma unroll
+        for (int m = 0; m < 4; ++m) xv[m] = keep[m] ? xv[m] : kn(tau, kv[m], z[m]);
+        store4(x + e0, true, xv);
+      },
+      one, ctr_skip);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -789,6 +832,33 @@ extern "C" int mri_step_table_advance(int64_t* t, int n, int64_t* k, const int64
     return set_error(-2, "mri_step_table_advance: null t / k / ts or rows < 1");
   step_table_advance_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(t, n, k, ts, rows);
   return check_launch("step_table_advance_kernel");
+}
+
+extern "C" int mri_inpaint_merge(float* x, const float* known, const uint8_t* mask,
+                                 const float* noise, const uint64_t* rng, uint64_t rng_skip,
+                                 const int64_t* t, int64_t t_delta, const float* sqrt_ac,
+                                 const float* sqrt_1mac, int samples, int64_t per_sample,
+                                 void* stream) {
+  if (samples < 1 || per_sample < 1) return set_error(-2, "mri_inpaint_merge: empty input");
+  if (x == nullptr || known == nullptr || mask == nullptr || t == nullptr || sqrt_ac == nullptr ||
+      sqrt_1mac == nullptr)
+    return set_error(-2, "mri_inpaint_merge: null x / known / mask / t / schedule table");
+  if ((noise == nullptr) == (rng == nullptr))
+    return set_error(-2, "mri_inpaint_merge: exactly one of noise / rng");
+  if (rng_skip % 4 != 0) return set_error(-2, "mri_inpaint_merge: rng_skip must be a multiple of 4");
+  const long long numel = (long long)samples * per_sample;
+  int rc = device_props();
+  if (rc) return rc;
+  const AtenGrid g = aten_grid(numel);
+  if (rng != nullptr)
+    inpaint_merge_kernel<true><<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
+        x, known, mask, nullptr, rng, rng_skip / 4, t, t_delta, sqrt_ac, sqrt_1mac, per_sample, numel,
+        g.Tt, g.n_iter);
+  else
+    inpaint_merge_kernel<false><<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
+        x, known, mask, noise, nullptr, 0, t, t_delta, sqrt_ac, sqrt_1mac, per_sample, numel, g.Tt,
+        g.n_iter);
+  return check_launch("inpaint_merge_kernel");
 }
 
 extern "C" int mri_rng_seed(uint64_t* rng, uint64_t seed, uint64_t offset, void* stream) {

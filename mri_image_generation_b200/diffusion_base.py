@@ -5,6 +5,7 @@ model arguments (z_pos, context) and the loss; everything that touches the GPU i
   - q_sample / p_sample / DDIM arithmetic: one fused fp32 kernel each (mri_q_sample,
     mri_ddpm_step, mri_ddim_step), bit-exact w.r.t. the reference's eager association order;
     DPM-Solver++(2M) (not in the reference): mri_dpmpp_step over a host-built coefficient table;
+    inpainting (not in the reference): mri_inpaint_merge after each update of either sampler;
   - the reverse loop: when the denoiser is one of this package's UNets, one CUDA graph holds a
     whole reverse step (time embedding, UNet, fused update with the noise drawn INSIDE the
     kernel, t -= 1) and is replayed T times.  The kernels draw Philox4x32-10 + Box-Muller
@@ -163,23 +164,91 @@ class DiffusionBase(nn.Module):
                              f"(got num_steps={M}, start_t={s})")
         return schedules.dpmpp_2m_table(self.alphas_cumprod, schedules.dpmpp_timesteps(s, M))
 
-    def _sample_dpmpp(self, img, table, prog, eps_fn: Callable) -> torch.Tensor:
+    def _sample_dpmpp(self, img, table, prog, eps_fn: Callable, inpaint=None) -> torch.Tensor:
         """Run the solver over `table` from x = img.  prog: a UNetProgram whose conditioning inputs
         the caller has set (replayed step graph), or None: eager, eps = eps_fn(x, t) per step.
+        inpaint: (known, mask) of _inpaint_inputs; after row i the kept region is replaced by
+        q_sample(known, ts[i + 1], noise=img), and by known itself after the last row.
         Returns the fp32 x0 estimate."""
         _require_cuda(img, "sample_dpmpp")
         ts, coef = table
         if prog is not None:
-            return self._reverse_loop(prog, img.float(), int(ts[0]), ts.numel(), "dpmpp", table=table)
+            return self._reverse_loop(prog, img.float(), int(ts[0]), ts.numel(), "dpmpp", table=table,
+                                      inpaint=inpaint)
         dev = img.device
         with torch.cuda.device(dev):
             coef = coef.to(dev)
             x = img.float().contiguous().clone()
+            x_T = x.clone() if inpaint is not None else None
             x0_prev = torch.empty_like(x)
+            tau = ts.tolist()[1:] + [-1]
             for i, t in enumerate(ts.tolist()):
                 tt = torch.full((x.shape[0],), t, device=dev, dtype=torch.long)
                 eps = eps_fn(x, tt)
                 ops.dpmpp_step(x, eps.float().contiguous(), x0_prev, coef[i], None, x)
+                if inpaint is not None:
+                    tt.fill_(tau[i])
+                    ops.inpaint_merge(x, inpaint[0], inpaint[1], tt, 0, self.sqrt_alphas_cumprod,
+                                      self.sqrt_one_minus_alphas_cumprod, noise=x_T)
+        return x
+
+    # ------------------------------------------------------------------ inpainting
+    def _inpaint_inputs(self, x_known, mask, rank: int) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Check (x_known, mask) and return them as the kernel reads them: x_known fp32, mask one
+        uint8 per element (1 = regenerate, 0 = keep), both contiguous on x_known's device.  Raises
+        ValueError on a bad shape or mask; callers check before anything is drawn."""
+        if not torch.is_tensor(x_known) or x_known.dim() != rank or x_known.shape[1] != self.channels:
+            raise ValueError(f"x_known must be a (B, {self.channels}, ...) tensor of rank {rank} "
+                             f"(got {tuple(x_known.shape) if torch.is_tensor(x_known) else type(x_known)})")
+        if x_known.numel() == 0:
+            raise ValueError("x_known is empty")
+        mask = torch.as_tensor(mask)
+        try:
+            ok = torch.broadcast_shapes(mask.shape, x_known.shape) == x_known.shape
+        except RuntimeError:
+            ok = False
+        if not ok:
+            raise ValueError(f"mask of shape {tuple(mask.shape)} does not broadcast to x_known's "
+                             f"{tuple(x_known.shape)}")
+        if mask.dtype != torch.bool and not bool(((mask == 0) | (mask == 1)).all()):
+            raise ValueError("mask must be bool or hold only 0 / 1 (1 = regenerate, 0 = keep)")
+        known = x_known.float().contiguous()
+        m = torch.empty(known.shape, dtype=torch.uint8, device=known.device)
+        m.copy_(mask.to(known.device).expand(known.shape))
+        return known, m
+
+    def _inpaint_buffers(self, prog, with_noise: bool) -> Dict[str, torch.Tensor]:
+        """The program's inpainting inputs: known, mask and, for DPM-Solver++, the x_T copy the
+        known region is noised with.  Each call copies into them, so one captured graph serves
+        every x_known and mask."""
+        bufs = prog.__dict__.setdefault("_inpaint_bufs", {})
+        if "known" not in bufs:
+            bufs["known"] = torch.zeros_like(prog.x_in)
+            bufs["mask"] = torch.zeros(prog.x_in.shape, dtype=torch.uint8, device=prog.x_in.device)
+        if with_noise and "noise" not in bufs:
+            bufs["noise"] = torch.zeros_like(prog.x_in)
+        return bufs
+
+    def _inpaint_ddpm(self, img, inpaint, prog, eps_fn: Callable) -> torch.Tensor:
+        """Ancestral sampling from x_T = img over every timestep with the kept region replaced after
+        each update by q_sample(known, i - 1, noise=randn_like(x)) (known itself after i = 0).
+        prog / eps_fn as for _sample_dpmpp."""
+        _require_cuda(img, "inpaint")
+        T = self.timesteps
+        if prog is not None:
+            return self._reverse_loop(prog, img.float(), T - 1, T, "ddpm", inpaint=inpaint)
+        dev = img.device
+        x = img.float().contiguous()
+        with torch.cuda.device(dev):
+            rng = self._rng(dev)
+            inc = ops.randn_offset_increment(x.numel())
+            for i in reversed(range(T)):
+                t = torch.full((x.shape[0],), i, device=dev, dtype=torch.long)
+                x = self._p_update(x, t, eps_fn(x, t))
+                off = rng.load()
+                ops.inpaint_merge(x, inpaint[0], inpaint[1], t, -1, self.sqrt_alphas_cumprod,
+                                  self.sqrt_one_minus_alphas_cumprod, rng=rng)
+                rng.commit(off + inc)
         return x
 
     def _dpmpp_buffers(self, prog, rows: int) -> Dict[str, torch.Tensor]:
@@ -193,7 +262,8 @@ class DiffusionBase(nn.Module):
                         k=torch.zeros(1, dtype=torch.int64, device=dev),
                         x0_prev=torch.zeros_like(prog.x_in))
             prog.__dict__["_dpmpp_bufs"] = bufs
-            prog.__dict__.get("_step_graphs", {}).pop("dpmpp", None)  # captured on the old buffers
+            for key in ("dpmpp", "dpmpp+inpaint"):   # captured on the old buffers
+                prog.__dict__.get("_step_graphs", {}).pop(key, None)
         return bufs
 
     # ------------------------------------------------------------------ graph-replayed loops
@@ -207,7 +277,7 @@ class DiffusionBase(nn.Module):
     def _schedule_ptrs(self) -> Tuple[int, ...]:
         return tuple(getattr(self, n).data_ptr() for n in
                      ("betas", "sqrt_one_minus_alphas_cumprod", "sqrt_recip_alphas",
-                      "posterior_variance", "alphas_cumprod"))
+                      "posterior_variance", "alphas_cumprod", "sqrt_alphas_cumprod"))
 
     def _step_graph(self, prog, mode: str, one_step, tprev):
         """The CUDA graph of one reverse step on `prog`.  The graph lives ON the program (it
@@ -249,17 +319,19 @@ class DiffusionBase(nn.Module):
 
     def _reverse_loop(self, prog, img: torch.Tensor, start_t: int, n_steps: int, mode: str,
                       use_graph: bool = True, t_vec: Optional[torch.Tensor] = None,
-                      stride: int = 1, table=None) -> torch.Tensor:
+                      stride: int = 1, table=None, inpaint=None) -> torch.Tensor:
         """Run n_steps reverse steps (i = start_t, start_t - stride, ...) on `prog` (a UNetProgram
         whose x_in is the sampler state).  mode: 'ddpm' | 'ddim' (t_prev = max(t - stride, 0)) |
-        'dpmpp' (table = (ts, coef) of schedules.dpmpp_2m_table, n_steps = its rows)."""
+        'dpmpp' (table = (ts, coef) of schedules.dpmpp_2m_table, n_steps = its rows).
+        inpaint: (known, mask) of _inpaint_inputs, 'ddpm' or 'dpmpp' only: mri_inpaint_merge
+        after every update, on a step graph of its own ('ddpm+inpaint' / 'dpmpp+inpaint')."""
         dev = img.device
         with torch.cuda.device(dev):
             return self._reverse_loop_on(prog, img, start_t, n_steps, mode, use_graph, t_vec, stride,
-                                         table)
+                                         table, inpaint)
 
     def _reverse_loop_on(self, prog, img, start_t, n_steps, mode, use_graph, t_vec, stride,
-                         table=None):
+                         table=None, inpaint=None):
         dev = img.device
         if prog.params_changed():
             prog.do_refresh()
@@ -273,6 +345,14 @@ class DiffusionBase(nn.Module):
             raise _lib.MriError("strided timesteps need the DDIM update")
         # the graph bakes the stride in: one graph per (mode, stride)
         gkey = mode if stride == 1 else f"{mode}/{stride}"
+        inp = None
+        if inpaint is not None:
+            if mode not in ("ddpm", "dpmpp") or stride != 1 or t_vec is not None:
+                raise _lib.MriError("inpainting runs on the full DDPM or the DPM-Solver++ loop")
+            inp = self._inpaint_buffers(prog, mode == "dpmpp")
+            gkey += "+inpaint"
+        # DDPM inpainting draws a second randn_like(x) per step (the merge's noise)
+        adv = 2 * inc if inp is not None else inc
 
         fused = (getattr(prog, "fused_head", None) is not None and not prog.training
                  and os.environ.get("MRI_FUSED_STEP", "1") != "0")
@@ -283,6 +363,16 @@ class DiffusionBase(nn.Module):
             kbuf, xp, rows = dpm["k"], dpm["x0_prev"], dpm["ts"].numel()
             kbuf.zero_()   # a valid row for the warm-up launch of a capture
 
+        def merge():
+            if mode == "ddpm":   # before step_advance: tau = t - 1, z drawn after the update's z
+                ops.inpaint_merge(prog.x_in, inp["known"], inp["mask"], prog.t_in, -1,
+                                  self.sqrt_alphas_cumprod, self.sqrt_one_minus_alphas_cumprod,
+                                  rng=rng, rng_skip=inc)
+            else:                # after step_table_advance: t = ts[k], -1 past the last row
+                ops.inpaint_merge(prog.x_in, inp["known"], inp["mask"], prog.t_in, 0,
+                                  self.sqrt_alphas_cumprod, self.sqrt_one_minus_alphas_cumprod,
+                                  noise=inp["noise"])
+
         def one_step():
             if fused:  # out_conv's tap sum + the update in one kernel: eps never goes to HBM
                 if mode == "ddpm":
@@ -290,10 +380,14 @@ class DiffusionBase(nn.Module):
                                         sqrt_1mac=self.sqrt_one_minus_alphas_cumprod,
                                         sqrt_recip_alphas=self.sqrt_recip_alphas,
                                         post_var=self.posterior_variance)
-                    ops.step_advance(prog.t_in, -1, rng=rng, rng_increment=inc)
+                    if inp is not None:
+                        merge()
+                    ops.step_advance(prog.t_in, -1, rng=rng, rng_increment=adv)
                 elif mode == "dpmpp":
                     prog.run_fused_step(3, x0_prev=xp, coef=dpm["coef"], k=kbuf)
                     ops.step_table_advance(prog.t_in, kbuf, dpm["ts"], rows)
+                    if inp is not None:
+                        merge()
                 else:
                     prog.run_fused_step(1, t=prog.t_in, t_prev=tprev, alphas_cumprod=self.alphas_cumprod)
                     ops.step_advance(prog.t_in, -stride, t_prev=tprev)
@@ -303,11 +397,15 @@ class DiffusionBase(nn.Module):
                 ops.ddpm_step_rng(prog.x_in, prog.eps_nhwc, rng, prog.t_in, self.betas,
                                   self.sqrt_one_minus_alphas_cumprod, self.sqrt_recip_alphas,
                                   self.posterior_variance, prog.x_in, eps_nhwc_ldc=ldc, channels=C)
-                ops.step_advance(prog.t_in, -1, rng=rng, rng_increment=inc)
+                if inp is not None:
+                    merge()
+                ops.step_advance(prog.t_in, -1, rng=rng, rng_increment=adv)
             elif mode == "dpmpp":
                 ops.dpmpp_step(prog.x_in, prog.eps_nhwc, xp, dpm["coef"], kbuf, prog.x_in,
                                eps_nhwc_ldc=ldc, channels=C)
                 ops.step_table_advance(prog.t_in, kbuf, dpm["ts"], rows)
+                if inp is not None:
+                    merge()
             else:
                 ops.ddim_step(prog.x_in, prog.eps_nhwc, prog.t_in, tprev, self.alphas_cumprod,
                               prog.x_in, eps_nhwc_ldc=ldc, channels=C)
@@ -327,8 +425,14 @@ class DiffusionBase(nn.Module):
             M = ts.numel()
             dpm["coef"][:M].copy_(coef)
             dpm["ts"][:M].copy_(ts)
-            dpm["ts"][M:].fill_(int(ts[-1]))
+            # with inpainting, t after the last row's advance is -1: the merge then keeps x_known
+            dpm["ts"][M:].fill_(-1 if inp is not None else int(ts[-1]))
             kbuf.zero_()
+        if inp is not None:
+            inp["known"].copy_(inpaint[0])
+            inp["mask"].copy_(inpaint[1])
+            if mode == "dpmpp":
+                inp["noise"].copy_(img)
         off = rng.load() if mode == "ddpm" else 0
         for _ in range(n_steps):
             if graph is not None:
@@ -336,6 +440,6 @@ class DiffusionBase(nn.Module):
             else:
                 one_step()
         if mode == "ddpm":  # z = randn_like(x) is drawn at every step, t = 0 included
-            rng.commit(off + n_steps * inc)
+            rng.commit(off + n_steps * adv)
         assert per_sample == prog.x_in[0].numel()
         return prog.x_in.clone()

@@ -80,3 +80,33 @@ class GaussianDiffusion(_GD2):
                 prog.ctx_in.copy_(context)
         return self._sample_dpmpp(img, table, prog,
                                   lambda x, t: self.model(x, t, z_pos, context=context))
+
+    @torch.no_grad()
+    def inpaint(self, x_known, mask, z_pos=0.5, context=None):
+        """Inpainting by replacement with the full DDPM sampler (not in the reference), e.g.
+        missing-modality imputation: x_known (B, 4, H, W) holds t1, t1ce, t2, flair and a mask of
+        shape (1, 4, 1, 1) set only at the missing channel regenerates that modality.  See the 2D
+        class's inpaint() for the method."""
+        known, m = self._inpaint_inputs(x_known, mask, 4)
+        device = self.betas.device
+        if context is not None:
+            context = context.to(device)
+        img, prog = self._inpaint_start(known, z_pos, context)
+        z_pos = self._z_tensor(z_pos, img.shape[0], device)
+        return self._inpaint_ddpm(img, (known.to(device), m.to(device)), prog,
+                                  lambda x, t: self.model(x, t, z_pos, context=context))
+
+    @torch.no_grad()
+    def inpaint_dpmpp(self, x_known, mask, z_pos=0.5, context=None, num_steps=20):
+        """inpaint() with DPM-Solver++(2M) in `num_steps` UNet calls (not in the reference); see
+        the 2D class's inpaint_dpmpp()."""
+        known, m = self._inpaint_inputs(x_known, mask, 4)
+        table = self._dpmpp_table(self.timesteps - 1, num_steps)
+        device = self.betas.device
+        if context is not None:
+            context = context.to(device)
+        img, prog = self._inpaint_start(known, z_pos, context)
+        z_pos = self._z_tensor(z_pos, img.shape[0], device)
+        return self._sample_dpmpp(img, table, prog,
+                                  lambda x, t: self.model(x, t, z_pos, context=context),
+                                  inpaint=(known.to(device), m.to(device)))

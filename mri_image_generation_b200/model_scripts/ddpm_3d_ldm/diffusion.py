@@ -146,9 +146,37 @@ class GaussianDiffusionLatent3D(DiffusionBase):
         (not in the reference); the result is the fp32 x0 estimate."""
         return self._dpmpp_from(x_t, self._dpmpp_table(start_t, num_steps), cond)
 
-    def _dpmpp_from(self, x_t, table, cond):
+    def _dpmpp_from(self, x_t, table, cond, inpaint=None):
         _require_cuda(x_t, "sample_from_dpmpp")
+        return self._sample_dpmpp(x_t, table, self._program_for(x_t, cond), self._eps_fn(cond),
+                                  inpaint=inpaint)
+
+    def _program_for(self, x, cond):
         eng = self._engine_model()
-        prog = eng.program(x_t.shape[0], x_t.shape[2:]) if eng is not None and cond is None else None
-        return self._sample_dpmpp(
-            x_t, table, prog, lambda x, t: self.model(x, t) if cond is None else self.model(x, t, cond))
+        return eng.program(x.shape[0], x.shape[2:]) if eng is not None and cond is None else None
+
+    def _eps_fn(self, cond):
+        return lambda x, t: self.model(x, t) if cond is None else self.model(x, t, cond)
+
+    @torch.no_grad()
+    def inpaint(self, x_known, mask, cond=None):
+        """Inpainting by replacement with the full DDPM sampler (not in the reference).  x_known:
+        (B, channels, D, H, W) latents; mask broadcasts to it, True / 1 = regenerate, False / 0 =
+        keep.  x_T is drawn as sample() draws it; after the update at every step i the kept region
+        is set to q_sample(x_known, i - 1, noise=randn_like(x)) (x_known itself after i = 0).  The
+        mask is at latent resolution: mapping an image-space mask to it (e.g. max-pooling by the
+        VAE's downsampling factor) is the caller's job."""
+        known, m = self._inpaint_inputs(x_known, mask, 5)
+        img = self._randn(known.shape, self.betas.device)
+        return self._inpaint_ddpm(img, (known.to(img.device), m.to(img.device)),
+                                  self._program_for(img, cond), self._eps_fn(cond))
+
+    @torch.no_grad()
+    def inpaint_dpmpp(self, x_known, mask, num_steps=20, cond=None):
+        """inpaint() with DPM-Solver++(2M) in `num_steps` UNet calls (not in the reference): after
+        each step the kept region is set to q_sample(x_known, next timestep, noise=x_T), and to
+        x_known after the last.  Conditions less strongly than inpaint() (DESIGN.md §4)."""
+        known, m = self._inpaint_inputs(x_known, mask, 5)
+        table = self._dpmpp_table(self.timesteps - 1, num_steps)
+        img = self._randn(known.shape, self.betas.device)
+        return self._dpmpp_from(img, table, cond, inpaint=(known.to(img.device), m.to(img.device)))

@@ -103,3 +103,42 @@ class GaussianDiffusion(DiffusionBase):
             prog = eng.program(batch_size, shape[2:], shape[1], 0)
             prog.z_in.copy_(z_pos.reshape(-1, 1))
         return self._sample_dpmpp(img, table, prog, lambda x, t: self.model(x, t, z_pos))
+
+    @torch.no_grad()
+    def inpaint(self, x_known, mask, z_pos=0.5):
+        """Inpainting by replacement with the full DDPM sampler (not in the reference).  x_known:
+        (B, channels, H, W); mask broadcasts to it, True / 1 = regenerate, False / 0 = keep.  x_T
+        is drawn as sample() draws it; after the update at every step i the kept region is set to
+        q_sample(x_known, i - 1, noise=randn_like(x)) (x_known itself after i = 0)."""
+        known, m = self._inpaint_inputs(x_known, mask, 4)
+        img, prog = self._inpaint_start(known, z_pos)
+        inp = (known.to(img.device), m.to(img.device))
+        z_pos = self._z_tensor(z_pos, img.shape[0], img.device)
+        return self._inpaint_ddpm(img, inp, prog, lambda x, t: self.model(x, t, z_pos))
+
+    @torch.no_grad()
+    def inpaint_dpmpp(self, x_known, mask, z_pos=0.5, num_steps=20):
+        """inpaint() with DPM-Solver++(2M) in `num_steps` UNet calls (not in the reference): after
+        each step the kept region is set to q_sample(x_known, next timestep, noise=x_T), and to
+        x_known after the last.  Conditions less strongly than inpaint() (DESIGN.md §4)."""
+        known, m = self._inpaint_inputs(x_known, mask, 4)
+        table = self._dpmpp_table(self.timesteps - 1, num_steps)
+        img, prog = self._inpaint_start(known, z_pos)
+        inp = (known.to(img.device), m.to(img.device))
+        z_pos = self._z_tensor(z_pos, img.shape[0], img.device)
+        return self._sample_dpmpp(img, table, prog, lambda x, t: self.model(x, t, z_pos), inpaint=inp)
+
+    def _inpaint_start(self, known, z_pos, context=None):
+        """x_T drawn as sample() draws it, and the program with its conditioning inputs set (None
+        for a model that is not one of this package's UNets)."""
+        device = self.betas.device
+        img = self._randn(known.shape, device)
+        eng = self._engine_model()
+        if eng is None:
+            return img, None
+        B = known.shape[0]
+        prog = eng.program(B, known.shape[2:], known.shape[1], 0 if context is None else context.shape[1])
+        prog.z_in.copy_(self._z_tensor(z_pos, B, device).reshape(-1, 1))
+        if context is not None:
+            prog.ctx_in.copy_(context)
+        return img, prog

@@ -253,6 +253,23 @@ def tap_gather_step(y, bias, samples, D, H, W, ndim, cout, ldy, x, mode: int, rn
         _s()), "mri_tap_gather_step")
 
 
+def inpaint_merge(x, known, mask, t, t_delta: int, sqrt_ac, sqrt_1mac, noise=None,
+                  rng: Optional[DeviceRng] = None, rng_skip: int = 0) -> None:
+    """x = where(mask, x, kn) in place, kn = known if tau < 0 else q_sample(known, tau, z) with
+    tau = t + t_delta per sample (t: device int64 [samples]).  mask: uint8, one byte per element
+    of x.  z: `noise`, or with rng the torch.randn_like drawn rng_skip past the generator offset."""
+    _chk_contig(x, known, mask, noise)
+    assert x.dtype == known.dtype == torch.float32 and mask.dtype == torch.uint8
+    assert known.numel() == mask.numel() == x.numel() and t.dtype == torch.int64
+    assert noise is None or (noise.dtype == torch.float32 and noise.numel() == x.numel())
+    n = x.shape[0]
+    _lib.check(_lib.load().mri_inpaint_merge(_p(x), _p(known), _p(mask), _p(noise),
+                                             _p(rng.state) if rng is not None else None,
+                                             int(rng_skip), _p(t), int(t_delta), _p(sqrt_ac),
+                                             _p(sqrt_1mac), n, x.numel() // n, _s()),
+               "mri_inpaint_merge")
+
+
 def step_advance(t: torch.Tensor, delta: int, t_prev=None, rng: Optional[DeviceRng] = None,
                  rng_increment: int = 0) -> None:
     _lib.check(_lib.load().mri_step_advance(_p(t), _p(t_prev), t.numel(), delta,

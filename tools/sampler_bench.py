@@ -1,12 +1,14 @@
 #!/usr/bin/env python
 """Cost of the three samplers (GPU only): ms per reverse step of the replayed step graph for
-DDPM (ancestral), strided DDIM and DPM-Solver++(2M), and end to end for sample_dpmpp(num_steps=20).
+DDPM (ancestral), strided DDIM and DPM-Solver++(2M), the DDPM and DPM-Solver++ inpainting steps
+(the same step plus mri_inpaint_merge, every element kept: the merge's worst case), and end to end for
+sample_dpmpp(num_steps=20).
 
   cfg4  ddpm_3d_ldm         UNet3DModelWithAttention(3, base 128, mults 1-2-4) B=16 3x40x48x40
   cfg2  slice_cond_2d_ddpm  UNet(1, base 64, mults 1-2-4-8)                   B=64 1x240x240
 
 Each step time is CUDA events around STEPS replays of one captured step graph (after warm-up
-replays); the three samplers are timed in turn, REPS times alternating, and the median and the
+replays); the step graphs are timed in turn, REPS times alternating, and the median and the
 spread ((max - min) / median) are reported.  End to end is CUDA events around the public call
 (x_T draw, table build and upload, 20 replays, result copy), REPS times.  Random-init weights:
 this measures sampling cost only, not sample quality.  GPU name and power limit are read with a
@@ -60,12 +62,22 @@ def summary(v):
 
 
 def step_times(diff, prog, x, steps, reps, warm=3):
-    """ms per replayed step of the DDPM, strided-DDIM and DPM-Solver++ step graphs on `prog`."""
+    """ms per replayed step of the DDPM, strided-DDIM, DPM-Solver++ and the two inpainting step
+    graphs on `prog`."""
+    # inpainting inputs: a known volume and a mask that keeps every element, the merge's most
+    # expensive case (it reads x and known and writes x everywhere; a group of four regenerated
+    # elements would be skipped)
+    known = torch.randn_like(x)
+    mask = torch.zeros(x.shape, dtype=torch.uint8, device=x.device)
     # one short run each captures the step graphs (and warms every shape)
     diff._reverse_loop(prog, x, T - 1, 3, "ddpm")
     diff._reverse_loop(prog, x, T - 1, 3, "ddim", stride=DDIM_STRIDE)
     diff._reverse_loop(prog, x, T - 1, 3, "dpmpp", table=diff._dpmpp_table(T - 1, steps))
-    g = {k: prog._step_graphs[k][2] for k in ("ddpm", f"ddim/{DDIM_STRIDE}", "dpmpp")}
+    diff._reverse_loop(prog, x, T - 1, 3, "ddpm", inpaint=(known, mask))
+    diff._reverse_loop(prog, x, T - 1, 3, "dpmpp", table=diff._dpmpp_table(T - 1, steps),
+                       inpaint=(known, mask))
+    g = {k: prog._step_graphs[k][2] for k in ("ddpm", f"ddim/{DDIM_STRIDE}", "dpmpp", "ddpm+inpaint",
+                                              "dpmpp+inpaint")}
     tprev, dpm = prog._tprev_buf, prog._dpmpp_bufs
     n_ddim = min(steps, (T - 1) // DDIM_STRIDE)   # t stays >= 0 over the timed replays
 
@@ -80,7 +92,8 @@ def step_times(diff, prog, x, steps, reps, warm=3):
         for _ in range(n):
             g[key].replay()
 
-    plan = {"ddpm": ("ddpm", steps), "ddim": (f"ddim/{DDIM_STRIDE}", n_ddim), "dpmpp": ("dpmpp", steps)}
+    plan = {"ddpm": ("ddpm", steps), "ddim": (f"ddim/{DDIM_STRIDE}", n_ddim), "dpmpp": ("dpmpp", steps),
+            "ddpm+inpaint": ("ddpm+inpaint", steps), "dpmpp+inpaint": ("dpmpp+inpaint", steps)}
     for name, (key, n) in plan.items():
         reset()
         replays(key, min(warm, n))
@@ -90,7 +103,11 @@ def step_times(diff, prog, x, steps, reps, warm=3):
             reset()
             out[name].append(events_ms(lambda: replays(key, n)) / n)
     assert torch.isfinite(prog.x_in).all()
-    return {k: summary(v) for k, v in out.items()}
+    res = {k: summary(v) for k, v in out.items()}
+    for k in ("ddpm", "dpmpp"):   # the inpainting step against the plain step, run by run
+        ratios = [a / b for a, b in zip(out[f"{k}+inpaint"], out[k])]
+        res[f"{k}+inpaint"]["ratio_to_plain"] = summary(ratios)
+    return res
 
 
 def end_to_end(fn, batch, reps):
