@@ -1,6 +1,6 @@
-// DDPM / DDIM arithmetic as single fused passes.  fp32, written with explicit round-to-nearest
-// intrinsics (never contracted into FMAs) in the reference's exact association order, so the
-// result is bit-identical to eager torch on the same inputs.
+// DDPM / DDIM / DPM-Solver++(2M) arithmetic as single fused passes.  fp32, written with explicit
+// round-to-nearest intrinsics (never contracted into FMAs) in the reference's exact association
+// order, so the result is bit-identical to eager torch on the same inputs.
 // Reference call sites: see include/mri_b200.h.
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
@@ -22,7 +22,10 @@ namespace mri {
 //   _curand_box_muller).  Here one thread owns FOUR consecutive subsequences, so that for each
 //   component it holds four consecutive elements: 16-byte loads and stores.
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+// block `ctr` of subsequence `sub` of the generator seeded with `seed`
+__device__ __forceinline__ uint4 philox4x32_10(uint64_t seed, uint64_t ctr, uint64_t sub) {
+  uint4 c = make_uint4((uint32_t)ctr, (uint32_t)(ctr >> 32), (uint32_t)sub, (uint32_t)(sub >> 32));
+  uint2 k = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
 #pragma unroll
   for (int i = 0; i < 10; ++i) {
     const uint32_t hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
@@ -81,12 +84,9 @@ static AtenGrid aten_grid(long long numel) {
 
 // z[m][ii]: component ii of subsequence j0 + m at counter c
 __device__ __forceinline__ void draw16(uint64_t seed, uint64_t c, uint64_t j0, float (&z)[4][4]) {
-  const uint2 key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
 #pragma unroll
   for (int m = 0; m < 4; ++m) {
-    const uint64_t sub = j0 + (uint64_t)m;
-    const uint4 r = philox4x32_10(
-        make_uint4((uint32_t)c, (uint32_t)(c >> 32), (uint32_t)sub, (uint32_t)(sub >> 32)), key);
+    const uint4 r = philox4x32_10(seed, c, j0 + (uint64_t)m);
     const float2 a = box_muller(r.x, r.y), b = box_muller(r.z, r.w);
     z[m][0] = a.x;
     z[m][1] = a.y;
@@ -95,32 +95,16 @@ __device__ __forceinline__ void draw16(uint64_t seed, uint64_t c, uint64_t j0, f
   }
 }
 
-// per-sample coefficients of one reverse step; the same fp32 operations as the reference:
-// q = beta / s ; c1 = sqrt_recip_alphas ; w = mask * sqrt(pv)
-struct StepCoef {
-  float q, c1, w;
-};
-struct StepTables {
-  const int64_t* t;
-  const float *betas, *sqrt_1mac, *sqrt_recip_alphas, *post_var;
-};
-__device__ __forceinline__ StepCoef step_coef(const StepTables& T, long long n) {
-  const int64_t ts = T.t[n];
-  StepCoef c;
-  c.q = __fdiv_rn(__ldg(T.betas + ts), __ldg(T.sqrt_1mac + ts));
-  c.c1 = __ldg(T.sqrt_recip_alphas + ts);
-  c.w = __fmul_rn(ts != 0 ? 1.0f : 0.0f, __fsqrt_rn(__ldg(T.post_var + ts)));
-  return c;
-}
-
-// eps of NC[D]HW element (sample n, in-sample index j): fp32 in x's layout (ldc = 0) or the bf16
-// channels-last UNet output [n][spatial][ldc]
-__device__ __forceinline__ float load_eps(const void* eps, int ldc, long long spatial,
-                                          long long per_sample, long long n, long long j) {
-  if (ldc == 0) return reinterpret_cast<const float*>(eps)[n * per_sample + j];
-  const long long c = j / spatial;
-  const long long s = j - c * spatial;
-  return __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(eps)[(n * spatial + s) * ldc + c]);
+// z of element idx of a draw at counter ctr0 with ATen's launch of Tt threads: component ii of
+// call `it` of subsequence j
+__device__ __forceinline__ float normal_at(uint64_t seed, uint64_t ctr0, long long idx, long long Tt) {
+  const long long it = idx / (4 * Tt);
+  const long long rem = idx - it * 4 * Tt;
+  const int ii = (int)(rem / Tt);
+  const long long j = rem - (long long)ii * Tt;
+  const uint4 r = philox4x32_10(seed, ctr0 + (uint64_t)it, (uint64_t)j);
+  const float2 bm = ii < 2 ? box_muller(r.x, r.y) : box_muller(r.z, r.w);
+  return (ii & 1) ? bm.y : bm.x;
 }
 
 // The element loop shared by the kernels below.  MODE_RNG: z comes from Philox (ATen mapping);
@@ -239,142 +223,141 @@ q_sample_kernel(const float* x0, const float* noise, const uint64_t* rng, const 
       one);
 }
 
-// x_{t-1} = c1 * (x - q * eps) + w * z.  x / out may alias (the sampler updates its state in place).
-template <bool RNG>
+// ------------------------------------------------------------------------------------------
+// The reverse-step updates, each defined once and shared by step_kernel and
+// tap_gather_step_kernel: coef(n) fetches sample n's coefficients, apply(c, x, eps, z, x0p) returns
+// one element's new state.  fp32 in the reference's association order:
+//   DDPM:  out = c1*(x - q*eps) + w*z,  q = beta[t]/sqrt_1mac[t], c1 = sqrt_recip_alphas[t],
+//          w = (t != 0)*sqrt(post_var[t])
+//   DDIM (eta = 0):  x0 = (x - sqrt(1-a_t)*eps)/max(sqrt(a_t), 1e-8),
+//          out = sqrt(a_p)*x0 + sqrt(1-a_p)*eps,  a_t / a_p = alphas_cumprod[t] / [t_prev]
+//   DPM-Solver++(2M), row k = (s, r, A, B, C) of schedules.dpmpp_2m_table:
+//          x0 = (x - s*eps)*r,  out = (A*x + B*x0) + C*(x0 - x0_prev),  x0_prev <- x0
+// kNoise: the update takes z.  kX0Prev: it keeps the x0_prev state (x0p: that state in, this
+// step's x0 out); the C term is skipped when C == 0, and the callers then do not read x0_prev at
+// all (second(c) false: it may hold anything there, NaN included).  kPerSample: the coefficients
+// depend on the sample (DPM-Solver++'s row does not, and step_kernel fetches it once).
+// ------------------------------------------------------------------------------------------
+struct DdpmUpdate {
+  static constexpr bool kNoise = true, kX0Prev = false, kPerSample = true;
+  struct Coef { float q, c1, w; };
+  const int64_t* t;
+  const float *betas, *sqrt_1mac, *sqrt_recip_alphas, *post_var;
+  __device__ __forceinline__ Coef coef(long long n) const {
+    const int64_t ts = t[n];
+    return Coef{__fdiv_rn(__ldg(betas + ts), __ldg(sqrt_1mac + ts)), __ldg(sqrt_recip_alphas + ts),
+                __fmul_rn(ts != 0 ? 1.0f : 0.0f, __fsqrt_rn(__ldg(post_var + ts)))};
+  }
+  __device__ __forceinline__ static float apply(const Coef& c, float x, float e, float z, float&) {
+    return __fadd_rn(__fmul_rn(c.c1, __fsub_rn(x, __fmul_rn(c.q, e))), __fmul_rn(c.w, z));
+  }
+};
+
+struct DdimUpdate {
+  static constexpr bool kNoise = false, kX0Prev = false, kPerSample = true;
+  struct Coef { float s1m_t, denom, sqrt_a_p, s1m_p; };
+  const int64_t *t, *t_prev;
+  const float* alphas_cumprod;
+  __device__ __forceinline__ Coef coef(long long n) const {
+    const float a_t = __ldg(alphas_cumprod + t[n]);
+    const float a_p = __ldg(alphas_cumprod + t_prev[n]);
+    return Coef{__fsqrt_rn(__fsub_rn(1.0f, a_t)), fmaxf(__fsqrt_rn(a_t), 1e-8f), __fsqrt_rn(a_p),
+                __fsqrt_rn(__fsub_rn(1.0f, a_p))};
+  }
+  __device__ __forceinline__ static float apply(const Coef& c, float x, float e, float, float&) {
+    const float x0 = __fdiv_rn(__fsub_rn(x, __fmul_rn(c.s1m_t, e)), c.denom);
+    return __fadd_rn(__fmul_rn(c.sqrt_a_p, x0), __fmul_rn(c.s1m_p, e));
+  }
+};
+
+struct DpmppUpdate {
+  static constexpr bool kNoise = false, kX0Prev = true, kPerSample = false;
+  struct Coef { float s, r, A, B, C; };
+  const float* table;   // [rows][5]
+  const int64_t* k;     // device row index; null: row 0
+  __device__ __forceinline__ Coef coef(long long) const {
+    const float* c = table + 5 * (k != nullptr ? *k : 0);
+    return Coef{c[0], c[1], c[2], c[3], c[4]};
+  }
+  __device__ __forceinline__ static bool second(const Coef& c) { return c.C != 0.f; }
+  __device__ __forceinline__ static float apply(const Coef& c, float x, float e, float, float& x0p) {
+    const float x0 = __fmul_rn(__fsub_rn(x, __fmul_rn(c.s, e)), c.r);
+    const float o = __fadd_rn(__fmul_rn(c.A, x), __fmul_rn(c.B, x0));
+    const float out = second(c) ? __fadd_rn(o, __fmul_rn(c.C, __fsub_rn(x0, x0p))) : o;
+    x0p = x0;
+    return out;
+  }
+};
+
+// eps of NC[D]HW element (sample n, in-sample index j): fp32 in x's layout (ldc = 0) or the bf16
+// channels-last UNet output [n][spatial][ldc]
+__device__ __forceinline__ float load_eps(const void* eps, int ldc, long long spatial,
+                                          long long per_sample, long long n, long long j) {
+  if (ldc == 0) return reinterpret_cast<const float*>(eps)[n * per_sample + j];
+  const long long c = j / spatial;
+  const long long s = j - c * spatial;
+  return __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(eps)[(n * spatial + s) * ldc + c]);
+}
+// the same for elements j .. j + 3, which lie in one channel; al: the fp32 eps is 16-byte aligned
+__device__ __forceinline__ void load_eps4(const void* eps, int ldc, long long spatial,
+                                          long long per_sample, long long n, long long j, bool al,
+                                          float (&v)[4]) {
+  if (ldc == 0) {
+    load4(reinterpret_cast<const float*>(eps) + n * per_sample + j, al, v);
+    return;
+  }
+  const long long c = j / spatial;
+  const long long s = j - c * spatial;
+  const __nv_bfloat16* p = reinterpret_cast<const __nv_bfloat16*>(eps) + (n * spatial + s) * ldc + c;
+#pragma unroll
+  for (int m = 0; m < 4; ++m) v[m] = __bfloat162float(p[(long long)m * ldc]);
+}
+
+// One reverse step of update U over the fp32 NC[D]HW state; x / out may alias (the sampler updates
+// its state in place).  z: Philox (RNG), else `noise`, null for updates without z; x0_prev: the
+// kX0Prev state in x's layout, null otherwise.
+template <class U, bool RNG>
 __global__ void __launch_bounds__(256)
-ddpm_step_kernel(const float* x, const void* eps, int ldc, int channels, const float* noise,
-                 const uint64_t* rng, StepTables T, float* out, long long per_sample,
-                 long long numel, long long Tt, int n_iter) {
+step_kernel(const U u, const float* x, const void* eps, int ldc, int channels, const float* noise,
+            const uint64_t* rng, float* x0_prev, float* out, long long per_sample, long long numel,
+            long long Tt, int n_iter) {
   const long long spatial = per_sample / (channels > 0 ? channels : 1);
-  const bool al = aligned16(x) && aligned16(out);
+  const bool al = aligned16(x) && aligned16(out) && aligned16(x0_prev);
   const bool eps_al = ldc == 0 && aligned16(eps);
+  const typename U::Coef c_all = U::kPerSample ? typename U::Coef{} : u.coef(0);   // same for all n
+  auto coef = [&](long long n) { return U::kPerSample ? u.coef(n) : c_all; };
   auto one = [&](long long e, float z) {
     const long long n = e / per_sample;
-    const StepCoef c = step_coef(T, n);
     const float ev = load_eps(eps, ldc, spatial, per_sample, n, e - n * per_sample);
-    out[e] = __fadd_rn(__fmul_rn(c.c1, __fsub_rn(x[e], __fmul_rn(c.q, ev))), __fmul_rn(c.w, z));
+    const typename U::Coef c = coef(n);
+    float p = 0.f;
+    if constexpr (U::kX0Prev) {
+      if (U::second(c)) p = x0_prev[e];
+    }
+    out[e] = U::apply(c, x[e], ev, z, p);
+    if constexpr (U::kX0Prev) x0_prev[e] = p;
   };
   element_loop<RNG>(numel, Tt, n_iter, rng, noise,
       [&](long long e0, const float (&z)[4]) {
         const long long n = e0 / per_sample;
         const long long j = e0 - n * per_sample;
         // four elements inside one sample and, for the channels-last eps, inside one channel
-        const bool same = (j + 3 < per_sample) && (ldc == 0 || (j % spatial) + 3 < spatial);
-        if (!same) {
+        if (j + 3 >= per_sample || (ldc != 0 && (j % spatial) + 3 >= spatial)) {
 #pragma unroll
           for (int m = 0; m < 4; ++m) one(e0 + m, z[m]);
           return;
         }
-        const StepCoef c = step_coef(T, n);
-        float xv[4], ev[4], o[4];
+        const typename U::Coef c = coef(n);
+        float xv[4], ev[4], pv[4] = {0.f, 0.f, 0.f, 0.f}, o[4];
         load4(x + e0, al, xv);
-        if (ldc == 0) {
-          load4(reinterpret_cast<const float*>(eps) + e0, eps_al, ev);
-        } else {
-          const long long ch = j / spatial;
-          const long long s = j - ch * spatial;
-          const __nv_bfloat16* ep =
-              reinterpret_cast<const __nv_bfloat16*>(eps) + (n * spatial + s) * ldc + ch;
-#pragma unroll
-          for (int m = 0; m < 4; ++m) ev[m] = __bfloat162float(ep[(long long)m * ldc]);
+        if constexpr (U::kX0Prev) {
+          if (U::second(c)) load4(x0_prev + e0, al, pv);
         }
+        load_eps4(eps, ldc, spatial, per_sample, n, j, eps_al, ev);
 #pragma unroll
-        for (int m = 0; m < 4; ++m)
-          o[m] = __fadd_rn(__fmul_rn(c.c1, __fsub_rn(xv[m], __fmul_rn(c.q, ev[m]))),
-                           __fmul_rn(c.w, z[m]));
+        for (int m = 0; m < 4; ++m) o[m] = U::apply(c, xv[m], ev[m], z[m], pv[m]);
         store4(out + e0, al, o);
-      },
-      one);
-}
-
-// deterministic DDIM step (eta = 0); x / out may alias
-__global__ void __launch_bounds__(256)
-ddim_step_kernel(const float* x, const void* eps, int ldc, int channels, const int64_t* t,
-                 const int64_t* t_prev, const float* ac, float* out, long long per_sample,
-                 long long numel, long long Tt, int n_iter) {
-  const long long spatial = per_sample / (channels > 0 ? channels : 1);
-  auto one = [&](long long e, float) {
-    const long long n = e / per_sample;
-    const float a_t = __ldg(ac + t[n]);
-    const float a_p = __ldg(ac + t_prev[n]);
-    const float sqrt_a_t = __fsqrt_rn(a_t);
-    const float s1m_t = __fsqrt_rn(__fsub_rn(1.0f, a_t));
-    const float denom = fmaxf(sqrt_a_t, 1e-8f);
-    const float sqrt_a_p = __fsqrt_rn(a_p);
-    const float s1m_p = __fsqrt_rn(__fsub_rn(1.0f, a_p));
-    const float ev = load_eps(eps, ldc, spatial, per_sample, n, e - n * per_sample);
-    const float x0 = __fdiv_rn(__fsub_rn(x[e], __fmul_rn(s1m_t, ev)), denom);
-    out[e] = __fadd_rn(__fmul_rn(sqrt_a_p, x0), __fmul_rn(s1m_p, ev));
-  };
-  element_loop<false>(numel, Tt, n_iter, nullptr, nullptr,
-      [&](long long e0, const float (&z)[4]) {
-#pragma unroll
-        for (int m = 0; m < 4; ++m) one(e0 + m, z[m]);
-      },
-      one);
-}
-
-// One DPM-Solver++(2M) step with coefficient row (s, r, A, B, C) (schedules.dpmpp_2m_table):
-//   x0 = (x - s*eps)*r ; out = (A*x + B*x0) + C*(x0 - x0_prev) ; x0_prev <- x0
-// The C term is skipped when C == 0, so x0_prev is never read on a first-order row (it may hold
-// anything there, NaN included).
-struct DpmRow {
-  float s, r, A, B, C;
-};
-__device__ __forceinline__ DpmRow dpm_row(const float* coef, const int64_t* k) {
-  const float* c = coef + 5 * (k != nullptr ? *k : 0);
-  return DpmRow{c[0], c[1], c[2], c[3], c[4]};
-}
-__device__ __forceinline__ float dpm_update(const DpmRow& c, float x, float e, float x0p, float& x0) {
-  x0 = __fmul_rn(__fsub_rn(x, __fmul_rn(c.s, e)), c.r);
-  const float o = __fadd_rn(__fmul_rn(c.A, x), __fmul_rn(c.B, x0));
-  return c.C != 0.f ? __fadd_rn(o, __fmul_rn(c.C, __fsub_rn(x0, x0p))) : o;
-}
-
-// x / out may alias; x0_prev is the solver's [samples][per_sample] fp32 state
-__global__ void __launch_bounds__(256)
-dpmpp_step_kernel(const float* x, const void* eps, int ldc, int channels, float* x0_prev,
-                  const float* coef, const int64_t* k, float* out, long long per_sample,
-                  long long numel, long long Tt, int n_iter) {
-  const long long spatial = per_sample / (channels > 0 ? channels : 1);
-  const DpmRow c = dpm_row(coef, k);
-  const bool second = c.C != 0.f;
-  const bool al = aligned16(x) && aligned16(out) && aligned16(x0_prev);
-  const bool eps_al = ldc == 0 && aligned16(eps);
-  auto one = [&](long long e, float) {
-    const long long n = e / per_sample;
-    const float ev = load_eps(eps, ldc, spatial, per_sample, n, e - n * per_sample);
-    float x0;
-    out[e] = dpm_update(c, x[e], ev, second ? x0_prev[e] : 0.f, x0);
-    x0_prev[e] = x0;
-  };
-  element_loop<false>(numel, Tt, n_iter, nullptr, nullptr,
-      [&](long long e0, const float (&)[4]) {
-        const long long n = e0 / per_sample;
-        const long long j = e0 - n * per_sample;
-        const bool same = (j + 3 < per_sample) && (ldc == 0 || (j % spatial) + 3 < spatial);
-        if (!same) {
-#pragma unroll
-          for (int m = 0; m < 4; ++m) one(e0 + m, 0.f);
-          return;
-        }
-        float xv[4], ev[4], pv[4] = {0.f, 0.f, 0.f, 0.f}, o[4], x0[4];
-        load4(x + e0, al, xv);
-        if (second) load4(x0_prev + e0, al, pv);
-        if (ldc == 0) {
-          load4(reinterpret_cast<const float*>(eps) + e0, eps_al, ev);
-        } else {
-          const long long ch = j / spatial;
-          const long long s = j - ch * spatial;
-          const __nv_bfloat16* ep =
-              reinterpret_cast<const __nv_bfloat16*>(eps) + (n * spatial + s) * ldc + ch;
-#pragma unroll
-          for (int m = 0; m < 4; ++m) ev[m] = __bfloat162float(ep[(long long)m * ldc]);
-        }
-#pragma unroll
-        for (int m = 0; m < 4; ++m) o[m] = dpm_update(c, xv[m], ev[m], pv[m], x0[m]);
-        store4(out + e0, al, o);
-        store4(x0_prev + e0, al, x0);
+        if constexpr (U::kX0Prev) store4(x0_prev + e0, al, pv);
       },
       one);
 }
@@ -447,17 +430,45 @@ struct FusedStepArgs {
   const float* bias;
   float* x;
   __nv_bfloat16* eps_out;   // optional bf16 [positions][ldo]
-  const uint64_t* rng;
-  const int64_t* t;
-  const int64_t* t_prev;    // DDIM
-  const float *betas, *sqrt_1mac, *sqrt_recip_alphas, *post_var, *alphas_cumprod;
-  float* x0_prev;           // DPM-Solver++: solver state, coefficient table, device row index
-  const float* coef;
-  const int64_t* k;
+  const uint64_t* rng;      // DDPM
+  float* x0_prev;           // DPM-Solver++
+  DdpmUpdate ddpm;
+  DdimUpdate ddim;
+  DpmppUpdate dpmpp;
   int samples, D, H, W, ndim, cout, ldy, ldo, mode;  // 0: DDPM, 1: DDIM, 2: eps only, 3: DPM-Solver++
   int TD, TH, TW, pitch_w;  // tile and shared-memory row pitch in 32-bit words
   long long Tt;             // ATen launch geometry of a randn over the whole state
 };
+
+// update U of the cout state elements of one output position (channel co at idx0 + co * spatial,
+// bf16-rounded eps e[co]); every load is issued before the first draw, whose latency it overlaps
+template <class U>
+__device__ __forceinline__ void fused_update(const U& u, const FusedStepArgs& a, int n, long long idx0,
+                                             long long spatial, const float (&e)[4]) {
+  const typename U::Coef c = u.coef(n);
+  float xv[4], p[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+  for (int co = 0; co < 4; ++co) {
+    if (co >= a.cout) break;
+    xv[co] = a.x[idx0 + co * spatial];
+    if constexpr (U::kX0Prev) {
+      if (U::second(c)) p[co] = a.x0_prev[idx0 + co * spatial];
+    }
+  }
+  uint64_t seed = 0, ctr0 = 0;
+  if constexpr (U::kNoise) {
+    seed = a.rng[0];
+    ctr0 = a.rng[1] >> 2;
+  }
+#pragma unroll
+  for (int co = 0; co < 4; ++co) {
+    if (co >= a.cout) break;
+    const long long idx = idx0 + (long long)co * spatial;
+    const float z = U::kNoise ? normal_at(seed, ctr0, idx, a.Tt) : 0.f;
+    a.x[idx] = U::apply(c, xv[co], e[co], z, p[co]);
+    if constexpr (U::kX0Prev) a.x0_prev[idx] = p[co];
+  }
+}
 
 template <int CH>   // 16-byte chunks per Y row that hold the tap products (0: run-time value)
 __global__ void __launch_bounds__(256)
@@ -553,61 +564,18 @@ tap_gather_step_kernel(const FusedStepArgs a) {
           if (co < a.cout) acc[co] += __bfloat162float(row[co]);   // halo rows outside the tensor are 0
       }
   const long long s = ((long long)d0 * a.H + h0) * a.W + w0;
-  const long long per_sample = (long long)a.cout * spatial;
-  // per-sample coefficients
-  float q_c = 0.f, c1 = 0.f, wn = 0.f, sqrt_a_t = 0.f, s1m_t = 0.f, denom = 1.f, sqrt_a_p = 0.f, s1m_p = 0.f;
-  if (a.mode == 0) {
-    StepTables T{a.t, a.betas, a.sqrt_1mac, a.sqrt_recip_alphas, a.post_var};
-    const StepCoef c = step_coef(T, n);
-    q_c = c.q;
-    c1 = c.c1;
-    wn = c.w;
-  } else if (a.mode == 1) {
-    const float a_t = __ldg(a.alphas_cumprod + a.t[n]);
-    const float a_p = __ldg(a.alphas_cumprod + a.t_prev[n]);
-    sqrt_a_t = __fsqrt_rn(a_t);
-    s1m_t = __fsqrt_rn(__fsub_rn(1.0f, a_t));
-    denom = fmaxf(sqrt_a_t, 1e-8f);
-    sqrt_a_p = __fsqrt_rn(a_p);
-    s1m_p = __fsqrt_rn(__fsub_rn(1.0f, a_p));
-  }
-  uint64_t seed = 0, ctr0 = 0;
-  if (a.mode == 0) {
-    seed = a.rng[0];
-    ctr0 = a.rng[1] >> 2;
-  }
+  float e[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
   for (int co = 0; co < 4; ++co) {
     if (co >= a.cout) break;
     const __nv_bfloat16 eb = __float2bfloat16_rn(acc[co]);
     if (a.eps_out != nullptr) a.eps_out[((size_t)n * spatial + s) * a.ldo + co] = eb;
-    if (a.mode == 2) continue;
-    const float e = __bfloat162float(eb);
-    const long long idx = (long long)n * per_sample + (long long)co * spatial + s;   // NC[D]HW element
-    const float xv = a.x[idx];
-    if (a.mode == 0) {
-      // z of element idx under ATen's mapping: call it, component ii of subsequence j
-      const long long it = idx / (4 * a.Tt);
-      const long long rem = idx - it * 4 * a.Tt;
-      const int ii = (int)(rem / a.Tt);
-      const long long j = rem - (long long)ii * a.Tt;
-      const uint64_t cc = ctr0 + (uint64_t)it;
-      const uint4 rr = philox4x32_10(
-          make_uint4((uint32_t)cc, (uint32_t)(cc >> 32), (uint32_t)j, (uint32_t)((uint64_t)j >> 32)),
-          make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
-      const float2 bm = (ii < 2) ? box_muller(rr.x, rr.y) : box_muller(rr.z, rr.w);
-      const float z = (ii & 1) ? bm.y : bm.x;
-      a.x[idx] = __fadd_rn(__fmul_rn(c1, __fsub_rn(xv, __fmul_rn(q_c, e))), __fmul_rn(wn, z));
-    } else if (a.mode == 3) {
-      const DpmRow c = dpm_row(a.coef, a.k);
-      float x0;
-      a.x[idx] = dpm_update(c, xv, e, c.C != 0.f ? a.x0_prev[idx] : 0.f, x0);
-      a.x0_prev[idx] = x0;
-    } else {
-      const float x0 = __fdiv_rn(__fsub_rn(xv, __fmul_rn(s1m_t, e)), denom);
-      a.x[idx] = __fadd_rn(__fmul_rn(sqrt_a_p, x0), __fmul_rn(s1m_p, e));
-    }
+    e[co] = __bfloat162float(eb);
   }
+  const long long idx0 = (long long)n * a.cout * spatial + s;   // NC[D]HW element of channel 0
+  if (a.mode == 0) fused_update(a.ddpm, a, n, idx0, spatial, e);
+  else if (a.mode == 1) fused_update(a.ddim, a, n, idx0, spatial, e);
+  else if (a.mode == 3) fused_update(a.dpmpp, a, n, idx0, spatial, e);
 }
 
 // one thread: t -= 1 for every sample (and t_prev), generator offset += rng_inc -- the bookkeeping
@@ -750,6 +718,25 @@ extern "C" int mri_q_sample_rng(const float* x0, const uint64_t* rng, const int6
                        stream);
 }
 
+// step_kernel<U> over samples * per_sample elements; z from Philox when rng is set (only DDPM
+// takes z, so only DdpmUpdate is instantiated with RNG)
+template <class U>
+static int step_launch(const char* who, const U& u, const float* x, const void* eps, int ldc,
+                       int channels, const float* noise, const uint64_t* rng, float* x0_prev,
+                       float* out, int samples, int64_t per_sample, void* stream) {
+  const long long numel = (long long)samples * per_sample;
+  int rc = device_props();
+  if (rc) return rc;
+  const AtenGrid g = aten_grid(numel);
+  if (rng != nullptr)
+    step_kernel<U, U::kNoise><<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
+        u, x, eps, ldc, channels, nullptr, rng, x0_prev, out, per_sample, numel, g.Tt, g.n_iter);
+  else
+    step_kernel<U, false><<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
+        u, x, eps, ldc, channels, noise, nullptr, x0_prev, out, per_sample, numel, g.Tt, g.n_iter);
+  return check_launch(who);
+}
+
 static int ddpm_step_impl(const float* x, const void* eps, int ldc, int channels, const float* noise,
                           const uint64_t* rng, const int64_t* t, const float* betas,
                           const float* sqrt_1mac, const float* sqrt_recip_alphas,
@@ -758,18 +745,8 @@ static int ddpm_step_impl(const float* x, const void* eps, int ldc, int channels
   if (samples < 1 || per_sample < 1) return set_error(-2, "mri_ddpm_step: empty input");
   if (ldc != 0 && (channels < 1 || per_sample % channels != 0))
     return set_error(-2, "mri_ddpm_step: per_sample must be channels * spatial");
-  const long long numel = (long long)samples * per_sample;
-  int rc = device_props();
-  if (rc) return rc;
-  const AtenGrid g = aten_grid(numel);
-  StepTables T{t, betas, sqrt_1mac, sqrt_recip_alphas, post_var};
-  if (rng != nullptr)
-    ddpm_step_kernel<true><<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
-        x, eps, ldc, channels, nullptr, rng, T, out, per_sample, numel, g.Tt, g.n_iter);
-  else
-    ddpm_step_kernel<false><<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
-        x, eps, ldc, channels, noise, nullptr, T, out, per_sample, numel, g.Tt, g.n_iter);
-  return check_launch("ddpm_step_kernel");
+  return step_launch("mri_ddpm_step", DdpmUpdate{t, betas, sqrt_1mac, sqrt_recip_alphas, post_var},
+                     x, eps, ldc, channels, noise, rng, nullptr, out, samples, per_sample, stream);
 }
 
 extern "C" int mri_ddpm_step(const float* x, const void* eps, int eps_nhwc_ldc, int channels,
@@ -798,14 +775,8 @@ extern "C" int mri_ddim_step(const float* x, const void* eps, int eps_nhwc_ldc, 
   if (samples < 1 || per_sample < 1) return set_error(-2, "mri_ddim_step: empty input");
   if (eps_nhwc_ldc != 0 && (channels < 1 || per_sample % channels != 0))
     return set_error(-2, "mri_ddim_step: per_sample must be channels * spatial");
-  const long long numel = (long long)samples * per_sample;
-  int rc = device_props();
-  if (rc) return rc;
-  const AtenGrid g = aten_grid(numel);
-  ddim_step_kernel<<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
-      x, eps, eps_nhwc_ldc, channels, t, t_prev, alphas_cumprod, out, per_sample, numel, g.Tt,
-      g.n_iter);
-  return check_launch("ddim_step_kernel");
+  return step_launch("mri_ddim_step", DdimUpdate{t, t_prev, alphas_cumprod}, x, eps, eps_nhwc_ldc,
+                     channels, nullptr, nullptr, nullptr, out, samples, per_sample, stream);
 }
 
 extern "C" int mri_dpmpp_step(const float* x, const void* eps, int eps_nhwc_ldc, int channels,
@@ -816,13 +787,8 @@ extern "C" int mri_dpmpp_step(const float* x, const void* eps, int eps_nhwc_ldc,
     return set_error(-2, "mri_dpmpp_step: null x / eps / x0_prev / coef / out");
   if (eps_nhwc_ldc != 0 && (channels < 1 || per_sample % channels != 0 || eps_nhwc_ldc < channels))
     return set_error(-2, "mri_dpmpp_step: per_sample must be channels * spatial, ldc >= channels");
-  const long long numel = (long long)samples * per_sample;
-  int rc = device_props();
-  if (rc) return rc;
-  const AtenGrid g = aten_grid(numel);
-  dpmpp_step_kernel<<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
-      x, eps, eps_nhwc_ldc, channels, x0_prev, coef, k, out, per_sample, numel, g.Tt, g.n_iter);
-  return check_launch("dpmpp_step_kernel");
+  return step_launch("mri_dpmpp_step", DpmppUpdate{coef, k}, x, eps, eps_nhwc_ldc, channels, nullptr,
+                     nullptr, x0_prev, out, samples, per_sample, stream);
 }
 
 extern "C" int mri_step_table_advance(int64_t* t, int n, int64_t* k, const int64_t* ts, int rows,
@@ -929,16 +895,10 @@ extern "C" int mri_tap_gather_step(const void* y, const float* bias, int samples
   a.x = x;
   a.eps_out = reinterpret_cast<__nv_bfloat16*>(eps_out);
   a.rng = rng;
-  a.t = t;
-  a.t_prev = t_prev;
-  a.betas = betas;
-  a.sqrt_1mac = sqrt_1mac;
-  a.sqrt_recip_alphas = sqrt_recip_alphas;
-  a.post_var = post_var;
-  a.alphas_cumprod = alphas_cumprod;
   a.x0_prev = x0_prev;
-  a.coef = coef;
-  a.k = k;
+  a.ddpm = DdpmUpdate{t, betas, sqrt_1mac, sqrt_recip_alphas, post_var};
+  a.ddim = DdimUpdate{t, t_prev, alphas_cumprod};
+  a.dpmpp = DpmppUpdate{coef, k};
   a.samples = samples; a.D = D; a.H = H; a.W = W; a.ndim = ndim; a.cout = cout; a.ldy = ldy; a.ldo = ldo;
   a.mode = mode;
   a.TD = ndim == 3 ? 4 : 1;
