@@ -307,6 +307,16 @@ int mri_inpaint_merge(float* x, const float* known, const uint8_t* mask, const f
                       const uint64_t* rng, uint64_t rng_skip, const int64_t* t, int64_t t_delta,
                       const float* sqrt_ac, const float* sqrt_1mac, int samples, int64_t per_sample,
                       void* stream);
+/* mri_repaint_undo: RePaint's undo step (not in the reference), in place per element with
+ * l = t[n] in [-1, T - 2] per sample:
+ *     x = sqrt(alphas[l + 1])*x + sqrt(betas[l + 1])*z
+ * fp32, two multiplies and one add rounded to nearest (no FMA contraction), sqrt rounded to
+ * nearest: bit-identical to eager alphas[l + 1].sqrt() * x + betas[l + 1].sqrt() * z.  z as for
+ * mri_inpaint_merge: `noise`, or with rng the Philox draw at offset rng[1] + rng_skip.  Exactly
+ * one of noise / rng. */
+int mri_repaint_undo(float* x, const float* noise, const uint64_t* rng, uint64_t rng_skip,
+                     const int64_t* t, const float* alphas, const float* betas, int samples,
+                     int64_t per_sample, void* stream);
 int mri_minsnr_loss(const float* pred, const float* noise, const int64_t* t, const float* snr,
                     float gamma, float* per_sample_out, float* loss_out, int samples,
                     int64_t per_sample, void* stream);

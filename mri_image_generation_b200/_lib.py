@@ -148,6 +148,7 @@ SIGNATURES = {
     "mri_dpmpp_step": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _i, _i64, _vp]),
     "mri_step_table_advance": (_i, [_vp, _i, _vp, _vp, _i, _vp]),
     "mri_inpaint_merge": (_i, [_vp, _vp, _vp, _vp, _vp, _u64, _vp, _i64, _vp, _vp, _i, _i64, _vp]),
+    "mri_repaint_undo": (_i, [_vp, _vp, _vp, _u64, _vp, _vp, _vp, _i, _i64, _vp]),
     "mri_minsnr_loss": (_i, [_vp, _vp, _vp, _vp, _f, _vp, _vp, _i, _i64, _vp]),
     "mri_add_i64": (_i, [_vp, _i, _i64, _vp]),
     "mri_randn_offset_increment": (_i, [_i64, C.POINTER(C.c_uint64)]),

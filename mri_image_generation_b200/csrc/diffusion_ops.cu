@@ -190,17 +190,33 @@ randn_kernel(float* out, long long numel, long long Tt, int n_iter, const uint64
       [&](long long e, float z) { out[e] = z; });
 }
 
-// x_t = sqrt_ac[t] * x0 + sqrt_1mac[t] * z ; z optionally written out (the loss needs it).
+// The forward-noising coefficients (a, b) of out = a * x + b * z at per-sample timestep t:
+//   q_sample:     x_0 -> x_t,      (sqrt_ac[t], sqrt_1mac[t])
+//   RePaint undo: x_l -> x_{l+1},  (sqrt(alphas[l + 1]), sqrt(betas[l + 1])), l >= -1
+struct QSampleCoef {
+  const float *sqrt_ac, *sqrt_1mac;
+  __device__ __forceinline__ float2 operator()(int64_t t) const {
+    return make_float2(__ldg(sqrt_ac + t), __ldg(sqrt_1mac + t));
+  }
+};
+struct UndoCoef {
+  const float *alphas, *betas;
+  __device__ __forceinline__ float2 operator()(int64_t l) const {
+    return make_float2(__fsqrt_rn(__ldg(alphas + l + 1)), __fsqrt_rn(__ldg(betas + l + 1)));
+  }
+};
+
+// out = a * x0 + b * z with (a, b) = coef(t[n]) ; z optionally written out (the loss needs it).
 // x0 / out may alias (no __restrict__).
-template <bool RNG>
+template <class Coef, bool RNG>
 __global__ void __launch_bounds__(256)
-q_sample_kernel(const float* x0, const float* noise, const uint64_t* rng, const int64_t* t,
-                const float* sqrt_ac, const float* sqrt_1mac, float* out, float* noise_out,
+q_sample_kernel(const Coef coef, const float* x0, const float* noise, const uint64_t* rng,
+                uint64_t ctr_skip, const int64_t* t, float* out, float* noise_out,
                 long long per_sample, long long numel, long long Tt, int n_iter) {
   const bool al = aligned16(x0) && aligned16(out) && (noise_out == nullptr || aligned16(noise_out));
   auto one = [&](long long e, float z) {
-    const int64_t ts = t[e / per_sample];
-    out[e] = __fadd_rn(__fmul_rn(__ldg(sqrt_ac + ts), x0[e]), __fmul_rn(__ldg(sqrt_1mac + ts), z));
+    const float2 c = coef(t[e / per_sample]);
+    out[e] = __fadd_rn(__fmul_rn(c.x, x0[e]), __fmul_rn(c.y, z));
     if (noise_out != nullptr) noise_out[e] = z;
   };
   element_loop<RNG>(numel, Tt, n_iter, rng, noise,
@@ -211,16 +227,15 @@ q_sample_kernel(const float* x0, const float* noise, const uint64_t* rng, const 
           for (int m = 0; m < 4; ++m) one(e0 + m, z[m]);
           return;
         }
-        const int64_t ts = t[n];
-        const float a = __ldg(sqrt_ac + ts), b = __ldg(sqrt_1mac + ts);
+        const float2 c = coef(t[n]);
         float xv[4], o[4];
         load4(x0 + e0, al, xv);
 #pragma unroll
-        for (int m = 0; m < 4; ++m) o[m] = __fadd_rn(__fmul_rn(a, xv[m]), __fmul_rn(b, z[m]));
+        for (int m = 0; m < 4; ++m) o[m] = __fadd_rn(__fmul_rn(c.x, xv[m]), __fmul_rn(c.y, z[m]));
         store4(out + e0, al, o);
         if (noise_out != nullptr) store4(noise_out + e0, al, z);
       },
-      one);
+      one, ctr_skip);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -685,21 +700,31 @@ extern "C" int mri_randn(float* out, int64_t numel, const uint64_t* rng, void* s
   return check_launch("randn_kernel");
 }
 
-static int q_sample_impl(const float* x0, const float* noise, const uint64_t* rng, const int64_t* t,
-                         const float* sqrt_ac, const float* sqrt_1mac, float* out, float* noise_out,
-                         int samples, int64_t per_sample, void* stream) {
-  if (samples < 1 || per_sample < 1) return set_error(-2, "mri_q_sample: empty input");
+// q_sample_kernel<Coef> over samples * per_sample elements; z from Philox (rng_skip past the
+// generator offset) when rng is set, else from `noise`
+template <class Coef>
+static int noise_launch(const char* who, const Coef& coef, const float* x0, const float* noise,
+                        const uint64_t* rng, uint64_t rng_skip, const int64_t* t, float* out,
+                        float* noise_out, int samples, int64_t per_sample, void* stream) {
   const long long numel = (long long)samples * per_sample;
   int rc = device_props();
   if (rc) return rc;
   const AtenGrid g = aten_grid(numel);
   if (rng != nullptr)
-    q_sample_kernel<true><<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
-        x0, nullptr, rng, t, sqrt_ac, sqrt_1mac, out, noise_out, per_sample, numel, g.Tt, g.n_iter);
+    q_sample_kernel<Coef, true><<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
+        coef, x0, nullptr, rng, rng_skip / 4, t, out, noise_out, per_sample, numel, g.Tt, g.n_iter);
   else
-    q_sample_kernel<false><<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
-        x0, noise, nullptr, t, sqrt_ac, sqrt_1mac, out, noise_out, per_sample, numel, g.Tt, g.n_iter);
-  return check_launch("q_sample_kernel");
+    q_sample_kernel<Coef, false><<<my_blocks(g), 256, 0, (cudaStream_t)stream>>>(
+        coef, x0, noise, nullptr, 0, t, out, noise_out, per_sample, numel, g.Tt, g.n_iter);
+  return check_launch(who);
+}
+
+static int q_sample_impl(const float* x0, const float* noise, const uint64_t* rng, const int64_t* t,
+                         const float* sqrt_ac, const float* sqrt_1mac, float* out, float* noise_out,
+                         int samples, int64_t per_sample, void* stream) {
+  if (samples < 1 || per_sample < 1) return set_error(-2, "mri_q_sample: empty input");
+  return noise_launch("q_sample_kernel", QSampleCoef{sqrt_ac, sqrt_1mac}, x0, noise, rng, 0, t, out,
+                      noise_out, samples, per_sample, stream);
 }
 
 extern "C" int mri_q_sample(const float* x0, const float* noise, const int64_t* t,
@@ -825,6 +850,19 @@ extern "C" int mri_inpaint_merge(float* x, const float* known, const uint8_t* ma
         x, known, mask, noise, nullptr, 0, t, t_delta, sqrt_ac, sqrt_1mac, per_sample, numel, g.Tt,
         g.n_iter);
   return check_launch("inpaint_merge_kernel");
+}
+
+extern "C" int mri_repaint_undo(float* x, const float* noise, const uint64_t* rng, uint64_t rng_skip,
+                                const int64_t* t, const float* alphas, const float* betas,
+                                int samples, int64_t per_sample, void* stream) {
+  if (samples < 1 || per_sample < 1) return set_error(-2, "mri_repaint_undo: empty input");
+  if (x == nullptr || t == nullptr || alphas == nullptr || betas == nullptr)
+    return set_error(-2, "mri_repaint_undo: null x / t / schedule table");
+  if ((noise == nullptr) == (rng == nullptr))
+    return set_error(-2, "mri_repaint_undo: exactly one of noise / rng");
+  if (rng_skip % 4 != 0) return set_error(-2, "mri_repaint_undo: rng_skip must be a multiple of 4");
+  return noise_launch("q_sample_kernel<UndoCoef>", UndoCoef{alphas, betas}, x, noise, rng, rng_skip, t, x,
+                      nullptr, samples, per_sample, stream);
 }
 
 extern "C" int mri_rng_seed(uint64_t* rng, uint64_t seed, uint64_t offset, void* stream) {

@@ -6,6 +6,7 @@ model arguments (z_pos, context) and the loss; everything that touches the GPU i
     mri_ddpm_step, mri_ddim_step), bit-exact w.r.t. the reference's eager association order;
     DPM-Solver++(2M) (not in the reference): mri_dpmpp_step over a host-built coefficient table;
     inpainting (not in the reference): mri_inpaint_merge after each update of either sampler;
+    RePaint's resampling (not in the reference): mri_repaint_undo between the inpainting steps;
   - the reverse loop: when the denoiser is one of this package's UNets, one CUDA graph holds a
     whole reverse step (time embedding, UNet, fused update with the noise drawn INSIDE the
     kernel, t -= 1) and is replayed T times.  The kernels draw Philox4x32-10 + Box-Muller
@@ -229,11 +230,19 @@ class DiffusionBase(nn.Module):
             bufs["noise"] = torch.zeros_like(prog.x_in)
         return bufs
 
-    def _inpaint_ddpm(self, img, inpaint, prog, eps_fn: Callable) -> torch.Tensor:
+    def _repaint_levels(self, jump_length, jump_n_sample) -> Optional[list]:
+        """schedules.repaint_levels for this schedule (ValueError on bad arguments), or None when
+        it has no undo step (jump_n_sample = 1 or jump_length >= T): plain replacement."""
+        levels = schedules.repaint_levels(self.timesteps, jump_length, jump_n_sample)
+        return levels if len(levels) > self.timesteps + 1 else None
+
+    def _inpaint_ddpm(self, img, inpaint, prog, eps_fn: Callable, levels=None) -> torch.Tensor:
         """Ancestral sampling from x_T = img over every timestep with the kept region replaced after
         each update by q_sample(known, i - 1, noise=randn_like(x)) (known itself after i = 0).
-        prog / eps_fn as for _sample_dpmpp."""
+        prog / eps_fn as for _sample_dpmpp.  levels: RePaint's resampling (_inpaint_repaint)."""
         _require_cuda(img, "inpaint")
+        if levels is not None:
+            return self._inpaint_repaint(img, inpaint, prog, eps_fn, levels)
         T = self.timesteps
         if prog is not None:
             return self._reverse_loop(prog, img.float(), T - 1, T, "ddpm", inpaint=inpaint)
@@ -243,11 +252,42 @@ class DiffusionBase(nn.Module):
             rng = self._rng(dev)
             inc = ops.randn_offset_increment(x.numel())
             for i in reversed(range(T)):
-                t = torch.full((x.shape[0],), i, device=dev, dtype=torch.long)
-                x = self._p_update(x, t, eps_fn(x, t))
+                x = self._inpaint_step(x, i, inpaint, eps_fn, rng, inc)
+        return x
+
+    def _inpaint_step(self, x, i, inpaint, eps_fn, rng, inc) -> torch.Tensor:
+        """One eager DDPM inpainting step at t = i: update, then the kept region becomes
+        q_sample(known, i - 1, noise=randn_like(x)) (known itself at i = 0)."""
+        t = torch.full((x.shape[0],), i, device=x.device, dtype=torch.long)
+        x = self._p_update(x, t, eps_fn(x, t))
+        off = rng.load()
+        ops.inpaint_merge(x, inpaint[0], inpaint[1], t, -1, self.sqrt_alphas_cumprod,
+                          self.sqrt_one_minus_alphas_cumprod, rng=rng)
+        rng.commit(off + inc)
+        return x
+
+    def _inpaint_repaint(self, img, inpaint, prog, eps_fn: Callable, levels) -> torch.Tensor:
+        """RePaint: _inpaint_ddpm's steps walked along `levels` (schedules.repaint_levels).  A move
+        l -> l - 1 is the inpainting step at t = l; a move l -> l + 1 re-noises the merged state by
+        one step, x = sqrt(alphas[l + 1]) x + sqrt(betas[l + 1]) z with z = randn_like(x), so that
+        the next steps reconcile the regenerated region with the kept one.  The generator advances
+        by (1 + 2 n_reverse + n_undo) draws, x_T included."""
+        n_reverse = sum(1 for a, b in zip(levels, levels[1:]) if b < a)
+        if prog is not None:
+            return self._reverse_loop(prog, img.float(), levels[0], n_reverse, "ddpm",
+                                      inpaint=inpaint, levels=levels)
+        dev = img.device
+        x = img.float().contiguous()
+        with torch.cuda.device(dev):
+            rng = self._rng(dev)
+            inc = ops.randn_offset_increment(x.numel())
+            for lv, nxt in zip(levels, levels[1:]):
+                if nxt < lv:
+                    x = self._inpaint_step(x, lv, inpaint, eps_fn, rng, inc)
+                    continue
+                t = torch.full((x.shape[0],), lv, device=dev, dtype=torch.long)
                 off = rng.load()
-                ops.inpaint_merge(x, inpaint[0], inpaint[1], t, -1, self.sqrt_alphas_cumprod,
-                                  self.sqrt_one_minus_alphas_cumprod, rng=rng)
+                ops.repaint_undo(x, t, self.alphas, self.betas, rng=rng)
                 rng.commit(off + inc)
         return x
 
@@ -277,7 +317,7 @@ class DiffusionBase(nn.Module):
     def _schedule_ptrs(self) -> Tuple[int, ...]:
         return tuple(getattr(self, n).data_ptr() for n in
                      ("betas", "sqrt_one_minus_alphas_cumprod", "sqrt_recip_alphas",
-                      "posterior_variance", "alphas_cumprod", "sqrt_alphas_cumprod"))
+                      "posterior_variance", "alphas_cumprod", "sqrt_alphas_cumprod", "alphas"))
 
     def _step_graph(self, prog, mode: str, one_step, tprev):
         """The CUDA graph of one reverse step on `prog`.  The graph lives ON the program (it
@@ -319,19 +359,22 @@ class DiffusionBase(nn.Module):
 
     def _reverse_loop(self, prog, img: torch.Tensor, start_t: int, n_steps: int, mode: str,
                       use_graph: bool = True, t_vec: Optional[torch.Tensor] = None,
-                      stride: int = 1, table=None, inpaint=None) -> torch.Tensor:
+                      stride: int = 1, table=None, inpaint=None, levels=None) -> torch.Tensor:
         """Run n_steps reverse steps (i = start_t, start_t - stride, ...) on `prog` (a UNetProgram
         whose x_in is the sampler state).  mode: 'ddpm' | 'ddim' (t_prev = max(t - stride, 0)) |
         'dpmpp' (table = (ts, coef) of schedules.dpmpp_2m_table, n_steps = its rows).
         inpaint: (known, mask) of _inpaint_inputs, 'ddpm' or 'dpmpp' only: mri_inpaint_merge
-        after every update, on a step graph of its own ('ddpm+inpaint' / 'dpmpp+inpaint')."""
+        after every update, on a step graph of its own ('ddpm+inpaint' / 'dpmpp+inpaint').
+        levels: RePaint's walk (schedules.repaint_levels), 'ddpm' with inpaint only: its n_steps
+        reverse steps replay 'ddpm+inpaint', its undo steps a graph of their own
+        ('repaint-undo': mri_repaint_undo at t, then t += 1), in the walk's order."""
         dev = img.device
         with torch.cuda.device(dev):
             return self._reverse_loop_on(prog, img, start_t, n_steps, mode, use_graph, t_vec, stride,
-                                         table, inpaint)
+                                         table, inpaint, levels)
 
     def _reverse_loop_on(self, prog, img, start_t, n_steps, mode, use_graph, t_vec, stride,
-                         table=None, inpaint=None):
+                         table=None, inpaint=None, levels=None):
         dev = img.device
         if prog.params_changed():
             prog.do_refresh()
@@ -351,6 +394,8 @@ class DiffusionBase(nn.Module):
                 raise _lib.MriError("inpainting runs on the full DDPM or the DPM-Solver++ loop")
             inp = self._inpaint_buffers(prog, mode == "dpmpp")
             gkey += "+inpaint"
+        if levels is not None and (inp is None or mode != "ddpm"):
+            raise _lib.MriError("RePaint resampling runs on the DDPM inpainting loop")
         # DDPM inpainting draws a second randn_like(x) per step (the merge's noise)
         adv = 2 * inc if inp is not None else inc
 
@@ -411,9 +456,17 @@ class DiffusionBase(nn.Module):
                               prog.x_in, eps_nhwc_ldc=ldc, channels=C)
                 ops.step_advance(prog.t_in, -stride, t_prev=tprev)
 
-        graph = None
-        if use_graph and (n_steps >= 3 or t_vec is not None):
+        def undo_step():
+            ops.repaint_undo(prog.x_in, prog.t_in, self.alphas, self.betas, rng=rng)
+            ops.step_advance(prog.t_in, 1, rng=rng, rng_increment=inc)
+
+        graph = undo = None
+        # the capture's warm-up runs the undo at t = 1, which reads alphas[2]
+        walk_ok = levels is None or self.timesteps >= 3
+        if use_graph and (n_steps >= 3 or t_vec is not None) and walk_ok:
             graph = self._step_graph(prog, gkey, one_step, tprev)
+            if levels is not None:   # both captured before x_in / t_in are loaded below
+                undo = self._step_graph(prog, "repaint-undo", undo_step, tprev)
         prog.x_in.copy_(img)
         if t_vec is not None:  # per-sample timesteps (p_sample called directly)
             prog.t_in.copy_(t_vec.to(dev).long())
@@ -434,12 +487,24 @@ class DiffusionBase(nn.Module):
             if mode == "dpmpp":
                 inp["noise"].copy_(img)
         off = rng.load() if mode == "ddpm" else 0
-        for _ in range(n_steps):
-            if graph is not None:
-                graph.replay()
-            else:
-                one_step()
+        n_undo = 0
+        if levels is None:
+            for _ in range(n_steps):
+                if graph is not None:
+                    graph.replay()
+                else:
+                    one_step()
+        else:   # no host synchronisation inside the walk
+            for a, b in zip(levels, levels[1:]):
+                if b < a:
+                    step, g = one_step, graph
+                else:
+                    step, g, n_undo = undo_step, undo, n_undo + 1
+                if g is not None:
+                    g.replay()
+                else:
+                    step()
         if mode == "ddpm":  # z = randn_like(x) is drawn at every step, t = 0 included
-            rng.commit(off + n_steps * adv)
+            rng.commit(off + n_steps * adv + n_undo * inc)
         assert per_sample == prog.x_in[0].numel()
         return prog.x_in.clone()

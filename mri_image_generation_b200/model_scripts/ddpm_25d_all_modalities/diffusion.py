@@ -82,19 +82,21 @@ class GaussianDiffusion(_GD2):
                                   lambda x, t: self.model(x, t, z_pos, context=context))
 
     @torch.no_grad()
-    def inpaint(self, x_known, mask, z_pos=0.5, context=None):
+    def inpaint(self, x_known, mask, z_pos=0.5, context=None, jump_length=10, jump_n_sample=1):
         """Inpainting by replacement with the full DDPM sampler (not in the reference), e.g.
         missing-modality imputation: x_known (B, 4, H, W) holds t1, t1ce, t2, flair and a mask of
         shape (1, 4, 1, 1) set only at the missing channel regenerates that modality.  See the 2D
-        class's inpaint() for the method."""
+        class's inpaint() for the method and the 3D class's for RePaint's resampling
+        (jump_length, jump_n_sample)."""
         known, m = self._inpaint_inputs(x_known, mask, 4)
+        levels = self._repaint_levels(jump_length, jump_n_sample)
         device = self.betas.device
         if context is not None:
             context = context.to(device)
         img, prog = self._inpaint_start(known, z_pos, context)
         z_pos = self._z_tensor(z_pos, img.shape[0], device)
         return self._inpaint_ddpm(img, (known.to(device), m.to(device)), prog,
-                                  lambda x, t: self.model(x, t, z_pos, context=context))
+                                  lambda x, t: self.model(x, t, z_pos, context=context), levels)
 
     @torch.no_grad()
     def inpaint_dpmpp(self, x_known, mask, z_pos=0.5, context=None, num_steps=20):

@@ -105,16 +105,19 @@ class GaussianDiffusion(DiffusionBase):
         return self._sample_dpmpp(img, table, prog, lambda x, t: self.model(x, t, z_pos))
 
     @torch.no_grad()
-    def inpaint(self, x_known, mask, z_pos=0.5):
+    def inpaint(self, x_known, mask, z_pos=0.5, jump_length=10, jump_n_sample=1):
         """Inpainting by replacement with the full DDPM sampler (not in the reference).  x_known:
         (B, channels, H, W); mask broadcasts to it, True / 1 = regenerate, False / 0 = keep.  x_T
         is drawn as sample() draws it; after the update at every step i the kept region is set to
-        q_sample(x_known, i - 1, noise=randn_like(x)) (x_known itself after i = 0)."""
+        q_sample(x_known, i - 1, noise=randn_like(x)) (x_known itself after i = 0).
+        jump_n_sample > 1 adds RePaint's resampling with jumps of jump_length steps: see the 3D
+        class's inpaint()."""
         known, m = self._inpaint_inputs(x_known, mask, 4)
+        levels = self._repaint_levels(jump_length, jump_n_sample)
         img, prog = self._inpaint_start(known, z_pos)
         inp = (known.to(img.device), m.to(img.device))
         z_pos = self._z_tensor(z_pos, img.shape[0], img.device)
-        return self._inpaint_ddpm(img, inp, prog, lambda x, t: self.model(x, t, z_pos))
+        return self._inpaint_ddpm(img, inp, prog, lambda x, t: self.model(x, t, z_pos), levels)
 
     @torch.no_grad()
     def inpaint_dpmpp(self, x_known, mask, z_pos=0.5, num_steps=20):

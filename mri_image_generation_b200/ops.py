@@ -270,6 +270,22 @@ def inpaint_merge(x, known, mask, t, t_delta: int, sqrt_ac, sqrt_1mac, noise=Non
                "mri_inpaint_merge")
 
 
+def repaint_undo(x, t, alphas, betas, noise=None, rng: Optional[DeviceRng] = None,
+                 rng_skip: int = 0) -> None:
+    """RePaint's undo step in place: x = sqrt(alphas[l + 1]) * x + sqrt(betas[l + 1]) * z with
+    l = t per sample (device int64 [samples], -1 <= l <= T - 2).  z: `noise`, or with rng the
+    torch.randn_like drawn rng_skip past the generator offset."""
+    _chk_contig(x, noise)
+    assert x.dtype == alphas.dtype == betas.dtype == torch.float32 and t.dtype == torch.int64
+    assert noise is None or (noise.dtype == torch.float32 and noise.numel() == x.numel())
+    n = x.shape[0]
+    _lib.check(_lib.load().mri_repaint_undo(_p(x), _p(noise),
+                                            _p(rng.state) if rng is not None else None,
+                                            int(rng_skip), _p(t), _p(alphas), _p(betas), n,
+                                            x.numel() // n, _s()),
+               "mri_repaint_undo")
+
+
 def step_advance(t: torch.Tensor, delta: int, t_prev=None, rng: Optional[DeviceRng] = None,
                  rng_increment: int = 0) -> None:
     _lib.check(_lib.load().mri_step_advance(_p(t), _p(t_prev), t.numel(), delta,

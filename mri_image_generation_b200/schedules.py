@@ -8,6 +8,7 @@ infers `timesteps` from betas.numel()), which tests/test_oracle_golden.py and te
 tests/golden/schedules.pt.
 """
 import math
+import numbers
 from collections import OrderedDict
 
 import torch
@@ -57,6 +58,32 @@ def dpmpp_timesteps(start_t: int, num_steps: int) -> list:
     if not 1 <= M <= s:
         raise ValueError(f"need 1 <= num_steps <= start_t (got num_steps={M}, start_t={s})")
     return [(2 * s * (M - i) + M) // (2 * M) for i in range(M)] + [-1]
+
+
+def repaint_levels(timesteps: int, jump_length: int, jump_n_sample: int) -> list:
+    """The noise levels RePaint's resampling visits, one timestep per training step (the jump rule
+    of diffusers' RePaintScheduler).  Level l means x ~ q_sample(x0, l); -1 means clean.  The list
+    starts at T - 1, ends at -1 and moves by exactly 1: l -> l - 1 is a reverse step at t = l,
+    l -> l + 1 an undo step (one step of forward noising).  After the reverse step at each jump
+    point j in range(0, T - L, L), the sampler jumps back up L levels, r - 1 times in all, and
+    each time walks down again: T + (r - 1) L P reverse and (r - 1) L P undo steps,
+    P = len(range(0, T - L, L)).  r = 1, or L >= T, gives [T - 1, ..., 0, -1]."""
+    T, L, r = timesteps, jump_length, jump_n_sample
+    for name, v in (("timesteps", T), ("jump_length", L), ("jump_n_sample", r)):
+        if isinstance(v, bool) or not isinstance(v, numbers.Integral) or v < 1:
+            raise ValueError(f"{name} must be an integer >= 1 (got {v!r})")
+    T, L, r = int(T), int(L), int(r)
+    jumps = {j: r - 1 for j in range(0, T - L, L)}
+    levels, t = [T - 1], T - 1
+    while t >= 0:
+        j = t
+        t -= 1
+        levels.append(t)
+        if jumps.get(j, 0) > 0:
+            jumps[j] -= 1
+            levels.extend(range(t + 1, t + L + 1))
+            t += L
+    return levels
 
 
 def dpmpp_2m_table(alphas_cumprod: torch.Tensor, timesteps):

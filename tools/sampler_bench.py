@@ -1,8 +1,10 @@
 #!/usr/bin/env python
 """Cost of the three samplers (GPU only): ms per reverse step of the replayed step graph for
 DDPM (ancestral), strided DDIM and DPM-Solver++(2M), the DDPM and DPM-Solver++ inpainting steps
-(the same step plus mri_inpaint_merge, every element kept: the merge's worst case), and end to end for
-sample_dpmpp(num_steps=20).
+(the same step plus mri_inpaint_merge, every element kept: the merge's worst case), ms per replay of
+RePaint's undo graph (mri_repaint_undo + step_advance), and end to end for
+sample_dpmpp(num_steps=20) and for inpaint() against inpaint(jump_length=10, jump_n_sample=2) at
+T = 1000 (1000 against 1990 UNet calls; half of each sample regenerated, one run each).
 
   cfg4  ddpm_3d_ldm         UNet3DModelWithAttention(3, base 128, mults 1-2-4) B=16 3x40x48x40
   cfg2  slice_cond_2d_ddpm  UNet(1, base 64, mults 1-2-4-8)                   B=64 1x240x240
@@ -76,14 +78,18 @@ def step_times(diff, prog, x, steps, reps, warm=3):
     diff._reverse_loop(prog, x, T - 1, 3, "ddpm", inpaint=(known, mask))
     diff._reverse_loop(prog, x, T - 1, 3, "dpmpp", table=diff._dpmpp_table(T - 1, steps),
                        inpaint=(known, mask))
+    # three reverse steps and one undo: captures the undo graph
+    diff._reverse_loop(prog, x, T - 1, 3, "ddpm", inpaint=(known, mask),
+                       levels=[T - 1, T - 2, T - 1, T - 2, T - 3])
     g = {k: prog._step_graphs[k][2] for k in ("ddpm", f"ddim/{DDIM_STRIDE}", "dpmpp", "ddpm+inpaint",
-                                              "dpmpp+inpaint")}
+                                              "dpmpp+inpaint", "repaint-undo")}
     tprev, dpm = prog._tprev_buf, prog._dpmpp_bufs
     n_ddim = min(steps, (T - 1) // DDIM_STRIDE)   # t stays >= 0 over the timed replays
 
-    def reset():
+    def reset(key):
         prog.x_in.copy_(x)
-        prog.t_in.fill_(T - 1)
+        # the undo steps t up by one per replay and reads alphas[t + 1]: start low enough
+        prog.t_in.fill_(T - 2 - steps if key == "repaint-undo" else T - 1)
         tprev.fill_(T - 1 - DDIM_STRIDE)
         dpm["k"].zero_()
         diff._rng(x.device).load()
@@ -93,14 +99,15 @@ def step_times(diff, prog, x, steps, reps, warm=3):
             g[key].replay()
 
     plan = {"ddpm": ("ddpm", steps), "ddim": (f"ddim/{DDIM_STRIDE}", n_ddim), "dpmpp": ("dpmpp", steps),
-            "ddpm+inpaint": ("ddpm+inpaint", steps), "dpmpp+inpaint": ("dpmpp+inpaint", steps)}
+            "ddpm+inpaint": ("ddpm+inpaint", steps), "dpmpp+inpaint": ("dpmpp+inpaint", steps),
+            "repaint-undo": ("repaint-undo", steps)}
     for name, (key, n) in plan.items():
-        reset()
+        reset(key)
         replays(key, min(warm, n))
     out = {k: [] for k in plan}
     for _ in range(reps):
         for name, (key, n) in plan.items():
-            reset()
+            reset(key)
             out[name].append(events_ms(lambda: replays(key, n)) / n)
     assert torch.isfinite(prog.x_in).all()
     res = {k: summary(v) for k, v in out.items()}
@@ -116,6 +123,20 @@ def end_to_end(fn, batch, reps):
     s = summary(ms)
     s["per_second"] = batch / (s["median"] / 1e3)
     return s
+
+
+def repaint_end_to_end(inpaint, x):
+    """ms of one inpaint() and one inpaint(jump_length=10, jump_n_sample=2) at T = 1000 on the step
+    graphs step_times captured; half of each sample regenerated."""
+    from mri_image_generation_b200 import schedules
+    lv = schedules.repaint_levels(T, 10, 2)
+    known = torch.randn_like(x)
+    mask = torch.zeros(x.shape, dtype=torch.bool, device=x.device)
+    mask[..., x.shape[-1] // 2:] = True
+    plain = events_ms(lambda: inpaint(known, mask))
+    rp = events_ms(lambda: inpaint(known, mask, jump_length=10, jump_n_sample=2))
+    return {"inpaint_ms": plain, "repaint_10_2_ms": rp, "ratio": rp / plain,
+            "unet_calls": {"inpaint": T, "repaint_10_2": sum(q < p for p, q in zip(lv, lv[1:]))}}
 
 
 def main():
@@ -150,6 +171,7 @@ def main():
         r["sample_dpmpp_ms"] = end_to_end(lambda: d.sample_dpmpp(B, shape, num_steps=args.steps), B, args.reps)
         r["volumes_per_s_dpmpp"] = r["sample_dpmpp_ms"]["per_second"]
         r["volumes_per_s_ddpm_1000_steps_derived"] = B / (T * r["ms_per_step"]["ddpm"]["median"] / 1e3)
+        r["repaint_end_to_end"] = repaint_end_to_end(d.inpaint, x)
         res["cfg4"] = r
         del m, d, x, prog
         torch.cuda.empty_cache()
@@ -168,6 +190,8 @@ def main():
                                           args.reps)
         r["slices_per_s_dpmpp"] = r["sample_dpmpp_ms"]["per_second"]
         r["slices_per_s_ddpm_1000_steps_derived"] = B / (T * r["ms_per_step"]["ddpm"]["median"] / 1e3)
+        r["repaint_end_to_end"] = repaint_end_to_end(
+            lambda known, mask, **kw: d.inpaint(known, mask, z_pos=z, **kw), x)
         res["cfg2"] = r
     line = json.dumps(res)
     print(line)
