@@ -317,6 +317,22 @@ int mri_inpaint_merge(float* x, const float* known, const uint8_t* mask, const f
 int mri_repaint_undo(float* x, const float* noise, const uint64_t* rng, uint64_t rng_skip,
                      const int64_t* t, const float* alphas, const float* betas, int samples,
                      int64_t per_sample, void* stream);
+/* mri_vb_terms: the per-sample sums of one evaluation step of the variational bound (not in the
+ * reference), at l = t[n] in [0, timesteps - 1] per sample (other values add nothing), for
+ * x_t = q_sample(x0, l, z) and the model's eps:
+ *     acc[n][l][0] += sum (eps - z)^2
+ *     l = 0:  acc[n][0][1] += sum -log p(x0 | x_t),  prior[n] += sum x0^2  (prior nullable)
+ * p(x0 | x_t) has the mean of mri_ddpm_step at t = 0 and log-scale 0.5 * post_log_var[0];
+ * decoder 0: discretized Gaussian over 8-bit bins of [-1, 1] (improved-diffusion's
+ * discretized_gaussian_log_likelihood), 1: Gaussian density (continuous data; may be negative).
+ * x0, x_t, z: fp32 [samples][per_sample]; eps as for mri_ddim_step (ldc >= channels).  acc: fp64
+ * [samples][timesteps][2], prior: fp64 [samples], both accumulated into.  fp32 per element, fp64
+ * partial sums with one atomicAdd per block, sample and quantity.  samples <= 65535. */
+int mri_vb_terms(const float* x0, const float* x_t, const void* eps, int eps_nhwc_ldc, int channels,
+                 const float* z, const int64_t* t, const float* betas, const float* sqrt_1mac,
+                 const float* sqrt_recip_alphas, const float* post_var, const float* post_log_var,
+                 int decoder, double* acc, double* prior, int timesteps, int samples,
+                 int64_t per_sample, void* stream);
 int mri_minsnr_loss(const float* pred, const float* noise, const int64_t* t, const float* snr,
                     float gamma, float* per_sample_out, float* loss_out, int samples,
                     int64_t per_sample, void* stream);

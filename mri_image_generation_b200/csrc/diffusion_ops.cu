@@ -430,6 +430,129 @@ inpaint_merge_kernel(float* x, const float* known, const uint8_t* mask, const fl
 }
 
 // ------------------------------------------------------------------------------------------
+// Terms of the variational bound on -log p(x0) for one evaluation step at per-sample timestep
+// t[n], given x0, x_t = q_sample(x0, t, z), z and the predicted eps:
+//   acc[n][t][0] += sum (eps - z)^2                      (L_t = lambda_t times this for t >= 1)
+//   t = 0:  acc[n][0][1] += sum -log p(x0 | x_t),  mean mu = DdpmUpdate::apply at t = 0 (w = 0),
+//           log-scale ls = 0.5 * post_log_var[0];  prior[n] += sum x0^2 (prior optional)
+// Per-element arithmetic is fp32; thread and block partials are fp64, one atomicAdd per block,
+// sample and quantity (order-insensitive to about 1e-16, as the GroupNorm statistics).
+// kDecDiscrete: improved-diffusion's discretized_gaussian_log_likelihood (data in [-1, 1], bins
+// +-1/255, edges at +-0.999, tanh CDF, logs clamped at 1e-12); otherwise the Gaussian density.
+// ------------------------------------------------------------------------------------------
+__device__ __forceinline__ float approx_std_normal_cdf(float x) {
+  const float k = 0.7978845608028654f;   // sqrt(2 / pi)
+  return 0.5f * (1.0f + tanhf(k * (x + 0.044715f * (x * x * x))));
+}
+
+template <bool kDecDiscrete>
+__device__ __forceinline__ float decoder_nll(float x0, float mu, float ls, float inv_std) {
+  const float c = x0 - mu;
+  if constexpr (kDecDiscrete) {
+    const float cdf_plus = approx_std_normal_cdf(inv_std * (c + 1.0f / 255.0f));
+    const float cdf_min = approx_std_normal_cdf(inv_std * (c - 1.0f / 255.0f));
+    const float lp = x0 < -0.999f ? logf(fmaxf(cdf_plus, 1e-12f))
+                     : x0 > 0.999f ? logf(fmaxf(1.0f - cdf_min, 1e-12f))
+                                   : logf(fmaxf(cdf_plus - cdf_min, 1e-12f));
+    return -lp;
+  } else {
+    const float y = c * inv_std;
+    return 0.5f * (y * y) + ls + 0.91893853320467274f;   // + 0.5 log(2 pi)
+  }
+}
+
+// grid (blocks, samples): block (b, n) strides over sample n only
+template <bool kDecDiscrete>
+__global__ void __launch_bounds__(256)
+vb_terms_kernel(const DdpmUpdate u, const float* x0, const float* xt, const void* eps, int ldc,
+                int channels, const float* z, const float* post_log_var, double* acc, double* prior,
+                int T, long long per_sample) {
+  const int n = blockIdx.y;
+  const int64_t ts = u.t[n];
+  if (ts < 0 || ts >= T) return;   // uniform over the block
+  const bool dec = ts == 0;
+  const long long spatial = per_sample / (channels > 0 ? channels : 1);
+  const long long base = (long long)n * per_sample;
+  DdpmUpdate::Coef c{0.f, 0.f, 0.f};
+  float ls = 0.f, inv_std = 0.f;
+  if (dec) {
+    c = u.coef(n);
+    ls = 0.5f * __ldg(post_log_var);
+    inv_std = expf(-ls);
+  }
+  double s_mse = 0.0, s_dec = 0.0, s_x2 = 0.0;
+  auto one = [&](long long j, float e, float zz) {
+    const float d = e - zz;
+    s_mse += (double)(d * d);
+    if (dec) {
+      const float x = x0[base + j];
+      float unused;
+      const float mu = DdpmUpdate::apply(c, xt[base + j], e, 0.f, unused);
+      s_dec += (double)decoder_nll<kDecDiscrete>(x, mu, ls, inv_std);
+      s_x2 += (double)(x * x);
+    }
+  };
+  const long long step = 4LL * gridDim.x * blockDim.x;
+  for (long long j = 4LL * ((long long)blockIdx.x * blockDim.x + threadIdx.x); j < per_sample; j += step) {
+    // four elements inside the sample and, for the channels-last eps, inside one channel
+    if (j + 3 >= per_sample || (ldc != 0 && (j % spatial) + 3 >= spatial)) {
+      for (int m = 0; m < 4 && j + m < per_sample; ++m)
+        one(j + m, load_eps(eps, ldc, spatial, per_sample, n, j + m), z[base + j + m]);
+      continue;
+    }
+    float zv[4], ev[4];
+    load4(z + base + j, aligned16(z + base + j), zv);
+    load_eps4(eps, ldc, spatial, per_sample, n, j,
+              ldc == 0 && aligned16(reinterpret_cast<const float*>(eps) + base + j), ev);
+    if (!dec) {
+#pragma unroll
+      for (int m = 0; m < 4; ++m) {
+        const float d = ev[m] - zv[m];
+        s_mse += (double)(d * d);
+      }
+      continue;
+    }
+    float xv[4], tv[4];
+    load4(x0 + base + j, aligned16(x0 + base + j), xv);
+    load4(xt + base + j, aligned16(xt + base + j), tv);
+#pragma unroll
+    for (int m = 0; m < 4; ++m) {
+      const float d = ev[m] - zv[m];
+      s_mse += (double)(d * d);
+      float unused;
+      const float mu = DdpmUpdate::apply(c, tv[m], ev[m], 0.f, unused);
+      s_dec += (double)decoder_nll<kDecDiscrete>(xv[m], mu, ls, inv_std);
+      s_x2 += (double)(xv[m] * xv[m]);
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    s_mse += __shfl_xor_sync(0xffffffffu, s_mse, o);
+    s_dec += __shfl_xor_sync(0xffffffffu, s_dec, o);
+    s_x2 += __shfl_xor_sync(0xffffffffu, s_x2, o);
+  }
+  __shared__ double part[3][8];
+  const int w = threadIdx.x >> 5;
+  if ((threadIdx.x & 31) == 0) {
+    part[0][w] = s_mse;
+    part[1][w] = s_dec;
+    part[2][w] = s_x2;
+  }
+  __syncthreads();
+  if (threadIdx.x != 0) return;
+  double tot[3] = {0.0, 0.0, 0.0};
+  for (int i = 0; i < (int)(blockDim.x >> 5); ++i)
+#pragma unroll
+    for (int q = 0; q < 3; ++q) tot[q] += part[q][i];
+  double* a = acc + ((long long)n * T + ts) * 2;
+  atomicAdd(a, tot[0]);
+  if (dec) {
+    atomicAdd(a + 1, tot[1]);
+    if (prior != nullptr) atomicAdd(prior + n, tot[2]);
+  }
+}
+
+// ------------------------------------------------------------------------------------------
 // Thin output convolution finished INSIDE the reverse step.  The k^d convolution with 1..4 output
 // channels (out_conv) is computed as one GEMM over all taps, Y[q][tap * cout + co] = W[tap][co] . a[q]
 // (the activation is read once); this kernel sums the shifted taps -- eps[q][co] = bias[co] +
@@ -863,6 +986,36 @@ extern "C" int mri_repaint_undo(float* x, const float* noise, const uint64_t* rn
   if (rng_skip % 4 != 0) return set_error(-2, "mri_repaint_undo: rng_skip must be a multiple of 4");
   return noise_launch("q_sample_kernel<UndoCoef>", UndoCoef{alphas, betas}, x, noise, rng, rng_skip, t, x,
                       nullptr, samples, per_sample, stream);
+}
+
+extern "C" int mri_vb_terms(const float* x0, const float* x_t, const void* eps, int eps_nhwc_ldc,
+                            int channels, const float* z, const int64_t* t, const float* betas,
+                            const float* sqrt_1mac, const float* sqrt_recip_alphas,
+                            const float* post_var, const float* post_log_var, int decoder,
+                            double* acc, double* prior, int timesteps, int samples,
+                            int64_t per_sample, void* stream) {
+  if (samples < 1 || per_sample < 1 || timesteps < 1) return set_error(-2, "mri_vb_terms: empty input");
+  if (samples > 65535) return set_error(-2, "mri_vb_terms: at most 65535 samples");
+  if (x0 == nullptr || x_t == nullptr || eps == nullptr || z == nullptr || t == nullptr ||
+      betas == nullptr || sqrt_1mac == nullptr || sqrt_recip_alphas == nullptr ||
+      post_var == nullptr || post_log_var == nullptr || acc == nullptr)
+    return set_error(-2, "mri_vb_terms: null input / schedule table / acc");
+  if (eps_nhwc_ldc != 0 && (channels < 1 || per_sample % channels != 0 || eps_nhwc_ldc < channels))
+    return set_error(-2, "mri_vb_terms: per_sample must be channels * spatial, ldc >= channels");
+  if (decoder != 0 && decoder != 1)
+    return set_error(-2, "mri_vb_terms: decoder 0 (discretized) / 1 (Gaussian)");
+  long long bx = (per_sample + 4 * 256 - 1) / (4 * 256);
+  const long long cap = (148 * 8 + samples - 1) / samples;
+  if (bx > cap) bx = cap;
+  const dim3 grid((unsigned)bx, (unsigned)samples);
+  const DdpmUpdate u{t, betas, sqrt_1mac, sqrt_recip_alphas, post_var};
+  if (decoder == 0)
+    vb_terms_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(
+        u, x0, x_t, eps, eps_nhwc_ldc, channels, z, post_log_var, acc, prior, timesteps, per_sample);
+  else
+    vb_terms_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(
+        u, x0, x_t, eps, eps_nhwc_ldc, channels, z, post_log_var, acc, prior, timesteps, per_sample);
+  return check_launch("vb_terms_kernel");
 }
 
 extern "C" int mri_rng_seed(uint64_t* rng, uint64_t seed, uint64_t offset, void* stream) {

@@ -7,6 +7,8 @@ model arguments (z_pos, context) and the loss; everything that touches the GPU i
     DPM-Solver++(2M) (not in the reference): mri_dpmpp_step over a host-built coefficient table;
     inpainting (not in the reference): mri_inpaint_merge after each update of either sampler;
     RePaint's resampling (not in the reference): mri_repaint_undo between the inpainting steps;
+    the variational bound in bits per dimension (not in the reference): mri_vb_terms after each
+    evaluation step, on a step graph of its own;
   - the reverse loop: when the denoiser is one of this package's UNets, one CUDA graph holds a
     whole reverse step (time embedding, UNet, fused update with the noise drawn INSIDE the
     kernel, t -= 1) and is replayed T times.  The kernels draw Philox4x32-10 + Box-Muller
@@ -17,6 +19,7 @@ model arguments (z_pos, context) and the loss; everything that touches the GPU i
 """
 from __future__ import annotations
 
+import math
 import os
 import weakref
 from typing import Callable, Dict, Optional, Tuple
@@ -306,6 +309,86 @@ class DiffusionBase(nn.Module):
                 prog.__dict__.get("_step_graphs", {}).pop(key, None)
         return bufs
 
+    # ------------------------------------------------------------------ variational bound
+    def _vb_input(self, x_start, rank: int) -> torch.Tensor:
+        """x_start as the kernels read it (fp32, contiguous).  ValueError on a bad shape, MriError
+        on a CPU tensor; callers check before anything is drawn."""
+        if not torch.is_tensor(x_start) or x_start.dim() != rank or x_start.shape[1] != self.channels:
+            raise ValueError(f"x_start must be a (B, {self.channels}, ...) tensor of rank {rank} "
+                             f"(got {tuple(x_start.shape) if torch.is_tensor(x_start) else type(x_start)})")
+        if x_start.numel() == 0:
+            raise ValueError("x_start is empty")
+        _require_cuda(x_start, "calc_bpd_loop")
+        return x_start.float().contiguous()
+
+    def _vb_buffers(self, prog) -> Dict[str, torch.Tensor]:
+        """The program's evaluation inputs and sums: x0 (copied into on every call, so one captured
+        graph serves every x_start), z, acc (B, T, 2) and prior (B,) in fp64."""
+        bufs = prog.__dict__.setdefault("_vb_bufs", {})
+        T = self.timesteps
+        if "acc" not in bufs or bufs["acc"].shape[1] != T:
+            B, dev = prog.x_in.shape[0], prog.x_in.device
+            bufs.update(x0=torch.zeros_like(prog.x_in), z=torch.zeros_like(prog.x_in),
+                        acc=torch.zeros(B, T, 2, dtype=torch.float64, device=dev),
+                        prior=torch.zeros(B, dtype=torch.float64, device=dev))
+            prog.__dict__.get("_step_graphs", {}).pop("vb", None)   # captured on the old buffers
+        return bufs
+
+    def _vb_loop(self, prog, x0: torch.Tensor, eps_fn: Callable, decoder: int) -> Dict[str, torch.Tensor]:
+        """The variational bound on -log p(x0) in bits per dimension (improved-diffusion's
+        calc_bpd_loop for the fixed-small-variance model).  For t = T - 1 ... 0: z = randn_like(x0),
+        x_t = q_sample(x0, t, z), eps = model(x_t, t), then mri_vb_terms.  prog: a UNetProgram whose
+        conditioning inputs the caller has set (one step graph 'vb' replayed T times), or None: the
+        same sequence eagerly with eps = eps_fn(x_t, t).  The generator advances by T draws."""
+        B, T, N = x0.shape[0], self.timesteps, x0[0].numel()
+        dev = x0.device
+        sched = (self.betas, self.sqrt_one_minus_alphas_cumprod, self.sqrt_recip_alphas,
+                 self.posterior_variance, self.posterior_log_variance_clipped)
+        with torch.cuda.device(dev):
+            rng = self._rng(dev)
+            inc = ops.randn_offset_increment(x0.numel())
+            if prog is None:
+                acc = torch.zeros(B, T, 2, dtype=torch.float64, device=dev)
+                prior = torch.zeros(B, dtype=torch.float64, device=dev)
+                for i in reversed(range(T)):
+                    t = torch.full((B,), i, device=dev, dtype=torch.long)
+                    x_t, z = self._q_sample_draw(x0, t)
+                    ops.vb_terms(x0, x_t, eps_fn(x_t, t).float().contiguous(), z, t, *sched, acc, prior,
+                                 decoder)
+            else:
+                if prog.params_changed():
+                    prog.do_refresh()
+                bufs = self._vb_buffers(prog)
+                tprev = prog.__dict__.setdefault("_tprev_buf", torch.zeros(B, dtype=torch.int64, device=dev))
+
+                def one_step():
+                    ops.q_sample_rng(bufs["x0"], rng, prog.t_in, self.sqrt_alphas_cumprod,
+                                     self.sqrt_one_minus_alphas_cumprod, prog.x_in, bufs["z"])
+                    prog.run()
+                    ops.vb_terms(bufs["x0"], prog.x_in, prog.eps_nhwc, bufs["z"], prog.t_in, *sched,
+                                 bufs["acc"], bufs["prior"], decoder, eps_nhwc_ldc=prog.cout_pad,
+                                 channels=prog.cout)
+                    ops.step_advance(prog.t_in, -1, rng=rng, rng_increment=inc)
+
+                graph = self._step_graph(prog, "vb", one_step, tprev)
+                acc, prior = bufs["acc"], bufs["prior"]
+                bufs["x0"].copy_(x0)
+                acc.zero_()      # after the capture: its warm-up launch accumulated at t = 1
+                prior.zero_()
+                prog.t_in.fill_(T - 1)
+                off = rng.load()
+                for _ in range(T):
+                    graph.replay()
+                rng.commit(off + T * inc)
+            c = schedules.vb_constants(self.betas)
+            lam = c["lam"].to(dev)
+            nats = acc[:, :, 0] * lam
+            nats[:, 0] = acc[:, 0, 1]
+            prior_nats = 0.5 * (N * c["prior_const"] + c["prior_coef"] * prior)
+            scale = 1.0 / (N * math.log(2.0))
+            return {"total_bpd": (prior_nats + nats.sum(1)) * scale, "prior_bpd": prior_nats * scale,
+                    "vb": nats * scale, "mse": acc[:, :, 0] / N}
+
     # ------------------------------------------------------------------ graph-replayed loops
     def _engine_model(self) -> Optional[EngineModule]:
         m = self.model
@@ -317,7 +400,8 @@ class DiffusionBase(nn.Module):
     def _schedule_ptrs(self) -> Tuple[int, ...]:
         return tuple(getattr(self, n).data_ptr() for n in
                      ("betas", "sqrt_one_minus_alphas_cumprod", "sqrt_recip_alphas",
-                      "posterior_variance", "alphas_cumprod", "sqrt_alphas_cumprod", "alphas"))
+                      "posterior_variance", "alphas_cumprod", "sqrt_alphas_cumprod", "alphas",
+                      "posterior_log_variance_clipped"))
 
     def _step_graph(self, prog, mode: str, one_step, tprev):
         """The CUDA graph of one reverse step on `prog`.  The graph lives ON the program (it

@@ -2,7 +2,7 @@
 `context` threaded through, plain MSE loss, no `snr` buffer)."""
 import torch
 
-from ... import schedules
+from ... import ops, schedules
 from ...diffusion_base import DiffusionBase, _require_cuda
 from ..slice_cond_2d_ddpm.diffusion import GaussianDiffusion as _GD2
 
@@ -80,6 +80,17 @@ class GaussianDiffusion(_GD2):
                 prog.ctx_in.copy_(context)
         return self._sample_dpmpp(img, table, prog,
                                   lambda x, t: self.model(x, t, z_pos, context=context))
+
+    @torch.no_grad()
+    def calc_bpd_loop(self, x_start, z_pos, context=None):
+        """The variational bound on -log p(x_start) in bits per dimension, x_start (B, 4, H, W) in
+        [-1, 1] (not in the reference): see the 2D class's calc_bpd_loop()."""
+        x0 = self._vb_input(x_start, 4)
+        z_pos = self._z_tensor(z_pos, x0.shape[0], x0.device)
+        if context is not None:
+            context = context.to(x0.device)
+        return self._vb_loop(self._cond_program(x0, z_pos, context), x0,
+                             lambda x, t: self.model(x, t, z_pos, context=context), ops.VB_DISCRETIZED)
 
     @torch.no_grad()
     def inpaint(self, x_known, mask, z_pos=0.5, context=None, jump_length=10, jump_n_sample=1):

@@ -6,7 +6,7 @@ denoiser is one of this package's UNets.
 """
 import torch
 
-from ... import schedules
+from ... import ops, schedules
 from ...diffusion_base import DiffusionBase, _require_cuda
 
 
@@ -179,6 +179,18 @@ class GaussianDiffusionLatent3D(DiffusionBase):
         img = self._randn(known.shape, self.betas.device)
         return self._inpaint_ddpm(img, (known.to(img.device), m.to(img.device)),
                                   self._program_for(img, cond), self._eps_fn(cond), levels)
+
+    @torch.no_grad()
+    def calc_bpd_loop(self, x_start, cond=None):
+        """The variational bound on -log p(x_start) in bits per dimension (not in the reference;
+        improved-diffusion's calc_bpd_loop for this fixed-small-variance model).  One UNet call per
+        timestep, with z = randn_like(x_start) drawn for t = T - 1 ... 0.  Returns float64 device
+        tensors: total_bpd (B,), prior_bpd (B,), vb (B, T) (the KL terms for t >= 1, the decoder's
+        -log p(x_start | x at t = 0) at t = 0) and mse (B, T) (the mean (eps - z)^2 at each t).
+        Latents are continuous, so the decoder term is a Gaussian density: it can be negative and
+        these numbers do not compare with the pixel-space classes' bits per dimension."""
+        x0 = self._vb_input(x_start, 5)
+        return self._vb_loop(self._program_for(x0, cond), x0, self._eps_fn(cond), ops.VB_GAUSSIAN)
 
     @torch.no_grad()
     def inpaint_dpmpp(self, x_known, mask, num_steps=20, cond=None):

@@ -1,7 +1,7 @@
 """Drop-in for model_scripts/slice_cond_2d_ddpm/diffusion.py (GaussianDiffusion, linear betas)."""
 import torch
 
-from ... import _lib, schedules
+from ... import _lib, ops, schedules
 from ...diffusion_base import DiffusionBase, _require_cuda
 
 
@@ -131,17 +131,34 @@ class GaussianDiffusion(DiffusionBase):
         z_pos = self._z_tensor(z_pos, img.shape[0], img.device)
         return self._sample_dpmpp(img, table, prog, lambda x, t: self.model(x, t, z_pos), inpaint=inp)
 
+    @torch.no_grad()
+    def calc_bpd_loop(self, x_start, z_pos):
+        """The variational bound on -log p(x_start) in bits per dimension (not in the reference;
+        improved-diffusion's calc_bpd_loop for this fixed-small-variance model), for slices in
+        [-1, 1]: the decoder term is the discretized Gaussian over 8-bit bins.  One UNet call per
+        timestep, with z = randn_like(x_start) drawn for t = T - 1 ... 0.  Returns float64 device
+        tensors: total_bpd (B,), prior_bpd (B,), vb (B, T) (the KL terms for t >= 1, the decoder's
+        -log p(x_start | x at t = 0) at t = 0) and mse (B, T) (the mean (eps - z)^2 at each t)."""
+        x0 = self._vb_input(x_start, 4)
+        z_pos = self._z_tensor(z_pos, x0.shape[0], x0.device)
+        return self._vb_loop(self._cond_program(x0, z_pos), x0, lambda x, t: self.model(x, t, z_pos),
+                             ops.VB_DISCRETIZED)
+
     def _inpaint_start(self, known, z_pos, context=None):
         """x_T drawn as sample() draws it, and the program with its conditioning inputs set (None
         for a model that is not one of this package's UNets)."""
-        device = self.betas.device
-        img = self._randn(known.shape, device)
+        img = self._randn(known.shape, self.betas.device)
+        return img, self._cond_program(known, z_pos, context)
+
+    def _cond_program(self, x, z_pos, context=None):
+        """The program for x's shape with z_pos (and context) set as sample() sets them, or None
+        for a model that is not one of this package's UNets."""
         eng = self._engine_model()
         if eng is None:
-            return img, None
-        B = known.shape[0]
-        prog = eng.program(B, known.shape[2:], known.shape[1], 0 if context is None else context.shape[1])
-        prog.z_in.copy_(self._z_tensor(z_pos, B, device).reshape(-1, 1))
+            return None
+        B = x.shape[0]
+        prog = eng.program(B, x.shape[2:], x.shape[1], 0 if context is None else context.shape[1])
+        prog.z_in.copy_(self._z_tensor(z_pos, B, self.betas.device).reshape(-1, 1))
         if context is not None:
             prog.ctx_in.copy_(context)
-        return img, prog
+        return prog

@@ -286,6 +286,30 @@ def repaint_undo(x, t, alphas, betas, noise=None, rng: Optional[DeviceRng] = Non
                "mri_repaint_undo")
 
 
+VB_DISCRETIZED, VB_GAUSSIAN = 0, 1   # decoder kinds of vb_terms
+
+
+def vb_terms(x0, x_t, eps, z, t, betas, sqrt_1mac, sqrt_recip_alphas, post_var, post_log_var, acc,
+             prior=None, decoder: int = VB_DISCRETIZED, eps_nhwc_ldc: int = 0,
+             channels: int = 0) -> None:
+    """Accumulate one evaluation step of the variational bound at l = t per sample (device int64
+    [samples]): acc[n, l, 0] += sum (eps - z)^2 and, where l = 0, acc[n, 0, 1] += the decoder's
+    -log p(x0 | x_t) summed and prior[n] += sum x0^2.  acc: fp64 (samples, T, 2), prior: fp64
+    (samples,) or None.  eps: fp32 in x0's layout, or the bf16 channels-last UNet output with
+    eps_nhwc_ldc / channels.  decoder: VB_DISCRETIZED (data in [-1, 1]) or VB_GAUSSIAN."""
+    _chk_contig(x0, x_t, eps, z, acc, prior)
+    n = x0.shape[0]
+    assert x0.dtype == x_t.dtype == z.dtype == torch.float32 and t.dtype == torch.int64
+    assert x_t.numel() == z.numel() == x0.numel() and t.numel() >= n
+    assert acc.dtype == torch.float64 and acc.dim() == 3 and acc.shape[0] == n and acc.shape[2] == 2
+    assert prior is None or (prior.dtype == torch.float64 and prior.numel() == n)
+    _lib.check(_lib.load().mri_vb_terms(_p(x0), _p(x_t), _p(eps), eps_nhwc_ldc, channels, _p(z), _p(t),
+                                        _p(betas), _p(sqrt_1mac), _p(sqrt_recip_alphas), _p(post_var),
+                                        _p(post_log_var), int(decoder), _p(acc), _p(prior),
+                                        acc.shape[1], n, x0.numel() // n, _s()),
+               "mri_vb_terms")
+
+
 def step_advance(t: torch.Tensor, delta: int, t_prev=None, rng: Optional[DeviceRng] = None,
                  rng_increment: int = 0) -> None:
     _lib.check(_lib.load().mri_step_advance(_p(t), _p(t_prev), t.numel(), delta,
