@@ -522,6 +522,31 @@ int mri_adam_step(const MriAdamSeg* segs_dev, int n_segs, int64_t total_blocks, 
                   float beta2, float eps, float weight_decay, float* step_dev, const float* grad_scale,
                   const float* found_inf, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Exponential moving average of the weights (optim.EMA; what DDPM / improved-diffusion /
+ * diffusers' training scripts sample from): one launch updates every shadow tensor,
+ * e <- lerp(e, p, w) with ATen's lerp (both of its branches, fp32, the same FMA contraction), so
+ * the result equals torch._foreach_lerp_(e, p, 1 - d) -- torch.optim.swa_utils'
+ * get_ema_multi_avg_fn(d) -- bit for bit.
+ * count_dev: device int64 holding the number of updates applied so far; update k = count + 1
+ * uses  d = decay                                           (warmup == 0)
+ *       d = 0 for k = 1, min(decay, k / (9 + k)) for k >= 2 (warmup != 0; diffusers' EMAModel
+ *                                                            with update_after_step = 0)
+ * computed in fp64, and w = (float)(1 - d), as torch converts the Python scalar 1 - decay.  decay
+ * is a double for that reason: a float 0.9999 would move w by 1.7e-4 relative.  The kernel
+ * advances the counter.  found_inf (device scalar, may be NULL): when *found_inf != 0 nothing is
+ * written and the counter stays -- the GradScaler skip rule of mri_adam_step.
+ * block0 = index of the segment's first 1024-element block; segs_dev lives in device memory.
+ * ------------------------------------------------------------------------------------------ */
+typedef struct MriEmaSeg {
+  float* e;
+  const float* p;
+  int64_t n;
+  int64_t block0;
+} MriEmaSeg;
+int mri_ema_update(const MriEmaSeg* segs_dev, int n_segs, int64_t total_blocks, double decay,
+                   int warmup, int64_t* count_dev, const float* found_inf, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Parameter-gradient finalisation: ONE launch per backward segment turns the raw products of the
  * backward kernels into `.grad` tensors in the reference layouts (what autograd leaves in

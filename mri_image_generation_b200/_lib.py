@@ -101,6 +101,10 @@ class MriAdamSeg(C.Structure):
                 ("n", C.c_int64), ("block0", C.c_int64)]
 
 
+class MriEmaSeg(C.Structure):
+    _fields_ = [("e", C.c_void_p), ("p", C.c_void_p), ("n", C.c_int64), ("block0", C.c_int64)]
+
+
 class MriFinalSeg(C.Structure):
     _fields_ = [("dst", C.c_void_p), ("src", C.c_void_p), ("idx", C.c_void_p), ("n", C.c_int64),
                 ("block0", C.c_int64), ("batch", C.c_int32), ("ld", C.c_int32)]
@@ -124,6 +128,7 @@ SIGNATURES = {
     "mri_linear": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     "mri_im2col": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "mri_adam_step": (_i, [_vp, _i, _i64, _f, _f, _f, _f, _f, _vp, _vp, _vp, _vp]),
+    "mri_ema_update": (_i, [_vp, _i, _i64, C.c_double, _i, _vp, _vp, _vp]),
     "mri_gather_pack": (_i, [_vp, _i, _i64, _vp]),
     "mri_grad_finalize": (_i, [_vp, _i, _i64, _vp]),
     "mri_im2col4": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),

@@ -513,6 +513,53 @@ __global__ void adam_advance_kernel(float* step_dev, const float* found_inf) {
   if (found_inf == nullptr || *found_inf == 0.f) *step_dev += 1.f;
 }
 
+// ATen's lerp (aten/src/ATen/native/Lerp.h) in fp32 opmath: the |w| < 0.5 branch and the other one
+// are written as ATen writes them, so nvcc contracts them to the same FMAs as ATen's CUDA build.
+__device__ __forceinline__ float ema_lerp(float e, float p, float w) {
+  return fabsf(w) < 0.5f ? e + w * (p - e) : p - (p - e) * (1.0f - w);
+}
+
+// Multi-tensor EMA of the weights (see mri_ema_update): e <- lerp(e, p, 1 - d) for every segment,
+// with d from the device-resident update counter.
+__global__ void __launch_bounds__(256)
+ema_update_kernel(const MriEmaSeg* __restrict__ segs, int n_segs, double decay, int warmup,
+                  const int64_t* __restrict__ count_dev, const float* __restrict__ found_inf) {
+  if (found_inf != nullptr && *found_inf != 0.f) return;  // skipped step: the average stays too
+  const int64_t k = *count_dev + 1;
+  const double d = !warmup ? decay : k <= 1 ? 0.0 : fmin(decay, (double)k / (9.0 + (double)k));
+  const float w = (float)(1.0 - d);
+  int lo = 0, hi = n_segs - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (segs[mid].block0 <= (int64_t)blockIdx.x) lo = mid; else hi = mid - 1;
+  }
+  const MriEmaSeg sg = segs[lo];
+  const int64_t b0 = ((int64_t)blockIdx.x - sg.block0) * 1024;
+  const bool vec = ((reinterpret_cast<uintptr_t>(sg.e) | reinterpret_cast<uintptr_t>(sg.p)) & 15u) == 0 &&
+                   b0 + 1024 <= sg.n;
+  if (vec) {  // whole 1024-element block, 16-byte aligned streams: one float4 per thread and stream
+    const int64_t i = b0 + (int64_t)threadIdx.x * 4;
+    float4 e4 = *reinterpret_cast<const float4*>(sg.e + i);
+    const float4 p4 = __ldg(reinterpret_cast<const float4*>(sg.p + i));
+    e4.x = ema_lerp(e4.x, p4.x, w);
+    e4.y = ema_lerp(e4.y, p4.y, w);
+    e4.z = ema_lerp(e4.z, p4.z, w);
+    e4.w = ema_lerp(e4.w, p4.w, w);
+    *reinterpret_cast<float4*>(sg.e + i) = e4;
+    return;
+  }
+#pragma unroll
+  for (int u = 0; u < 4; ++u) {
+    const int64_t i = b0 + threadIdx.x + (int64_t)u * 256;
+    if (i >= sg.n) break;
+    sg.e[i] = ema_lerp(sg.e[i], __ldg(sg.p + i), w);
+  }
+}
+
+__global__ void ema_advance_kernel(int64_t* count_dev, const float* found_inf) {
+  if (found_inf == nullptr || *found_inf == 0.f) *count_dev += 1;
+}
+
 // One launch finalises every parameter gradient of a backward segment (see MriFinalSeg).
 __global__ void __launch_bounds__(256)
 grad_finalize_kernel(const MriFinalSeg* __restrict__ segs, int n_segs) {
@@ -587,6 +634,20 @@ extern "C" int mri_adam_step(const MriAdamSeg* segs_dev, int n_segs, int64_t tot
   if (rc != 0) return rc;
   adam_advance_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(step_dev, found_inf);
   return check_launch("adam_advance_kernel");
+}
+
+extern "C" int mri_ema_update(const MriEmaSeg* segs_dev, int n_segs, int64_t total_blocks, double decay,
+                              int warmup, int64_t* count_dev, const float* found_inf, void* stream) {
+  if (count_dev == nullptr) return set_error(-2, "mri_ema_update: update counter missing");
+  if (!(decay >= 0.0 && decay < 1.0)) return set_error(-2, "mri_ema_update: decay outside [0, 1)");
+  if (n_segs < 1 || total_blocks < 1) return 0;
+  if (total_blocks > 0x7fffffffLL) return set_error(-2, "mri_ema_update: too many blocks");
+  ema_update_kernel<<<(unsigned)total_blocks, 256, 0, (cudaStream_t)stream>>>(
+      segs_dev, n_segs, decay, warmup, count_dev, found_inf);
+  int rc = check_launch("ema_update_kernel");
+  if (rc != 0) return rc;
+  ema_advance_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(count_dev, found_inf);
+  return check_launch("ema_advance_kernel");
 }
 
 extern "C" int mri_grad_finalize(const MriFinalSeg* segs_dev, int n_segs, int64_t total_blocks,
