@@ -307,6 +307,26 @@ int mri_inpaint_merge(float* x, const float* known, const uint8_t* mask, const f
                       const uint64_t* rng, uint64_t rng_skip, const int64_t* t, int64_t t_delta,
                       const float* sqrt_ac, const float* sqrt_1mac, int samples, int64_t per_sample,
                       void* stream);
+/* mri_kspace_work_bytes: the size of mri_kspace_merge's work buffer, samples * channels * H *
+ * (W / 2 + 1) complex fp32 values.  H and W must be at most 512. */
+int mri_kspace_work_bytes(int samples, int channels, int H, int W, size_t* bytes_out);
+/* mri_kspace_merge: k-space data consistency (not in the reference; Song et al., ICLR 2022), in
+ * place on x (fp32, NCHW, samples x channels planes of H x W), per sample with tau = t[n] + t_delta:
+ *     x = x - P(x - sqrt_1mac[tau]*z) + sqrt_ac[tau]*x_zf        (tau >= 0)
+ *     x = x - P x + x_zf                                          (tau < 0; z is not used)
+ * P u = Re F^-1(M . F u), F the orthonormal unshifted 2-D DFT of each plane, M = kmask (one uint8
+ * per element of x, nonzero = measured).  kmask MUST be Hermitian-symmetric, M(k) = M(-k): the
+ * kernel forms only the half spectrum (W / 2 + 1 columns), so P is then the orthogonal projector
+ * P = P^T = P^2; the host completes a measured mask before the call.  x_zf: fp32 in x's layout.
+ * z as for mri_inpaint_merge: `noise`, or with rng the Philox draw at offset rng[1] + rng_skip.
+ * Exactly one of noise / rng.  work: caller-owned, at least mri_kspace_work_bytes, 8-byte aligned.
+ * Three launches (row DFT, column DFT + mask + inverse column DFT, inverse row DFT + update), each
+ * a direct fp32 summation against an exactly indexed sincospi twiddle table: O(HW(H + W)) per
+ * plane, relative error near fp32 rounding.  H and W at most 512. */
+int mri_kspace_merge(float* x, const float* x_zf, const uint8_t* kmask, const float* noise,
+                     const uint64_t* rng, uint64_t rng_skip, const int64_t* t, int64_t t_delta,
+                     const float* sqrt_ac, const float* sqrt_1mac, void* work, size_t work_bytes,
+                     int samples, int channels, int H, int W, void* stream);
 /* mri_repaint_undo: RePaint's undo step (not in the reference), in place per element with
  * l = t[n] in [-1, T - 2] per sample:
  *     x = sqrt(alphas[l + 1])*x + sqrt(betas[l + 1])*z

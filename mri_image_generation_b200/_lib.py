@@ -153,6 +153,9 @@ SIGNATURES = {
     "mri_dpmpp_step": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _i, _i64, _vp]),
     "mri_step_table_advance": (_i, [_vp, _i, _vp, _vp, _i, _vp]),
     "mri_inpaint_merge": (_i, [_vp, _vp, _vp, _vp, _vp, _u64, _vp, _i64, _vp, _vp, _i, _i64, _vp]),
+    "mri_kspace_work_bytes": (_i, [_i, _i, _i, _i, _vp]),
+    "mri_kspace_merge": (_i, [_vp, _vp, _vp, _vp, _vp, _u64, _vp, _i64, _vp, _vp, _vp, C.c_size_t, _i,
+                              _i, _i, _i, _vp]),
     "mri_repaint_undo": (_i, [_vp, _vp, _vp, _u64, _vp, _vp, _vp, _i, _i64, _vp]),
     "mri_vb_terms": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _i,
                           _i, _i64, _vp]),

@@ -430,6 +430,234 @@ inpaint_merge_kernel(float* x, const float* known, const uint8_t* mask, const fl
 }
 
 // ------------------------------------------------------------------------------------------
+// k-space data consistency (mri_kspace_merge): per sample, tau = t[n] + t_delta and
+//   x <- x - P(x - s1m[tau] z) + (tau < 0 ? x_zf : sac[tau] x_zf)    (no z term at tau < 0)
+// with P u = Re F^-1(M . F u), F the orthonormal 2-D DFT of each (H, W) plane and M the
+// Hermitian-symmetric mask.  Because M is Hermitian, M . F u of a real u is Hermitian, so only
+// the half spectrum k < Wh = W/2 + 1 is formed.  Three passes over a complex [plane][H][Wh] work
+// buffer, each a direct fp32 summation (FMA) against a twiddle table in shared memory with the
+// exact index (j k) mod N:
+//   A  u = x - s1m z per row, forward row DFT (real -> half spectrum)        kKsRows rows a block
+//   B  forward column DFT, times M, inverse column DFT                      kKsCols columns a block
+//   C  inverse row DFT (half spectrum -> real), P u / (H W), the update       kKsRows rows a block
+// ------------------------------------------------------------------------------------------
+constexpr int kKsMaxN = 512;      // H, W limit: pass B keeps two H x kKsCols complex tiles
+constexpr int kKsRows = 16;       // rows per block of passes A and C
+constexpr int kKsCols = 16;       // columns per block of pass B (128-byte rows of the tile)
+constexpr int kKsThreadsA = 128, kKsThreadsB = 256, kKsThreadsC = 256;
+
+struct KspaceArgs {
+  float* x;
+  const float* zf;
+  const uint8_t* mask;
+  const float* noise;
+  const uint64_t* rng;
+  uint64_t ctr_skip;
+  const int64_t* t;
+  long long t_delta;
+  const float* sqrt_ac;
+  const float* sqrt_1mac;
+  float2* work;
+  int channels, H, W, Wh;
+  long long Tt;     // ATen's launch for a draw of the whole x (normal_at)
+};
+
+// The twiddle table takes an even number of float2 entries, so the arrays after it, read with
+// 16-byte loads, stay 16-byte aligned for odd H and W.
+__host__ __device__ __forceinline__ int ks_tw_len(int n) { return (n + 1) & ~1; }
+static int ks_smem_a(int W) { return ks_tw_len(W) * 8 + W * kKsRows * 4; }
+static int ks_smem_b(int H) { return ks_tw_len(H) * 8 + 2 * H * kKsCols * 8 + H * 4; }
+static int ks_smem_c(int W) { return ks_tw_len(W) * 8 + (W / 2 + 1) * kKsRows * 8; }
+
+// tw[j] = exp(-2 pi i j / n), j < n: fp64 sincospi, rounded once to fp32
+__device__ __forceinline__ void ks_twiddles(float2* tw, int n) {
+  for (int j = threadIdx.x; j < n; j += blockDim.x) {
+    double s, c;
+    sincospi(2.0 * j / n, &s, &c);
+    tw[j] = make_float2((float)c, (float)-s);
+  }
+}
+
+template <bool RNG>
+__global__ void __launch_bounds__(kKsThreadsA) kspace_rows_fwd_kernel(const KspaceArgs a) {
+  extern __shared__ float4 ks_smem[];
+  float2* tw = reinterpret_cast<float2*>(ks_smem);
+  float* u = reinterpret_cast<float*>(tw + ks_tw_len(a.W));    // [W][kKsRows]
+  const int nrb = (a.H + kKsRows - 1) / kKsRows;
+  const long long plane = blockIdx.x / nrb;
+  const int h0 = (int)(blockIdx.x % nrb) * kKsRows;
+  const long long tau = a.t[plane / a.channels] + a.t_delta;
+  ks_twiddles(tw, a.W);
+  uint64_t seed = 0, ctr0 = 0;
+  if (RNG) {
+    seed = a.rng[0];
+    ctr0 = (a.rng[1] >> 2) + a.ctr_skip;
+  }
+  const float s = tau < 0 ? 0.f : __ldg(a.sqrt_1mac + tau);
+  for (int i = threadIdx.x; i < kKsRows * a.W; i += blockDim.x) {
+    const int r = i / a.W, w = i - r * a.W;
+    float v = 0.f;
+    if (h0 + r < a.H) {
+      const long long e = (plane * a.H + h0 + r) * a.W + w;
+      v = a.x[e];
+      if (tau >= 0) v = __fsub_rn(v, __fmul_rn(s, RNG ? normal_at(seed, ctr0, e, a.Tt) : a.noise[e]));
+    }
+    u[w * kKsRows + r] = v;
+  }
+  __syncthreads();
+  for (int k = threadIdx.x; k < a.Wh; k += blockDim.x) {
+    float re[kKsRows], im[kKsRows];
+#pragma unroll
+    for (int r = 0; r < kKsRows; ++r) re[r] = im[r] = 0.f;
+    int idx = 0;
+    for (int w = 0; w < a.W; ++w) {
+      const float2 c = tw[idx];
+      const float4* up = reinterpret_cast<const float4*>(u + w * kKsRows);
+#pragma unroll
+      for (int q = 0; q < kKsRows / 4; ++q) {
+        const float4 v = up[q];
+        const float vv[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int m = 0; m < 4; ++m) {
+          re[4 * q + m] = fmaf(vv[m], c.x, re[4 * q + m]);
+          im[4 * q + m] = fmaf(vv[m], c.y, im[4 * q + m]);
+        }
+      }
+      idx += k;
+      if (idx >= a.W) idx -= a.W;
+    }
+#pragma unroll
+    for (int r = 0; r < kKsRows; ++r)
+      if (h0 + r < a.H) a.work[(plane * a.H + h0 + r) * a.Wh + k] = make_float2(re[r], im[r]);
+  }
+}
+
+__global__ void __launch_bounds__(kKsThreadsB) kspace_cols_kernel(const KspaceArgs a) {
+  extern __shared__ float4 ks_smem[];
+  const int H = a.H;
+  float2* tw = reinterpret_cast<float2*>(ks_smem);
+  float2* U = tw + ks_tw_len(H);       // [H][kKsCols]: the row spectra, then their inverse
+  float2* V = U + H * kKsCols;         // [H][kKsCols]: M . column spectra
+  int* live = reinterpret_cast<int*>(V + H * kKsCols);   // row m of V has a measured sample
+  const int nct = (a.Wh + kKsCols - 1) / kKsCols;
+  const long long plane = blockIdx.x / nct;
+  const int c0 = (int)(blockIdx.x % nct) * kKsCols;
+  ks_twiddles(tw, H);
+  for (int i = threadIdx.x; i < H * kKsCols; i += blockDim.x) {
+    const int h = i / kKsCols, c = c0 + i % kKsCols;
+    U[i] = c < a.Wh ? a.work[(plane * H + h) * a.Wh + c] : make_float2(0.f, 0.f);
+  }
+  __syncthreads();
+  // forward: thread m sums over h for the tile's columns, so the U loads are warp broadcasts
+  for (int m = threadIdx.x; m < H; m += blockDim.x) {
+    float re[kKsCols], im[kKsCols];
+#pragma unroll
+    for (int j = 0; j < kKsCols; ++j) re[j] = im[j] = 0.f;
+    int idx = 0;
+    for (int h = 0; h < H; ++h) {
+      const float2 c = tw[idx];
+      const float4* up = reinterpret_cast<const float4*>(U + h * kKsCols);
+#pragma unroll
+      for (int q = 0; q < kKsCols / 2; ++q) {
+        const float4 v = up[q];
+        re[2 * q] = fmaf(-v.y, c.y, fmaf(v.x, c.x, re[2 * q]));
+        im[2 * q] = fmaf(v.y, c.x, fmaf(v.x, c.y, im[2 * q]));
+        re[2 * q + 1] = fmaf(-v.w, c.y, fmaf(v.z, c.x, re[2 * q + 1]));
+        im[2 * q + 1] = fmaf(v.w, c.x, fmaf(v.z, c.y, im[2 * q + 1]));
+      }
+      idx += m;
+      if (idx >= H) idx -= H;
+    }
+    const uint8_t* mrow = a.mask + (plane * H + m) * a.W + c0;
+    int any = 0;
+#pragma unroll
+    for (int j = 0; j < kKsCols; ++j) {
+      const bool keep = c0 + j < a.Wh && mrow[j] != 0;
+      any |= keep;
+      V[m * kKsCols + j] = keep ? make_float2(re[j], im[j]) : make_float2(0.f, 0.f);
+    }
+    live[m] = any;
+  }
+  __syncthreads();
+  // inverse: exp(+2 pi i h m / H) = conj(tw); rows of V with no measured sample add nothing
+  for (int h = threadIdx.x; h < H; h += blockDim.x) {
+    float re[kKsCols], im[kKsCols];
+#pragma unroll
+    for (int j = 0; j < kKsCols; ++j) re[j] = im[j] = 0.f;
+    int idx = 0;
+    for (int m = 0; m < H; ++m) {
+      if (live[m]) {
+        const float2 c = tw[idx];
+        const float4* vp = reinterpret_cast<const float4*>(V + m * kKsCols);
+#pragma unroll
+        for (int q = 0; q < kKsCols / 2; ++q) {
+          const float4 v = vp[q];
+          re[2 * q] = fmaf(v.y, c.y, fmaf(v.x, c.x, re[2 * q]));
+          im[2 * q] = fmaf(-v.x, c.y, fmaf(v.y, c.x, im[2 * q]));
+          re[2 * q + 1] = fmaf(v.w, c.y, fmaf(v.z, c.x, re[2 * q + 1]));
+          im[2 * q + 1] = fmaf(-v.z, c.y, fmaf(v.w, c.x, im[2 * q + 1]));
+        }
+      }
+      idx += h;
+      if (idx >= H) idx -= H;
+    }
+    float2* out = a.work + (plane * H + h) * a.Wh + c0;
+#pragma unroll
+    for (int j = 0; j < kKsCols; ++j)
+      if (c0 + j < a.Wh) out[j] = make_float2(re[j], im[j]);
+  }
+}
+
+__global__ void __launch_bounds__(kKsThreadsC) kspace_rows_inv_kernel(const KspaceArgs a) {
+  extern __shared__ float4 ks_smem[];
+  float2* tw = reinterpret_cast<float2*>(ks_smem);
+  float2* us = tw + ks_tw_len(a.W);                 // [Wh][kKsRows]
+  const int nrb = (a.H + kKsRows - 1) / kKsRows;
+  const long long plane = blockIdx.x / nrb;
+  const int h0 = (int)(blockIdx.x % nrb) * kKsRows;
+  const long long tau = a.t[plane / a.channels] + a.t_delta;
+  ks_twiddles(tw, a.W);
+  // Re of the full inverse sum: bins 0 and W/2 (W even) once, every other bin twice (its mirror)
+  for (int i = threadIdx.x; i < kKsRows * a.Wh; i += blockDim.x) {
+    const int r = i / a.Wh, k = i - r * a.Wh;
+    float2 v = make_float2(0.f, 0.f);
+    if (h0 + r < a.H) {
+      v = a.work[(plane * a.H + h0 + r) * a.Wh + k];
+      if (k != 0 && 2 * k != a.W) v = make_float2(2.f * v.x, 2.f * v.y);
+    }
+    us[k * kKsRows + r] = v;
+  }
+  __syncthreads();
+  const float scale = (float)(1.0 / ((double)a.H * a.W));
+  const float sac = tau < 0 ? 1.f : __ldg(a.sqrt_ac + tau);
+  for (int w = threadIdx.x; w < a.W; w += blockDim.x) {
+    float acc[kKsRows];
+#pragma unroll
+    for (int r = 0; r < kKsRows; ++r) acc[r] = 0.f;
+    int idx = 0;
+    for (int k = 0; k < a.Wh; ++k) {
+      const float2 c = tw[idx];          // Re(v exp(+i theta)) = v.x cos - v.y sin = v.x c.x + v.y c.y
+      const float4* vp = reinterpret_cast<const float4*>(us + k * kKsRows);
+#pragma unroll
+      for (int q = 0; q < kKsRows / 2; ++q) {
+        const float4 v = vp[q];
+        acc[2 * q] = fmaf(v.y, c.y, fmaf(v.x, c.x, acc[2 * q]));
+        acc[2 * q + 1] = fmaf(v.w, c.y, fmaf(v.z, c.x, acc[2 * q + 1]));
+      }
+      idx += w;
+      if (idx >= a.W) idx -= a.W;
+    }
+#pragma unroll
+    for (int r = 0; r < kKsRows; ++r) {
+      if (h0 + r >= a.H) break;
+      const long long e = (plane * a.H + h0 + r) * a.W + w;
+      const float add = tau < 0 ? a.zf[e] : __fmul_rn(sac, a.zf[e]);
+      a.x[e] = __fadd_rn(__fsub_rn(a.x[e], __fmul_rn(acc[r], scale)), add);
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------
 // Terms of the variational bound on -log p(x0) for one evaluation step at per-sample timestep
 // t[n], given x0, x_t = q_sample(x0, t, z), z and the predicted eps:
 //   acc[n][t][0] += sum (eps - z)^2                      (L_t = lambda_t times this for t >= 1)
@@ -973,6 +1201,78 @@ extern "C" int mri_inpaint_merge(float* x, const float* known, const uint8_t* ma
         x, known, mask, noise, nullptr, 0, t, t_delta, sqrt_ac, sqrt_1mac, per_sample, numel, g.Tt,
         g.n_iter);
   return check_launch("inpaint_merge_kernel");
+}
+
+static int kspace_dims(const char* who, int samples, int channels, int H, int W) {
+  if (samples < 1 || channels < 1 || H < 1 || W < 1) return set_error(-2, who);
+  if (H > kKsMaxN || W > kKsMaxN) return set_error(-2, "mri_kspace_merge: H and W must be at most 512");
+  if ((long long)samples * channels * ((H + kKsRows - 1) / kKsRows) > 0x7fffffffLL)
+    return set_error(-2, "mri_kspace_merge: too many planes");
+  return 0;
+}
+
+extern "C" int mri_kspace_work_bytes(int samples, int channels, int H, int W, size_t* bytes_out) {
+  int rc = kspace_dims("mri_kspace_work_bytes: empty input", samples, channels, H, W);
+  if (rc) return rc;
+  if (bytes_out == nullptr) return set_error(-2, "mri_kspace_work_bytes: null output");
+  *bytes_out = (size_t)samples * channels * H * (W / 2 + 1) * sizeof(float2);
+  return 0;
+}
+
+extern "C" int mri_kspace_merge(float* x, const float* x_zf, const uint8_t* kmask, const float* noise,
+                                const uint64_t* rng, uint64_t rng_skip, const int64_t* t,
+                                int64_t t_delta, const float* sqrt_ac, const float* sqrt_1mac,
+                                void* work, size_t work_bytes, int samples, int channels, int H, int W,
+                                void* stream) {
+  size_t need = 0;
+  int rc = mri_kspace_work_bytes(samples, channels, H, W, &need);
+  if (rc) return rc;
+  if (x == nullptr || x_zf == nullptr || kmask == nullptr || t == nullptr || sqrt_ac == nullptr ||
+      sqrt_1mac == nullptr || work == nullptr)
+    return set_error(-2, "mri_kspace_merge: null x / x_zf / kmask / t / schedule table / work");
+  if ((noise == nullptr) == (rng == nullptr))
+    return set_error(-2, "mri_kspace_merge: exactly one of noise / rng");
+  if (rng_skip % 4 != 0) return set_error(-2, "mri_kspace_merge: rng_skip must be a multiple of 4");
+  if (work_bytes < need || (reinterpret_cast<uintptr_t>(work) & 7) != 0)
+    return set_error(-2, "mri_kspace_merge: work smaller than mri_kspace_work_bytes or not 8-byte aligned");
+  rc = device_props();
+  if (rc) return rc;
+  static bool configured = false;   // once, at the largest size (not re-done inside a graph capture)
+  if (!configured) {
+    cudaError_t e = cudaFuncSetAttribute(kspace_cols_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         ks_smem_b(kKsMaxN));
+    if (e != cudaSuccess) return set_cuda_error(e, "cudaFuncSetAttribute(kspace_cols_kernel)");
+    configured = true;
+  }
+  KspaceArgs a;
+  a.x = x;
+  a.zf = x_zf;
+  a.mask = kmask;
+  a.noise = noise;
+  a.rng = rng;
+  a.ctr_skip = rng_skip / 4;
+  a.t = t;
+  a.t_delta = t_delta;
+  a.sqrt_ac = sqrt_ac;
+  a.sqrt_1mac = sqrt_1mac;
+  a.work = static_cast<float2*>(work);
+  a.channels = channels; a.H = H; a.W = W; a.Wh = W / 2 + 1;
+  const long long planes = (long long)samples * channels;
+  a.Tt = aten_grid(planes * H * W).Tt;
+  cudaStream_t st = (cudaStream_t)stream;
+  const unsigned rows_grid = (unsigned)(planes * ((H + kKsRows - 1) / kKsRows));
+  if (rng != nullptr)
+    kspace_rows_fwd_kernel<true><<<rows_grid, kKsThreadsA, ks_smem_a(W), st>>>(a);
+  else
+    kspace_rows_fwd_kernel<false><<<rows_grid, kKsThreadsA, ks_smem_a(W), st>>>(a);
+  rc = check_launch("kspace_rows_fwd_kernel");
+  if (rc) return rc;
+  kspace_cols_kernel<<<(unsigned)(planes * ((a.Wh + kKsCols - 1) / kKsCols)), kKsThreadsB, ks_smem_b(H),
+                       st>>>(a);
+  rc = check_launch("kspace_cols_kernel");
+  if (rc) return rc;
+  kspace_rows_inv_kernel<<<rows_grid, kKsThreadsC, ks_smem_c(W), st>>>(a);
+  return check_launch("kspace_rows_inv_kernel");
 }
 
 extern "C" int mri_repaint_undo(float* x, const float* noise, const uint64_t* rng, uint64_t rng_skip,

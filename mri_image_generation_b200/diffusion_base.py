@@ -6,6 +6,7 @@ model arguments (z_pos, context) and the loss; everything that touches the GPU i
     mri_ddpm_step, mri_ddim_step), bit-exact w.r.t. the reference's eager association order;
     DPM-Solver++(2M) (not in the reference): mri_dpmpp_step over a host-built coefficient table;
     inpainting (not in the reference): mri_inpaint_merge after each update of either sampler;
+    undersampled k-space reconstruction (not in the reference): mri_kspace_merge in the same slot;
     RePaint's resampling (not in the reference): mri_repaint_undo between the inpainting steps;
     the variational bound in bits per dimension (not in the reference): mri_vb_terms after each
     evaluation step, on a step graph of its own;
@@ -35,6 +36,18 @@ def _require_cuda(x: torch.Tensor, what: str) -> None:
     if not x.is_cuda:
         raise _lib.MriError(f"{what}: tensors must live on a B200 GPU (got {x.device}); "
                             "this framework has no CPU fallback")
+
+
+def kspace_completion(y: torch.Tensor, m: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Hermitian completion of a measured k-space, on y's device: (x_zf, M) with M = m | m(-k),
+    y(k) = conj(y(-k)) where k is measured only at its mirror, and x_zf = Re ifft2(M y) in fp64
+    (orthonormal, unshifted).  y: complex (..., H, W); m: bool of y's shape.  Values of y outside
+    m are never read."""
+    mir = lambda a: torch.roll(torch.flip(a, (-2, -1)), (1, 1), (-2, -1))   # a(-k)
+    full = m | mir(m)
+    y = y.to(torch.complex128)
+    y = torch.where(m, y, torch.where(full, mir(y).conj(), torch.zeros_like(y)))
+    return torch.fft.ifft2(y, norm="ortho").real, full
 
 
 class _LossFn(torch.autograd.Function):
@@ -168,17 +181,19 @@ class DiffusionBase(nn.Module):
                              f"(got num_steps={M}, start_t={s})")
         return schedules.dpmpp_2m_table(self.alphas_cumprod, schedules.dpmpp_timesteps(s, M))
 
-    def _sample_dpmpp(self, img, table, prog, eps_fn: Callable, inpaint=None) -> torch.Tensor:
+    def _sample_dpmpp(self, img, table, prog, eps_fn: Callable, inpaint=None,
+                      kspace: bool = False) -> torch.Tensor:
         """Run the solver over `table` from x = img.  prog: a UNetProgram whose conditioning inputs
         the caller has set (replayed step graph), or None: eager, eps = eps_fn(x, t) per step.
         inpaint: (known, mask) of _inpaint_inputs; after row i the kept region is replaced by
-        q_sample(known, ts[i + 1], noise=img), and by known itself after the last row.
+        q_sample(known, ts[i + 1], noise=img), and by known itself after the last row.  With
+        kspace, (x_zf, mask) of _kspace_inputs, and the merge is the k-space one (_merge).
         Returns the fp32 x0 estimate."""
         _require_cuda(img, "sample_dpmpp")
         ts, coef = table
         if prog is not None:
             return self._reverse_loop(prog, img.float(), int(ts[0]), ts.numel(), "dpmpp", table=table,
-                                      inpaint=inpaint)
+                                      inpaint=inpaint, kspace=kspace)
         dev = img.device
         with torch.cuda.device(dev):
             coef = coef.to(dev)
@@ -192,8 +207,7 @@ class DiffusionBase(nn.Module):
                 ops.dpmpp_step(x, eps.float().contiguous(), x0_prev, coef[i], None, x)
                 if inpaint is not None:
                     tt.fill_(tau[i])
-                    ops.inpaint_merge(x, inpaint[0], inpaint[1], tt, 0, self.sqrt_alphas_cumprod,
-                                      self.sqrt_one_minus_alphas_cumprod, noise=x_T)
+                    self._merge(x, inpaint, tt, 0, kspace, noise=x_T)
         return x
 
     # ------------------------------------------------------------------ inpainting
@@ -221,17 +235,62 @@ class DiffusionBase(nn.Module):
         m.copy_(mask.to(known.device).expand(known.shape))
         return known, m
 
-    def _inpaint_buffers(self, prog, with_noise: bool) -> Dict[str, torch.Tensor]:
+    def _inpaint_buffers(self, prog, with_noise: bool, kspace: bool = False) -> Dict[str, torch.Tensor]:
         """The program's inpainting inputs: known, mask and, for DPM-Solver++, the x_T copy the
         known region is noised with.  Each call copies into them, so one captured graph serves
-        every x_known and mask."""
+        every x_known and mask.  The k-space merge reads x_zf and its mask from the same buffers
+        and adds a work buffer of its own (mri_kspace_work_bytes)."""
         bufs = prog.__dict__.setdefault("_inpaint_bufs", {})
         if "known" not in bufs:
             bufs["known"] = torch.zeros_like(prog.x_in)
             bufs["mask"] = torch.zeros(prog.x_in.shape, dtype=torch.uint8, device=prog.x_in.device)
         if with_noise and "noise" not in bufs:
             bufs["noise"] = torch.zeros_like(prog.x_in)
+        if kspace and "work" not in bufs:
+            bufs["work"] = torch.zeros(ops.kspace_work_bytes(*prog.x_in.shape), dtype=torch.uint8,
+                                       device=prog.x_in.device)
         return bufs
+
+    def _merge(self, x, cond, t, t_delta: int, kspace: bool, work=None, **z) -> None:
+        """The merge after a reverse update, in place on x: mri_inpaint_merge with cond = (known,
+        mask), or with kspace mri_kspace_merge with cond = (x_zf, mask) and its work buffer (None:
+        allocated per call).  z: noise= or rng= / rng_skip= as the ops take them."""
+        if kspace:
+            ops.kspace_merge(x, cond[0], cond[1], t, t_delta, self.sqrt_alphas_cumprod,
+                             self.sqrt_one_minus_alphas_cumprod, work=work, **z)
+        else:
+            ops.inpaint_merge(x, cond[0], cond[1], t, t_delta, self.sqrt_alphas_cumprod,
+                              self.sqrt_one_minus_alphas_cumprod, **z)
+
+    # ------------------------------------------------------------------ k-space reconstruction
+    def _kspace_inputs(self, kspace, kmask) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Check (kspace, kmask) and complete them once per call: M = m | m(-k), y(k) = conj(y(-k))
+        where k is measured only at its mirror, x_zf = Re ifft2(M y) (orthonormal, in fp64).
+        Returns (x_zf fp32, M as one uint8 per element) on the model's device, as mri_kspace_merge
+        reads them.  ValueError on a bad kspace or mask, MriError on a CPU tensor or H, W over the
+        kernel's limit; callers check before anything is drawn."""
+        if not torch.is_tensor(kspace) or not kspace.is_complex() or kspace.dim() != 4 \
+                or kspace.shape[1] != self.channels:
+            got = (tuple(kspace.shape), kspace.dtype) if torch.is_tensor(kspace) else type(kspace)
+            raise ValueError(f"kspace must be a complex (B, {self.channels}, H, W) tensor (got {got})")
+        if kspace.numel() == 0:
+            raise ValueError("kspace is empty")
+        mask = torch.as_tensor(kmask)
+        try:
+            ok = torch.broadcast_shapes(mask.shape, kspace.shape) == kspace.shape
+        except RuntimeError:
+            ok = False
+        if not ok:
+            raise ValueError(f"kmask of shape {tuple(mask.shape)} does not broadcast to kspace's "
+                             f"{tuple(kspace.shape)}")
+        if mask.dtype != torch.bool and not bool(((mask == 0) | (mask == 1)).all()):
+            raise ValueError("kmask must be bool or hold only 0 / 1 (1 = measured)")
+        _require_cuda(kspace, "reconstruct")
+        ops.kspace_work_bytes(*kspace.shape)      # MriError when H or W is over the kernel's limit
+        dev = self.betas.device
+        with torch.cuda.device(dev):
+            x_zf, full = kspace_completion(kspace.to(dev), mask.to(dev).expand(kspace.shape).bool())
+            return x_zf.float().contiguous(), full.to(torch.uint8).contiguous()
 
     def _repaint_levels(self, jump_length, jump_n_sample) -> Optional[list]:
         """schedules.repaint_levels for this schedule (ValueError on bad arguments), or None when
@@ -239,33 +298,36 @@ class DiffusionBase(nn.Module):
         levels = schedules.repaint_levels(self.timesteps, jump_length, jump_n_sample)
         return levels if len(levels) > self.timesteps + 1 else None
 
-    def _inpaint_ddpm(self, img, inpaint, prog, eps_fn: Callable, levels=None) -> torch.Tensor:
+    def _inpaint_ddpm(self, img, inpaint, prog, eps_fn: Callable, levels=None,
+                      kspace: bool = False) -> torch.Tensor:
         """Ancestral sampling from x_T = img over every timestep with the kept region replaced after
         each update by q_sample(known, i - 1, noise=randn_like(x)) (known itself after i = 0).
-        prog / eps_fn as for _sample_dpmpp.  levels: RePaint's resampling (_inpaint_repaint)."""
+        prog / eps_fn / kspace as for _sample_dpmpp.  levels: RePaint's resampling
+        (_inpaint_repaint; not with kspace)."""
         _require_cuda(img, "inpaint")
         if levels is not None:
             return self._inpaint_repaint(img, inpaint, prog, eps_fn, levels)
         T = self.timesteps
         if prog is not None:
-            return self._reverse_loop(prog, img.float(), T - 1, T, "ddpm", inpaint=inpaint)
+            return self._reverse_loop(prog, img.float(), T - 1, T, "ddpm", inpaint=inpaint,
+                                      kspace=kspace)
         dev = img.device
         x = img.float().contiguous()
         with torch.cuda.device(dev):
             rng = self._rng(dev)
             inc = ops.randn_offset_increment(x.numel())
             for i in reversed(range(T)):
-                x = self._inpaint_step(x, i, inpaint, eps_fn, rng, inc)
+                x = self._inpaint_step(x, i, inpaint, eps_fn, rng, inc, kspace)
         return x
 
-    def _inpaint_step(self, x, i, inpaint, eps_fn, rng, inc) -> torch.Tensor:
+    def _inpaint_step(self, x, i, inpaint, eps_fn, rng, inc, kspace: bool = False) -> torch.Tensor:
         """One eager DDPM inpainting step at t = i: update, then the kept region becomes
-        q_sample(known, i - 1, noise=randn_like(x)) (known itself at i = 0)."""
+        q_sample(known, i - 1, noise=randn_like(x)) (known itself at i = 0); with kspace the
+        k-space merge with the same z."""
         t = torch.full((x.shape[0],), i, device=x.device, dtype=torch.long)
         x = self._p_update(x, t, eps_fn(x, t))
         off = rng.load()
-        ops.inpaint_merge(x, inpaint[0], inpaint[1], t, -1, self.sqrt_alphas_cumprod,
-                          self.sqrt_one_minus_alphas_cumprod, rng=rng)
+        self._merge(x, inpaint, t, -1, kspace, rng=rng)
         rng.commit(off + inc)
         return x
 
@@ -305,7 +367,7 @@ class DiffusionBase(nn.Module):
                         k=torch.zeros(1, dtype=torch.int64, device=dev),
                         x0_prev=torch.zeros_like(prog.x_in))
             prog.__dict__["_dpmpp_bufs"] = bufs
-            for key in ("dpmpp", "dpmpp+inpaint"):   # captured on the old buffers
+            for key in ("dpmpp", "dpmpp+inpaint", "dpmpp+kspace"):   # captured on the old buffers
                 prog.__dict__.get("_step_graphs", {}).pop(key, None)
         return bufs
 
@@ -443,22 +505,25 @@ class DiffusionBase(nn.Module):
 
     def _reverse_loop(self, prog, img: torch.Tensor, start_t: int, n_steps: int, mode: str,
                       use_graph: bool = True, t_vec: Optional[torch.Tensor] = None,
-                      stride: int = 1, table=None, inpaint=None, levels=None) -> torch.Tensor:
+                      stride: int = 1, table=None, inpaint=None, levels=None,
+                      kspace: bool = False) -> torch.Tensor:
         """Run n_steps reverse steps (i = start_t, start_t - stride, ...) on `prog` (a UNetProgram
         whose x_in is the sampler state).  mode: 'ddpm' | 'ddim' (t_prev = max(t - stride, 0)) |
         'dpmpp' (table = (ts, coef) of schedules.dpmpp_2m_table, n_steps = its rows).
         inpaint: (known, mask) of _inpaint_inputs, 'ddpm' or 'dpmpp' only: mri_inpaint_merge
         after every update, on a step graph of its own ('ddpm+inpaint' / 'dpmpp+inpaint').
+        kspace: inpaint holds (x_zf, mask) of _kspace_inputs and the merge is mri_kspace_merge with
+        the same z, on 'ddpm+kspace' / 'dpmpp+kspace'.
         levels: RePaint's walk (schedules.repaint_levels), 'ddpm' with inpaint only: its n_steps
         reverse steps replay 'ddpm+inpaint', its undo steps a graph of their own
         ('repaint-undo': mri_repaint_undo at t, then t += 1), in the walk's order."""
         dev = img.device
         with torch.cuda.device(dev):
             return self._reverse_loop_on(prog, img, start_t, n_steps, mode, use_graph, t_vec, stride,
-                                         table, inpaint, levels)
+                                         table, inpaint, levels, kspace)
 
     def _reverse_loop_on(self, prog, img, start_t, n_steps, mode, use_graph, t_vec, stride,
-                         table=None, inpaint=None, levels=None):
+                         table=None, inpaint=None, levels=None, kspace=False):
         dev = img.device
         if prog.params_changed():
             prog.do_refresh()
@@ -476,9 +541,9 @@ class DiffusionBase(nn.Module):
         if inpaint is not None:
             if mode not in ("ddpm", "dpmpp") or stride != 1 or t_vec is not None:
                 raise _lib.MriError("inpainting runs on the full DDPM or the DPM-Solver++ loop")
-            inp = self._inpaint_buffers(prog, mode == "dpmpp")
-            gkey += "+inpaint"
-        if levels is not None and (inp is None or mode != "ddpm"):
+            inp = self._inpaint_buffers(prog, mode == "dpmpp", kspace)
+            gkey += "+kspace" if kspace else "+inpaint"
+        if levels is not None and (inp is None or mode != "ddpm" or kspace):
             raise _lib.MriError("RePaint resampling runs on the DDPM inpainting loop")
         # DDPM inpainting draws a second randn_like(x) per step (the merge's noise)
         adv = 2 * inc if inp is not None else inc
@@ -493,14 +558,11 @@ class DiffusionBase(nn.Module):
             kbuf.zero_()   # a valid row for the warm-up launch of a capture
 
         def merge():
+            cond, work = (inp["known"], inp["mask"]), inp.get("work")
             if mode == "ddpm":   # before step_advance: tau = t - 1, z drawn after the update's z
-                ops.inpaint_merge(prog.x_in, inp["known"], inp["mask"], prog.t_in, -1,
-                                  self.sqrt_alphas_cumprod, self.sqrt_one_minus_alphas_cumprod,
-                                  rng=rng, rng_skip=inc)
+                self._merge(prog.x_in, cond, prog.t_in, -1, kspace, work, rng=rng, rng_skip=inc)
             else:                # after step_table_advance: t = ts[k], -1 past the last row
-                ops.inpaint_merge(prog.x_in, inp["known"], inp["mask"], prog.t_in, 0,
-                                  self.sqrt_alphas_cumprod, self.sqrt_one_minus_alphas_cumprod,
-                                  noise=inp["noise"])
+                self._merge(prog.x_in, cond, prog.t_in, 0, kspace, work, noise=inp["noise"])
 
         def one_step():
             if fused:  # out_conv's tap sum + the update in one kernel: eps never goes to HBM

@@ -110,6 +110,35 @@ class GaussianDiffusion(_GD2):
                                   lambda x, t: self.model(x, t, z_pos, context=context), levels)
 
     @torch.no_grad()
+    def reconstruct(self, kspace, kmask, z_pos=0.5, context=None):
+        """Reconstruction from undersampled k-space with the full DDPM sampler (not in the
+        reference), e.g. multi-contrast: t1, t1ce and t2 fully sampled (kmask 1 on their channels)
+        and an undersampled flair.  See the 2D class's reconstruct()."""
+        zf, m = self._kspace_inputs(kspace, kmask)
+        device = self.betas.device
+        if context is not None:
+            context = context.to(device)
+        img, prog = self._inpaint_start(zf, z_pos, context)
+        z_pos = self._z_tensor(z_pos, img.shape[0], device)
+        return self._inpaint_ddpm(img, (zf, m), prog,
+                                  lambda x, t: self.model(x, t, z_pos, context=context), kspace=True)
+
+    @torch.no_grad()
+    def reconstruct_dpmpp(self, kspace, kmask, z_pos=0.5, context=None, num_steps=20):
+        """reconstruct() with DPM-Solver++(2M) in `num_steps` UNet calls (not in the reference);
+        see the 2D class's reconstruct_dpmpp()."""
+        table = self._dpmpp_table(self.timesteps - 1, num_steps)
+        zf, m = self._kspace_inputs(kspace, kmask)
+        device = self.betas.device
+        if context is not None:
+            context = context.to(device)
+        img, prog = self._inpaint_start(zf, z_pos, context)
+        z_pos = self._z_tensor(z_pos, img.shape[0], device)
+        return self._sample_dpmpp(img, table, prog,
+                                  lambda x, t: self.model(x, t, z_pos, context=context),
+                                  inpaint=(zf, m), kspace=True)
+
+    @torch.no_grad()
     def inpaint_dpmpp(self, x_known, mask, z_pos=0.5, context=None, num_steps=20):
         """inpaint() with DPM-Solver++(2M) in `num_steps` UNet calls (not in the reference); see
         the 2D class's inpaint_dpmpp()."""

@@ -132,6 +132,34 @@ class GaussianDiffusion(DiffusionBase):
         return self._sample_dpmpp(img, table, prog, lambda x, t: self.model(x, t, z_pos), inpaint=inp)
 
     @torch.no_grad()
+    def reconstruct(self, kspace, kmask, z_pos=0.5):
+        """Reconstruction from undersampled k-space with the full DDPM sampler (not in the
+        reference; Song, Shen, Xing & Ermon, ICLR 2022).  kspace: complex (B, channels, H, W), the
+        orthonormal unshifted fft2 of the image (DC at [0, 0]); kmask broadcasts to it, True / 1 =
+        measured (values outside it are ignored).  The mask is completed to M = m | m(-k).  x_T is
+        drawn as sample() draws it; after the update at every step i, with tau = i - 1 and
+        n = randn_like(x), x = x - P(x - sqrt(1 - abar_tau) n) + sqrt(abar_tau) x_zf, and
+        x = x - P x + x_zf after i = 0, where P u = Re ifft2(M fft2(u)) and x_zf = Re ifft2(M y).
+        The result matches the measured k-space to fp32 rounding."""
+        zf, m = self._kspace_inputs(kspace, kmask)
+        img, prog = self._inpaint_start(zf, z_pos)
+        z_pos = self._z_tensor(z_pos, img.shape[0], img.device)
+        return self._inpaint_ddpm(img, (zf, m), prog, lambda x, t: self.model(x, t, z_pos),
+                                  kspace=True)
+
+    @torch.no_grad()
+    def reconstruct_dpmpp(self, kspace, kmask, z_pos=0.5, num_steps=20):
+        """reconstruct() with DPM-Solver++(2M) in `num_steps` UNet calls (not in the reference):
+        after each step, with tau the next timestep (-1 after the last),
+        x = x - P(x - sqrt(1 - abar_tau) x_T) + sqrt(abar_tau) x_zf.  Nothing is drawn after x_T."""
+        table = self._dpmpp_table(self.timesteps - 1, num_steps)
+        zf, m = self._kspace_inputs(kspace, kmask)
+        img, prog = self._inpaint_start(zf, z_pos)
+        z_pos = self._z_tensor(z_pos, img.shape[0], img.device)
+        return self._sample_dpmpp(img, table, prog, lambda x, t: self.model(x, t, z_pos),
+                                  inpaint=(zf, m), kspace=True)
+
+    @torch.no_grad()
     def calc_bpd_loop(self, x_start, z_pos):
         """The variational bound on -log p(x_start) in bits per dimension (not in the reference;
         improved-diffusion's calc_bpd_loop for this fixed-small-variance model), for slices in

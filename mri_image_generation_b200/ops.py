@@ -270,6 +270,37 @@ def inpaint_merge(x, known, mask, t, t_delta: int, sqrt_ac, sqrt_1mac, noise=Non
                "mri_inpaint_merge")
 
 
+def kspace_work_bytes(samples: int, channels: int, H: int, W: int) -> int:
+    """Bytes of kspace_merge's complex work buffer; MriError when H or W is over 512."""
+    import ctypes as C
+    out = C.c_size_t(0)
+    _lib.check(_lib.load().mri_kspace_work_bytes(int(samples), int(channels), int(H), int(W),
+                                                 C.byref(out)), "mri_kspace_work_bytes")
+    return int(out.value)
+
+
+def kspace_merge(x, x_zf, kmask, t, t_delta: int, sqrt_ac, sqrt_1mac, work=None, noise=None,
+                 rng: Optional[DeviceRng] = None, rng_skip: int = 0) -> None:
+    """k-space data consistency in place on x (B, C, H, W) fp32: x = x - P(x - s1m z) + sac x_zf
+    with tau = t + t_delta per sample (x - P x + x_zf at tau < 0), P u = Re ifft2(M fft2(u)) in
+    the orthonormal convention.  kmask: uint8, one byte per element of x, Hermitian-symmetric.
+    z: `noise`, or with rng the torch.randn_like drawn rng_skip past the generator offset.
+    work: a uint8 buffer of at least kspace_work_bytes (None: allocated here)."""
+    _chk_contig(x, x_zf, kmask, noise, work)
+    assert x.dim() == 4 and x.dtype == x_zf.dtype == torch.float32 and kmask.dtype == torch.uint8
+    assert x_zf.numel() == kmask.numel() == x.numel() and t.dtype == torch.int64
+    assert noise is None or (noise.dtype == torch.float32 and noise.numel() == x.numel())
+    B, C, H, W = x.shape
+    if work is None:
+        work = torch.empty(kspace_work_bytes(B, C, H, W), dtype=torch.uint8, device=x.device)
+    _lib.check(_lib.load().mri_kspace_merge(_p(x), _p(x_zf), _p(kmask), _p(noise),
+                                            _p(rng.state) if rng is not None else None,
+                                            int(rng_skip), _p(t), int(t_delta), _p(sqrt_ac),
+                                            _p(sqrt_1mac), _p(work), work.numel() * work.element_size(),
+                                            B, C, H, W, _s()),
+               "mri_kspace_merge")
+
+
 def repaint_undo(x, t, alphas, betas, noise=None, rng: Optional[DeviceRng] = None,
                  rng_skip: int = 0) -> None:
     """RePaint's undo step in place: x = sqrt(alphas[l + 1]) * x + sqrt(betas[l + 1]) * z with
