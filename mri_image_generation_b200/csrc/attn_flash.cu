@@ -17,7 +17,8 @@
 //              second MMA; at the end O / l is written to the token-major output.
 // Operand layouts: Q, K rows come straight from the qkv GEMM's token-major output [B][n][3C]
 // (d contiguous = K-major for both operands of S); V^T comes from the kvT GEMM's output
-// [B][rows][npad] (keys contiguous = K-major B operand of P V).
+// [B][rows][npad] (keys contiguous = K-major B operand of P V).  Precondition: V^T columns
+// [n, npad) must be finite -- the masked keys meet P = 0 there, and 0 * NaN is NaN.
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
