@@ -327,6 +327,49 @@ int mri_kspace_merge(float* x, const float* x_zf, const uint8_t* kmask, const fl
                      const uint64_t* rng, uint64_t rng_skip, const int64_t* t, int64_t t_delta,
                      const float* sqrt_ac, const float* sqrt_1mac, void* work, size_t work_bytes,
                      int samples, int channels, int H, int W, void* stream);
+/* mri_kspace3d_work_bytes: the size of mri_dc_project3d's work buffer: samples * channels * D * H *
+ * (W / 2 + 1) complex fp32 values (rounded up to 256 bytes), then one fp64 partial sum per 16 rows
+ * of every (sample, channel) volume.  D, H and W must be at most 512. */
+int mri_kspace3d_work_bytes(int samples, int channels, int D, int H, int W, size_t* bytes_out);
+/* mri_dc_project3d: the k-space data term of measurement-guided sampling (not in the reference),
+ * per (sample, channel) volume of u (fp32 NCDHW, D x H x W):
+ *     g = Re F^-1(M . F u) - x_zf,        gg[n] = sum over sample n of g^2   (fp32 out)
+ * F the orthonormal unshifted 3-D DFT over (D, H, W), M = kmask (one uint8 per element of u,
+ * nonzero = measured) and MUST be Hermitian-symmetric, M(k) = M(-k): only the half spectrum
+ * (W / 2 + 1 bins) is formed, as in mri_kspace_merge.  x_zf, g: fp32 in u's layout.  Five DFT
+ * launches (rows, forward H, forward D . M . inverse D, inverse H, inverse rows + g), each a direct
+ * fp32 summation against an exactly indexed sincospi twiddle table (the sums of mri_kspace_merge),
+ * and one reduction: gg is summed in fp64 in a fixed order, so two launches are bit-identical.
+ * work: caller-owned, at least mri_kspace3d_work_bytes, 8-byte aligned.  D, H, W at most 512. */
+int mri_dc_project3d(const float* u, const float* x_zf, const uint8_t* kmask, float* g, float* gg,
+                     void* work, size_t work_bytes, int samples, int channels, int D, int H, int W,
+                     void* stream);
+/* mri_dc_mask: the image-space data term of measurement-guided sampling (not in the reference):
+ *     g = mask ? 0 : u - known,           gg[n] = sum over sample n of g^2   (fp32 out)
+ * mask: one uint8 per element, nonzero = regenerate (known is not read there), 0 = keep; u, known,
+ * g fp32 of samples * per_sample elements.  gg is summed in fp64 in a fixed order.  work: at least
+ * 1024 bytes per sample, 8-byte aligned.  At most 65535 samples. */
+int mri_dc_mask(const float* u, const float* known, const uint8_t* mask, float* g, float* gg, void* work,
+                size_t work_bytes, int samples, int64_t per_sample, void* stream);
+/* mri_guided_x0: the clean estimate of a guided step, divided by the latent scale (not in the
+ * reference), per element with ts = t[n]:
+ *     out = (z - sqrt_1mac[ts]*eps) / sqrt_ac[ts] * inv_s[0]
+ * fp32 with round-to-nearest in that order.  eps as the step ops read it: fp32 in z's layout
+ * (eps_nhwc_ldc = 0) or the bf16 channels-last UNet output [n][spatial][ldc].  inv_s: one device
+ * fp32 value (1 / latent scale). */
+int mri_guided_x0(const float* z, const void* eps, int eps_nhwc_ldc, int channels, const int64_t* t,
+                  const float* sqrt_ac, const float* sqrt_1mac, const float* inv_s, float* out,
+                  int samples, int64_t per_sample, void* stream);
+/* mri_guided_eps: the guided noise prediction (not in the reference; DPS's normalisation, Chung et
+ * al. ICLR 2023, applied to the clean estimate as MPGD, He et al. ICLR 2024), per element with
+ * ts = t[n] and c = lam[0] / sqrt(gg[n]) (c = 0 when gg[n] = 0):
+ *     delta = -c * (dz * inv_s[0]),   out = eps - (sqrt_ac[ts] / sqrt_1mac[ts]) * delta
+ * and out = eps exactly where c = 0.  dz: the decoder's input gradient D^T g (fp32 in out's
+ * layout), gg: mri_dc_project3d's / mri_dc_mask's sums, lam / inv_s: one device fp32 value each.
+ * eps as for mri_guided_x0; out: fp32 NCDHW, the eps an unchanged reverse-step update then reads. */
+int mri_guided_eps(const void* eps, int eps_nhwc_ldc, int channels, const float* dz, const float* gg,
+                   const float* lam, const float* inv_s, const int64_t* t, const float* sqrt_ac,
+                   const float* sqrt_1mac, float* out, int samples, int64_t per_sample, void* stream);
 /* mri_repaint_undo: RePaint's undo step (not in the reference), in place per element with
  * l = t[n] in [-1, T - 2] per sample:
  *     x = sqrt(alphas[l + 1])*x + sqrt(betas[l + 1])*z

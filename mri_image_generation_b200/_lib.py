@@ -156,6 +156,11 @@ SIGNATURES = {
     "mri_kspace_work_bytes": (_i, [_i, _i, _i, _i, _vp]),
     "mri_kspace_merge": (_i, [_vp, _vp, _vp, _vp, _vp, _u64, _vp, _i64, _vp, _vp, _vp, C.c_size_t, _i,
                               _i, _i, _i, _vp]),
+    "mri_kspace3d_work_bytes": (_i, [_i, _i, _i, _i, _i, _vp]),
+    "mri_dc_project3d": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, C.c_size_t, _i, _i, _i, _i, _i, _vp]),
+    "mri_dc_mask": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, C.c_size_t, _i, _i64, _vp]),
+    "mri_guided_x0": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _i64, _vp]),
+    "mri_guided_eps": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _vp]),
     "mri_repaint_undo": (_i, [_vp, _vp, _vp, _u64, _vp, _vp, _vp, _i, _i64, _vp]),
     "mri_vb_terms": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _i,
                           _i, _i64, _vp]),

@@ -159,6 +159,9 @@ class BackwardMixin:
         self._final: List[Tuple[int, torch.Tensor, torch.Tensor, Optional[torch.Tensor], int, int]] = []
         self._final_tables: Dict[Tuple[int, int], Optional[tuple]] = {}
         self._fuse_final = os.environ.get("MRI_NO_FINAL_FUSION") != "1"
+        # False: data gradients only -- no weight-gradient launches, bias / norm-parameter sums or
+        # final gathers, and no gradient arena (a decoder differentiated w.r.t. its input alone)
+        self.wgrad = True
 
     def badd(self, name: str, fn: Callable[[], None]) -> None:
         self.bwd_names.append(name)
@@ -319,9 +322,10 @@ class BackwardMixin:
         C = r.y.shape[-1]
         if r.residual is not None:
             self.pass_grad(r.residual, dy)
-        self._bwd_bias_and_tproj(dy, C, r.bias_params, r.tproj_off, r.name)
+        if self.wgrad:
+            self._bwd_bias_and_tproj(dy, C, r.bias_params, r.tproj_off, r.name)
         # ---- weight gradient over the forward k-table ------------------------------------
-        if r.weight is not None:
+        if r.weight is not None and self.wgrad:
             pl = r.plan
             K = pl.n_kb * P.BLOCK_K
             dw = self.zeros_each_bwd(pl.n_class, max(r.cout, 8), K)
@@ -429,13 +433,14 @@ class BackwardMixin:
         xs, st, cpg = x.t, x.stats, x.cpg
         self.badd(f"gn_bwd_reduce:{r.name}", lambda: ops.gn_bwd_reduce(
             xs, dy, st, gamma, beta, sums, B, S, C, r.groups, cpg, r.eps, r.silu))
-        if r.gparam is not None:   # padded copies feed the kernels; the real channels come first
-            gg, gb = self.pg(r.gparam), self.pg(r.bparam)
-        else:
-            gg = self.pg(r.gamma)[r.c_off:r.c_off + C]
-            gb = self.pg(r.beta)[r.c_off:r.c_off + C]
-        self.bfinal_bsum(gg, sums[2], "gn_param_grad")
-        self.bfinal_bsum(gb, sums[1], "gn_param_grad")
+        if self.wgrad:
+            if r.gparam is not None:   # padded copies feed the kernels; the real channels come first
+                gg, gb = self.pg(r.gparam), self.pg(r.bparam)
+            else:
+                gg = self.pg(r.gamma)[r.c_off:r.c_off + C]
+                gb = self.pg(r.beta)[r.c_off:r.c_off + C]
+            self.bfinal_bsum(gg, sums[2], "gn_param_grad")
+            self.bfinal_bsum(gb, sums[1], "gn_param_grad")
         if r.tproj_off is not None:
             dst = self.dtproj[:, r.tproj_off:r.tproj_off + C]
             self.badd("dtproj", lambda: ops.copy_cast(sums[0], dst))

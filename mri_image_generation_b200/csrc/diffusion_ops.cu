@@ -478,6 +478,100 @@ __device__ __forceinline__ void ks_twiddles(float2* tw, int n) {
   }
 }
 
+// The four DFT sums the 2-D and 3-D passes share, each in one fixed FMA order.
+// Bin k of the forward real DFT of kKsRows rows held as u[W][kKsRows].
+__device__ __forceinline__ void ks_row_fwd(const float2* tw, const float* u, int W, int k,
+                                           float (&re)[kKsRows], float (&im)[kKsRows]) {
+#pragma unroll
+  for (int r = 0; r < kKsRows; ++r) re[r] = im[r] = 0.f;
+  int idx = 0;
+  for (int w = 0; w < W; ++w) {
+    const float2 c = tw[idx];
+    const float4* up = reinterpret_cast<const float4*>(u + w * kKsRows);
+#pragma unroll
+    for (int q = 0; q < kKsRows / 4; ++q) {
+      const float4 v = up[q];
+      const float vv[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+      for (int m = 0; m < 4; ++m) {
+        re[4 * q + m] = fmaf(vv[m], c.x, re[4 * q + m]);
+        im[4 * q + m] = fmaf(vv[m], c.y, im[4 * q + m]);
+      }
+    }
+    idx += k;
+    if (idx >= W) idx -= W;
+  }
+}
+
+// Sample w of Re(inverse DFT) of kKsRows half spectra held as us[Wh][kKsRows] (bins other than 0
+// and W/2 already doubled), unscaled.
+__device__ __forceinline__ void ks_row_inv(const float2* tw, const float2* us, int W, int Wh, int w,
+                                           float (&acc)[kKsRows]) {
+#pragma unroll
+  for (int r = 0; r < kKsRows; ++r) acc[r] = 0.f;
+  int idx = 0;
+  for (int k = 0; k < Wh; ++k) {
+    const float2 c = tw[idx];          // Re(v exp(+i theta)) = v.x cos - v.y sin = v.x c.x + v.y c.y
+    const float4* vp = reinterpret_cast<const float4*>(us + k * kKsRows);
+#pragma unroll
+    for (int q = 0; q < kKsRows / 2; ++q) {
+      const float4 v = vp[q];
+      acc[2 * q] = fmaf(v.y, c.y, fmaf(v.x, c.x, acc[2 * q]));
+      acc[2 * q + 1] = fmaf(v.w, c.y, fmaf(v.z, c.x, acc[2 * q + 1]));
+    }
+    idx += w;
+    if (idx >= W) idx -= W;
+  }
+}
+
+// Bin m of the forward DFT of length N of kKsCols complex columns held as U[N][kKsCols]; thread m
+// sums over n, so the U loads are warp broadcasts.
+__device__ __forceinline__ void ks_col_fwd(const float2* tw, const float2* U, int N, int m,
+                                           float (&re)[kKsCols], float (&im)[kKsCols]) {
+#pragma unroll
+  for (int j = 0; j < kKsCols; ++j) re[j] = im[j] = 0.f;
+  int idx = 0;
+  for (int h = 0; h < N; ++h) {
+    const float2 c = tw[idx];
+    const float4* up = reinterpret_cast<const float4*>(U + h * kKsCols);
+#pragma unroll
+    for (int q = 0; q < kKsCols / 2; ++q) {
+      const float4 v = up[q];
+      re[2 * q] = fmaf(-v.y, c.y, fmaf(v.x, c.x, re[2 * q]));
+      im[2 * q] = fmaf(v.y, c.x, fmaf(v.x, c.y, im[2 * q]));
+      re[2 * q + 1] = fmaf(-v.w, c.y, fmaf(v.z, c.x, re[2 * q + 1]));
+      im[2 * q + 1] = fmaf(v.w, c.x, fmaf(v.z, c.y, im[2 * q + 1]));
+    }
+    idx += m;
+    if (idx >= N) idx -= N;
+  }
+}
+
+// Sample h of the inverse DFT (unscaled) of V[N][kKsCols]: exp(+2 pi i h m / N) = conj(tw); rows
+// of V with live[m] == 0 add nothing
+__device__ __forceinline__ void ks_col_inv(const float2* tw, const float2* V, const int* live, int N,
+                                           int h, float (&re)[kKsCols], float (&im)[kKsCols]) {
+#pragma unroll
+  for (int j = 0; j < kKsCols; ++j) re[j] = im[j] = 0.f;
+  int idx = 0;
+  for (int m = 0; m < N; ++m) {
+    if (live[m]) {
+      const float2 c = tw[idx];
+      const float4* vp = reinterpret_cast<const float4*>(V + m * kKsCols);
+#pragma unroll
+      for (int q = 0; q < kKsCols / 2; ++q) {
+        const float4 v = vp[q];
+        re[2 * q] = fmaf(v.y, c.y, fmaf(v.x, c.x, re[2 * q]));
+        im[2 * q] = fmaf(-v.x, c.y, fmaf(v.y, c.x, im[2 * q]));
+        re[2 * q + 1] = fmaf(v.w, c.y, fmaf(v.z, c.x, re[2 * q + 1]));
+        im[2 * q + 1] = fmaf(-v.z, c.y, fmaf(v.w, c.x, im[2 * q + 1]));
+      }
+    }
+    idx += h;
+    if (idx >= N) idx -= N;
+  }
+}
+
 template <bool RNG>
 __global__ void __launch_bounds__(kKsThreadsA) kspace_rows_fwd_kernel(const KspaceArgs a) {
   extern __shared__ float4 ks_smem[];
@@ -507,104 +601,93 @@ __global__ void __launch_bounds__(kKsThreadsA) kspace_rows_fwd_kernel(const Kspa
   __syncthreads();
   for (int k = threadIdx.x; k < a.Wh; k += blockDim.x) {
     float re[kKsRows], im[kKsRows];
-#pragma unroll
-    for (int r = 0; r < kKsRows; ++r) re[r] = im[r] = 0.f;
-    int idx = 0;
-    for (int w = 0; w < a.W; ++w) {
-      const float2 c = tw[idx];
-      const float4* up = reinterpret_cast<const float4*>(u + w * kKsRows);
-#pragma unroll
-      for (int q = 0; q < kKsRows / 4; ++q) {
-        const float4 v = up[q];
-        const float vv[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-        for (int m = 0; m < 4; ++m) {
-          re[4 * q + m] = fmaf(vv[m], c.x, re[4 * q + m]);
-          im[4 * q + m] = fmaf(vv[m], c.y, im[4 * q + m]);
-        }
-      }
-      idx += k;
-      if (idx >= a.W) idx -= a.W;
-    }
+    ks_row_fwd(tw, u, a.W, k, re, im);
 #pragma unroll
     for (int r = 0; r < kKsRows; ++r)
       if (h0 + r < a.H) a.work[(plane * a.H + h0 + r) * a.Wh + k] = make_float2(re[r], im[r]);
   }
 }
 
-__global__ void __launch_bounds__(kKsThreadsB) kspace_cols_kernel(const KspaceArgs a) {
+// The column passes over a complex work buffer of half spectra: `line` indexes the 1-D transforms
+// of length N, element n of column c of line l at work[(l / inner) * outer + (l % inner) * inner_ld
+// + n * ld + c], its mask byte likewise with the m_* strides.
+struct KsColGeom {
+  float2* work;
+  const uint8_t* mask;
+  int N, Wh, inner;
+  long long outer, inner_ld, ld;
+  long long m_outer, m_inner_ld, m_ld;
+};
+
+// kKsCols columns of one line a block.  kMode 0: forward DFT; 1: forward DFT, times M, inverse DFT;
+// 2: inverse DFT.  In place: the block reads its whole tile before it writes.
+template <int kMode>
+__global__ void __launch_bounds__(kKsThreadsB) kspace_cols_kernel(const KsColGeom g) {
   extern __shared__ float4 ks_smem[];
-  const int H = a.H;
+  const int N = g.N;
   float2* tw = reinterpret_cast<float2*>(ks_smem);
-  float2* U = tw + ks_tw_len(H);       // [H][kKsCols]: the row spectra, then their inverse
-  float2* V = U + H * kKsCols;         // [H][kKsCols]: M . column spectra
-  int* live = reinterpret_cast<int*>(V + H * kKsCols);   // row m of V has a measured sample
-  const int nct = (a.Wh + kKsCols - 1) / kKsCols;
-  const long long plane = blockIdx.x / nct;
+  float2* U = tw + ks_tw_len(N);       // [N][kKsCols]: the input spectra
+  float2* V = U + N * kKsCols;         // [N][kKsCols]: what the inverse reads
+  int* live = reinterpret_cast<int*>(V + N * kKsCols);   // row m of V has a measured sample
+  const int nct = (g.Wh + kKsCols - 1) / kKsCols;
+  const long long line = blockIdx.x / nct;
   const int c0 = (int)(blockIdx.x % nct) * kKsCols;
-  ks_twiddles(tw, H);
-  for (int i = threadIdx.x; i < H * kKsCols; i += blockDim.x) {
-    const int h = i / kKsCols, c = c0 + i % kKsCols;
-    U[i] = c < a.Wh ? a.work[(plane * H + h) * a.Wh + c] : make_float2(0.f, 0.f);
+  float2* base = g.work + (line / g.inner) * g.outer + (line % g.inner) * g.inner_ld + c0;
+  ks_twiddles(tw, N);
+  float2* in = kMode == 2 ? V : U;
+  for (int i = threadIdx.x; i < N * kKsCols; i += blockDim.x) {
+    const int n = i / kKsCols, c = i % kKsCols;
+    in[i] = c0 + c < g.Wh ? base[n * g.ld + c] : make_float2(0.f, 0.f);
   }
+  if (kMode == 2)
+    for (int m = threadIdx.x; m < N; m += blockDim.x) live[m] = 1;
   __syncthreads();
-  // forward: thread m sums over h for the tile's columns, so the U loads are warp broadcasts
-  for (int m = threadIdx.x; m < H; m += blockDim.x) {
-    float re[kKsCols], im[kKsCols];
+  if (kMode != 2) {
+    const uint8_t* mbase = g.mask + (line / g.inner) * g.m_outer + (line % g.inner) * g.m_inner_ld + c0;
+    for (int m = threadIdx.x; m < N; m += blockDim.x) {
+      float re[kKsCols], im[kKsCols];
+      ks_col_fwd(tw, U, N, m, re, im);
+      if (kMode == 0) {
 #pragma unroll
-    for (int j = 0; j < kKsCols; ++j) re[j] = im[j] = 0.f;
-    int idx = 0;
-    for (int h = 0; h < H; ++h) {
-      const float2 c = tw[idx];
-      const float4* up = reinterpret_cast<const float4*>(U + h * kKsCols);
-#pragma unroll
-      for (int q = 0; q < kKsCols / 2; ++q) {
-        const float4 v = up[q];
-        re[2 * q] = fmaf(-v.y, c.y, fmaf(v.x, c.x, re[2 * q]));
-        im[2 * q] = fmaf(v.y, c.x, fmaf(v.x, c.y, im[2 * q]));
-        re[2 * q + 1] = fmaf(-v.w, c.y, fmaf(v.z, c.x, re[2 * q + 1]));
-        im[2 * q + 1] = fmaf(v.w, c.x, fmaf(v.z, c.y, im[2 * q + 1]));
+        for (int j = 0; j < kKsCols; ++j)
+          if (c0 + j < g.Wh) base[m * g.ld + j] = make_float2(re[j], im[j]);
+        continue;
       }
-      idx += m;
-      if (idx >= H) idx -= H;
-    }
-    const uint8_t* mrow = a.mask + (plane * H + m) * a.W + c0;
-    int any = 0;
+      const uint8_t* mrow = mbase + m * g.m_ld;
+      int any = 0;
 #pragma unroll
-    for (int j = 0; j < kKsCols; ++j) {
-      const bool keep = c0 + j < a.Wh && mrow[j] != 0;
-      any |= keep;
-      V[m * kKsCols + j] = keep ? make_float2(re[j], im[j]) : make_float2(0.f, 0.f);
+      for (int j = 0; j < kKsCols; ++j) {
+        const bool keep = c0 + j < g.Wh && mrow[j] != 0;
+        any |= keep;
+        V[m * kKsCols + j] = keep ? make_float2(re[j], im[j]) : make_float2(0.f, 0.f);
+      }
+      live[m] = any;
     }
-    live[m] = any;
+    if (kMode == 0) return;
+    __syncthreads();
   }
-  __syncthreads();
-  // inverse: exp(+2 pi i h m / H) = conj(tw); rows of V with no measured sample add nothing
-  for (int h = threadIdx.x; h < H; h += blockDim.x) {
+  for (int h = threadIdx.x; h < N; h += blockDim.x) {
     float re[kKsCols], im[kKsCols];
-#pragma unroll
-    for (int j = 0; j < kKsCols; ++j) re[j] = im[j] = 0.f;
-    int idx = 0;
-    for (int m = 0; m < H; ++m) {
-      if (live[m]) {
-        const float2 c = tw[idx];
-        const float4* vp = reinterpret_cast<const float4*>(V + m * kKsCols);
-#pragma unroll
-        for (int q = 0; q < kKsCols / 2; ++q) {
-          const float4 v = vp[q];
-          re[2 * q] = fmaf(v.y, c.y, fmaf(v.x, c.x, re[2 * q]));
-          im[2 * q] = fmaf(-v.x, c.y, fmaf(v.y, c.x, im[2 * q]));
-          re[2 * q + 1] = fmaf(v.w, c.y, fmaf(v.z, c.x, re[2 * q + 1]));
-          im[2 * q + 1] = fmaf(-v.z, c.y, fmaf(v.w, c.x, im[2 * q + 1]));
-        }
-      }
-      idx += h;
-      if (idx >= H) idx -= H;
-    }
-    float2* out = a.work + (plane * H + h) * a.Wh + c0;
+    ks_col_inv(tw, V, live, N, h, re, im);
+    float2* out = base + h * g.ld;
 #pragma unroll
     for (int j = 0; j < kKsCols; ++j)
-      if (c0 + j < a.Wh) out[j] = make_float2(re[j], im[j]);
+      if (c0 + j < g.Wh) out[j] = make_float2(re[j], im[j]);
+  }
+}
+
+// the half spectra of kKsRows rows starting at row h0 of `plane` into us[Wh][kKsRows], bins other
+// than 0 and W/2 doubled: Re of the full inverse sum counts them twice (their mirror)
+__device__ __forceinline__ void ks_load_half_rows(float2* us, const float2* work, long long plane, int rows,
+                                                  int h0, int W, int Wh) {
+  for (int i = threadIdx.x; i < kKsRows * Wh; i += blockDim.x) {
+    const int r = i / Wh, k = i - r * Wh;
+    float2 v = make_float2(0.f, 0.f);
+    if (h0 + r < rows) {
+      v = work[(plane * rows + h0 + r) * Wh + k];
+      if (k != 0 && 2 * k != W) v = make_float2(2.f * v.x, 2.f * v.y);
+    }
+    us[k * kKsRows + r] = v;
   }
 }
 
@@ -617,36 +700,13 @@ __global__ void __launch_bounds__(kKsThreadsC) kspace_rows_inv_kernel(const Kspa
   const int h0 = (int)(blockIdx.x % nrb) * kKsRows;
   const long long tau = a.t[plane / a.channels] + a.t_delta;
   ks_twiddles(tw, a.W);
-  // Re of the full inverse sum: bins 0 and W/2 (W even) once, every other bin twice (its mirror)
-  for (int i = threadIdx.x; i < kKsRows * a.Wh; i += blockDim.x) {
-    const int r = i / a.Wh, k = i - r * a.Wh;
-    float2 v = make_float2(0.f, 0.f);
-    if (h0 + r < a.H) {
-      v = a.work[(plane * a.H + h0 + r) * a.Wh + k];
-      if (k != 0 && 2 * k != a.W) v = make_float2(2.f * v.x, 2.f * v.y);
-    }
-    us[k * kKsRows + r] = v;
-  }
+  ks_load_half_rows(us, a.work, plane, a.H, h0, a.W, a.Wh);
   __syncthreads();
   const float scale = (float)(1.0 / ((double)a.H * a.W));
   const float sac = tau < 0 ? 1.f : __ldg(a.sqrt_ac + tau);
   for (int w = threadIdx.x; w < a.W; w += blockDim.x) {
     float acc[kKsRows];
-#pragma unroll
-    for (int r = 0; r < kKsRows; ++r) acc[r] = 0.f;
-    int idx = 0;
-    for (int k = 0; k < a.Wh; ++k) {
-      const float2 c = tw[idx];          // Re(v exp(+i theta)) = v.x cos - v.y sin = v.x c.x + v.y c.y
-      const float4* vp = reinterpret_cast<const float4*>(us + k * kKsRows);
-#pragma unroll
-      for (int q = 0; q < kKsRows / 2; ++q) {
-        const float4 v = vp[q];
-        acc[2 * q] = fmaf(v.y, c.y, fmaf(v.x, c.x, acc[2 * q]));
-        acc[2 * q + 1] = fmaf(v.w, c.y, fmaf(v.z, c.x, acc[2 * q + 1]));
-      }
-      idx += w;
-      if (idx >= a.W) idx -= a.W;
-    }
+    ks_row_inv(tw, us, a.W, a.Wh, w, acc);
 #pragma unroll
     for (int r = 0; r < kKsRows; ++r) {
       if (h0 + r >= a.H) break;
@@ -654,6 +714,158 @@ __global__ void __launch_bounds__(kKsThreadsC) kspace_rows_inv_kernel(const Kspa
       const float add = tau < 0 ? a.zf[e] : __fmul_rn(sac, a.zf[e]);
       a.x[e] = __fadd_rn(__fsub_rn(a.x[e], __fmul_rn(acc[r], scale)), add);
     }
+  }
+}
+
+// ------------------------------------------------------------------------------------------
+// Measurement-guided sampling of the 3-D latent model (mri_dc_project3d, mri_dc_mask,
+// mri_guided_x0, mri_guided_eps).  The data terms write g = P u - x_zf and the per-sample
+// ||g||^2; the sums of squares are fp64, per block in a fixed tree order, then per sample over
+// the blocks in index order (dc_norm_kernel): no atomics, so a replay is bit-reproducible.
+// ------------------------------------------------------------------------------------------
+constexpr int kDcMaskBlocks = 128;     // blocks per sample of the image-mask term
+
+// the fp64 sum of v over the block in a fixed order; valid in thread 0
+__device__ __forceinline__ double block_sum_fixed(double v, double* red) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  if (lane == 0) red[wid] = v;
+  __syncthreads();
+  double s = 0.0;
+  if (threadIdx.x == 0)
+    for (int i = 0; i < (int)(blockDim.x >> 5); ++i) s += red[i];
+  return s;
+}
+
+// gg[n] = sum of partial[n * per][0 .. per), in order per thread, then a fixed tree
+__global__ void __launch_bounds__(256) dc_norm_kernel(const double* partial, int per, float* gg) {
+  __shared__ double red[8];
+  const double* p = partial + (long long)blockIdx.x * per;
+  double v = 0.0;
+  for (int i = threadIdx.x; i < per; i += blockDim.x) v += p[i];
+  const double s = block_sum_fixed(v, red);
+  if (threadIdx.x == 0) gg[blockIdx.x] = (float)s;
+}
+
+struct Dc3Args {
+  const float* u;
+  const float* zf;
+  float* g;
+  float2* work;
+  double* partial;     // one per block of the inverse row pass
+  int rows, W, Wh;     // rows = D * H per plane
+};
+
+// forward real row DFT of u, rows of all planes: work[plane][D][H][Wh]
+__global__ void __launch_bounds__(kKsThreadsA) dc3_rows_fwd_kernel(const Dc3Args a) {
+  extern __shared__ float4 ks_smem[];
+  float2* tw = reinterpret_cast<float2*>(ks_smem);
+  float* u = reinterpret_cast<float*>(tw + ks_tw_len(a.W));    // [W][kKsRows]
+  const int nrb = (a.rows + kKsRows - 1) / kKsRows;
+  const long long plane = blockIdx.x / nrb;
+  const int h0 = (int)(blockIdx.x % nrb) * kKsRows;
+  ks_twiddles(tw, a.W);
+  for (int i = threadIdx.x; i < kKsRows * a.W; i += blockDim.x) {
+    const int r = i / a.W, w = i - r * a.W;
+    u[w * kKsRows + r] = h0 + r < a.rows ? a.u[(plane * a.rows + h0 + r) * a.W + w] : 0.f;
+  }
+  __syncthreads();
+  for (int k = threadIdx.x; k < a.Wh; k += blockDim.x) {
+    float re[kKsRows], im[kKsRows];
+    ks_row_fwd(tw, u, a.W, k, re, im);
+#pragma unroll
+    for (int r = 0; r < kKsRows; ++r)
+      if (h0 + r < a.rows) a.work[(plane * a.rows + h0 + r) * a.Wh + k] = make_float2(re[r], im[r]);
+  }
+}
+
+// inverse real row DFT, g = P u - x_zf, and this block's sum of g^2
+__global__ void __launch_bounds__(kKsThreadsC) dc3_rows_inv_kernel(const Dc3Args a, float scale) {
+  extern __shared__ float4 ks_smem[];
+  __shared__ double red[kKsThreadsC / 32];
+  float2* tw = reinterpret_cast<float2*>(ks_smem);
+  float2* us = tw + ks_tw_len(a.W);                 // [Wh][kKsRows]
+  const int nrb = (a.rows + kKsRows - 1) / kKsRows;
+  const long long plane = blockIdx.x / nrb;
+  const int h0 = (int)(blockIdx.x % nrb) * kKsRows;
+  ks_twiddles(tw, a.W);
+  ks_load_half_rows(us, a.work, plane, a.rows, h0, a.W, a.Wh);
+  __syncthreads();
+  double ss = 0.0;
+  for (int w = threadIdx.x; w < a.W; w += blockDim.x) {
+    float acc[kKsRows];
+    ks_row_inv(tw, us, a.W, a.Wh, w, acc);
+#pragma unroll
+    for (int r = 0; r < kKsRows; ++r) {
+      if (h0 + r >= a.rows) break;
+      const long long e = (plane * a.rows + h0 + r) * a.W + w;
+      const float gv = __fsub_rn(__fmul_rn(acc[r], scale), a.zf[e]);
+      a.g[e] = gv;
+      ss += (double)gv * gv;
+    }
+  }
+  const double s = block_sum_fixed(ss, red);
+  if (threadIdx.x == 0) a.partial[blockIdx.x] = s;
+}
+
+// g = mask ? 0 : u - known (select: known is not read where mask != 0), grid (kDcMaskBlocks, samples)
+__global__ void __launch_bounds__(256)
+dc_mask_kernel(const float* u, const float* known, const uint8_t* mask, float* g, double* partial,
+               long long per_sample) {
+  __shared__ double red[8];
+  const long long off = (long long)blockIdx.y * per_sample;
+  double ss = 0.0;
+  for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < per_sample;
+       j += (long long)gridDim.x * blockDim.x) {
+    const long long e = off + j;
+    const float gv = mask[e] != 0 ? 0.f : __fsub_rn(u[e], known[e]);
+    g[e] = gv;
+    ss += (double)gv * gv;
+  }
+  const double s = block_sum_fixed(ss, red);
+  if (threadIdx.x == 0) partial[(long long)blockIdx.y * gridDim.x + blockIdx.x] = s;
+}
+
+// out = (z - s1m[t] eps) / sac[t] * inv_s per element (step 2 of the guided step)
+__global__ void __launch_bounds__(256)
+guided_x0_kernel(const float* z, const void* eps, int ldc, int channels, const int64_t* t,
+                 const float* sqrt_ac, const float* sqrt_1mac, const float* inv_s, float* out,
+                 long long per_sample, long long numel) {
+  const long long spatial = per_sample / (channels > 0 ? channels : 1);
+  const float is = *inv_s;
+  for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < numel;
+       e += (long long)gridDim.x * blockDim.x) {
+    const long long n = e / per_sample;
+    const int64_t ts = t[n];
+    const float ev = load_eps(eps, ldc, spatial, per_sample, n, e - n * per_sample);
+    const float x0 = __fdiv_rn(__fsub_rn(z[e], __fmul_rn(__ldg(sqrt_1mac + ts), ev)), __ldg(sqrt_ac + ts));
+    out[e] = __fmul_rn(x0, is);
+  }
+}
+
+// eps' = eps - (sac[t] / s1m[t]) * delta, delta = -(lam / sqrt(gg[n])) * (dz * inv_s); eps' = eps
+// where that coefficient is 0 (lam = 0 or ||g|| = 0)
+__global__ void __launch_bounds__(256)
+guided_eps_kernel(const void* eps, int ldc, int channels, const float* dz, const float* gg,
+                  const float* lam, const float* inv_s, const int64_t* t, const float* sqrt_ac,
+                  const float* sqrt_1mac, float* out, long long per_sample, long long numel) {
+  const long long spatial = per_sample / (channels > 0 ? channels : 1);
+  const float l = *lam, is = *inv_s;
+  for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < numel;
+       e += (long long)gridDim.x * blockDim.x) {
+    const long long n = e / per_sample;
+    const int64_t ts = t[n];
+    const float ev = load_eps(eps, ldc, spatial, per_sample, n, e - n * per_sample);
+    const float q = gg[n];
+    const float coef = q > 0.f ? __fdiv_rn(l, __fsqrt_rn(q)) : 0.f;
+    if (coef == 0.f) {
+      out[e] = ev;
+      continue;
+    }
+    const float delta = __fmul_rn(-coef, __fmul_rn(dz[e], is));
+    const float r = __fdiv_rn(__ldg(sqrt_ac + ts), __ldg(sqrt_1mac + ts));
+    out[e] = __fsub_rn(ev, __fmul_rn(r, delta));
   }
 }
 
@@ -1203,6 +1415,19 @@ extern "C" int mri_inpaint_merge(float* x, const float* known, const uint8_t* ma
   return check_launch("inpaint_merge_kernel");
 }
 
+// the column kernels' shared memory, once at the largest size (not re-done inside a graph capture)
+static int ks_configure() {
+  static bool configured = false;
+  if (configured) return 0;
+  void (*kerns[3])(const KsColGeom) = {kspace_cols_kernel<0>, kspace_cols_kernel<1>, kspace_cols_kernel<2>};
+  for (auto k : kerns) {
+    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, ks_smem_b(kKsMaxN));
+    if (e != cudaSuccess) return set_cuda_error(e, "cudaFuncSetAttribute(kspace_cols_kernel)");
+  }
+  configured = true;
+  return 0;
+}
+
 static int kspace_dims(const char* who, int samples, int channels, int H, int W) {
   if (samples < 1 || channels < 1 || H < 1 || W < 1) return set_error(-2, who);
   if (H > kKsMaxN || W > kKsMaxN) return set_error(-2, "mri_kspace_merge: H and W must be at most 512");
@@ -1237,13 +1462,8 @@ extern "C" int mri_kspace_merge(float* x, const float* x_zf, const uint8_t* kmas
     return set_error(-2, "mri_kspace_merge: work smaller than mri_kspace_work_bytes or not 8-byte aligned");
   rc = device_props();
   if (rc) return rc;
-  static bool configured = false;   // once, at the largest size (not re-done inside a graph capture)
-  if (!configured) {
-    cudaError_t e = cudaFuncSetAttribute(kspace_cols_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         ks_smem_b(kKsMaxN));
-    if (e != cudaSuccess) return set_cuda_error(e, "cudaFuncSetAttribute(kspace_cols_kernel)");
-    configured = true;
-  }
+  rc = ks_configure();
+  if (rc) return rc;
   KspaceArgs a;
   a.x = x;
   a.zf = x_zf;
@@ -1267,12 +1487,145 @@ extern "C" int mri_kspace_merge(float* x, const float* x_zf, const uint8_t* kmas
     kspace_rows_fwd_kernel<false><<<rows_grid, kKsThreadsA, ks_smem_a(W), st>>>(a);
   rc = check_launch("kspace_rows_fwd_kernel");
   if (rc) return rc;
-  kspace_cols_kernel<<<(unsigned)(planes * ((a.Wh + kKsCols - 1) / kKsCols)), kKsThreadsB, ks_smem_b(H),
-                       st>>>(a);
+  KsColGeom g{a.work, kmask, H, a.Wh, 1, (long long)H * a.Wh, 0, a.Wh, (long long)H * W, 0, W};
+  kspace_cols_kernel<1><<<(unsigned)(planes * ((a.Wh + kKsCols - 1) / kKsCols)), kKsThreadsB, ks_smem_b(H),
+                          st>>>(g);
   rc = check_launch("kspace_cols_kernel");
   if (rc) return rc;
   kspace_rows_inv_kernel<<<rows_grid, kKsThreadsC, ks_smem_c(W), st>>>(a);
   return check_launch("kspace_rows_inv_kernel");
+}
+
+static int dc3_dims(int samples, int channels, int D, int H, int W) {
+  if (samples < 1 || channels < 1 || D < 1 || H < 1 || W < 1)
+    return set_error(-2, "mri_dc_project3d: empty input");
+  if (D > kKsMaxN || H > kKsMaxN || W > kKsMaxN)
+    return set_error(-2, "mri_dc_project3d: D, H and W must be at most 512");
+  const long long planes = (long long)samples * channels;
+  if (planes * ((D * H + kKsRows - 1) / kKsRows) > 0x7fffffffLL || planes * H * ((W / 2 + 1 + kKsCols - 1) / kKsCols) > 0x7fffffffLL ||
+      planes * D * ((W / 2 + 1 + kKsCols - 1) / kKsCols) > 0x7fffffffLL)
+    return set_error(-2, "mri_dc_project3d: too many rows");
+  return 0;
+}
+
+// the complex half spectra, then the fp64 partial sums of the inverse row pass
+static size_t dc3_spectrum_bytes(int samples, int channels, int D, int H, int W) {
+  const size_t b = (size_t)samples * channels * D * H * (W / 2 + 1) * sizeof(float2);
+  return (b + 255) & ~(size_t)255;
+}
+
+extern "C" int mri_kspace3d_work_bytes(int samples, int channels, int D, int H, int W, size_t* bytes_out) {
+  int rc = dc3_dims(samples, channels, D, H, W);
+  if (rc) return rc;
+  if (bytes_out == nullptr) return set_error(-2, "mri_kspace3d_work_bytes: null output");
+  const size_t nrb = (size_t)(D * H + kKsRows - 1) / kKsRows;
+  *bytes_out = dc3_spectrum_bytes(samples, channels, D, H, W) + (size_t)samples * channels * nrb * sizeof(double);
+  return 0;
+}
+
+extern "C" int mri_dc_project3d(const float* u, const float* x_zf, const uint8_t* kmask, float* g,
+                                float* gg, void* work, size_t work_bytes, int samples, int channels,
+                                int D, int H, int W, void* stream) {
+  size_t need = 0;
+  int rc = mri_kspace3d_work_bytes(samples, channels, D, H, W, &need);
+  if (rc) return rc;
+  if (u == nullptr || x_zf == nullptr || kmask == nullptr || g == nullptr || gg == nullptr || work == nullptr)
+    return set_error(-2, "mri_dc_project3d: null u / x_zf / kmask / g / gg / work");
+  if (work_bytes < need || (reinterpret_cast<uintptr_t>(work) & 7) != 0)
+    return set_error(-2, "mri_dc_project3d: work smaller than mri_kspace3d_work_bytes or not 8-byte aligned");
+  rc = ks_configure();
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long planes = (long long)samples * channels;
+  const int Wh = W / 2 + 1, nct = (Wh + kKsCols - 1) / kKsCols;
+  const int rows = D * H, nrb = (rows + kKsRows - 1) / kKsRows;
+  Dc3Args a;
+  a.u = u;
+  a.zf = x_zf;
+  a.g = g;
+  a.work = static_cast<float2*>(work);
+  a.partial = reinterpret_cast<double*>(static_cast<char*>(work) + dc3_spectrum_bytes(samples, channels, D, H, W));
+  a.rows = rows; a.W = W; a.Wh = Wh;
+  const long long vol = (long long)D * H * Wh, slab = (long long)H * Wh;
+  const long long mvol = (long long)D * H * W, mslab = (long long)H * W;
+  dc3_rows_fwd_kernel<<<(unsigned)(planes * nrb), kKsThreadsA, ks_smem_a(W), st>>>(a);
+  rc = check_launch("dc3_rows_fwd_kernel");
+  if (rc) return rc;
+  // forward along H: line (plane, d)
+  const KsColGeom gh{a.work, nullptr, H, Wh, 1, slab, 0, Wh, 0, 0, 0};
+  kspace_cols_kernel<0><<<(unsigned)(planes * D * nct), kKsThreadsB, ks_smem_b(H), st>>>(gh);
+  rc = check_launch("kspace_cols_kernel<0>");
+  if (rc) return rc;
+  // forward along D, times M, inverse along D: line (plane, h)
+  const KsColGeom gd{a.work, kmask, D, Wh, H, vol, Wh, slab, mvol, W, mslab};
+  kspace_cols_kernel<1><<<(unsigned)(planes * H * nct), kKsThreadsB, ks_smem_b(D), st>>>(gd);
+  rc = check_launch("kspace_cols_kernel<1>");
+  if (rc) return rc;
+  kspace_cols_kernel<2><<<(unsigned)(planes * D * nct), kKsThreadsB, ks_smem_b(H), st>>>(gh);
+  rc = check_launch("kspace_cols_kernel<2>");
+  if (rc) return rc;
+  const float scale = (float)(1.0 / ((double)D * H * W));
+  dc3_rows_inv_kernel<<<(unsigned)(planes * nrb), kKsThreadsC, ks_smem_c(W), st>>>(a, scale);
+  rc = check_launch("dc3_rows_inv_kernel");
+  if (rc) return rc;
+  dc_norm_kernel<<<(unsigned)samples, 256, 0, st>>>(a.partial, (int)(channels * nrb), gg);
+  return check_launch("dc_norm_kernel");
+}
+
+extern "C" int mri_dc_mask(const float* u, const float* known, const uint8_t* mask, float* g, float* gg,
+                           void* work, size_t work_bytes, int samples, int64_t per_sample, void* stream) {
+  if (samples < 1 || per_sample < 1) return set_error(-2, "mri_dc_mask: empty input");
+  if (samples > 65535) return set_error(-2, "mri_dc_mask: at most 65535 samples");
+  if (u == nullptr || known == nullptr || mask == nullptr || g == nullptr || gg == nullptr || work == nullptr)
+    return set_error(-2, "mri_dc_mask: null u / known / mask / g / gg / work");
+  if (work_bytes < (size_t)samples * kDcMaskBlocks * sizeof(double) || (reinterpret_cast<uintptr_t>(work) & 7) != 0)
+    return set_error(-2, "mri_dc_mask: work smaller than 1024 bytes per sample or not 8-byte aligned");
+  double* partial = static_cast<double*>(work);
+  cudaStream_t st = (cudaStream_t)stream;
+  dc_mask_kernel<<<dim3(kDcMaskBlocks, (unsigned)samples), 256, 0, st>>>(u, known, mask, g, partial, per_sample);
+  int rc = check_launch("dc_mask_kernel");
+  if (rc) return rc;
+  dc_norm_kernel<<<(unsigned)samples, 256, 0, st>>>(partial, kDcMaskBlocks, gg);
+  return check_launch("dc_norm_kernel");
+}
+
+static int guided_dims(const char* who, const void* eps, int ldc, int channels, int samples,
+                       int64_t per_sample) {
+  if (samples < 1 || per_sample < 1) return set_error(-2, who);
+  if (eps == nullptr) return set_error(-2, who);
+  if (ldc != 0 && (channels < 1 || per_sample % channels != 0 || ldc < channels)) return set_error(-2, who);
+  return device_props();
+}
+
+extern "C" int mri_guided_x0(const float* z, const void* eps, int eps_nhwc_ldc, int channels,
+                             const int64_t* t, const float* sqrt_ac, const float* sqrt_1mac,
+                             const float* inv_s, float* out, int samples, int64_t per_sample,
+                             void* stream) {
+  int rc = guided_dims("mri_guided_x0: empty input, null eps or per_sample not channels * spatial, ldc >= channels",
+                       eps, eps_nhwc_ldc, channels, samples, per_sample);
+  if (rc) return rc;
+  if (z == nullptr || t == nullptr || sqrt_ac == nullptr || sqrt_1mac == nullptr || inv_s == nullptr || out == nullptr)
+    return set_error(-2, "mri_guided_x0: null z / t / schedule table / inv_s / out");
+  const long long numel = (long long)samples * per_sample;
+  guided_x0_kernel<<<my_blocks(aten_grid(numel)), 256, 0, (cudaStream_t)stream>>>(
+      z, eps, eps_nhwc_ldc, channels, t, sqrt_ac, sqrt_1mac, inv_s, out, per_sample, numel);
+  return check_launch("guided_x0_kernel");
+}
+
+extern "C" int mri_guided_eps(const void* eps, int eps_nhwc_ldc, int channels, const float* dz,
+                              const float* gg, const float* lam, const float* inv_s, const int64_t* t,
+                              const float* sqrt_ac, const float* sqrt_1mac, float* out, int samples,
+                              int64_t per_sample, void* stream) {
+  int rc = guided_dims("mri_guided_eps: empty input, null eps or per_sample not channels * spatial, ldc >= channels",
+                       eps, eps_nhwc_ldc, channels, samples, per_sample);
+  if (rc) return rc;
+  if (dz == nullptr || gg == nullptr || lam == nullptr || inv_s == nullptr || t == nullptr ||
+      sqrt_ac == nullptr || sqrt_1mac == nullptr || out == nullptr)
+    return set_error(-2, "mri_guided_eps: null dz / gg / lam / inv_s / t / schedule table / out");
+  const long long numel = (long long)samples * per_sample;
+  guided_eps_kernel<<<my_blocks(aten_grid(numel)), 256, 0, (cudaStream_t)stream>>>(
+      eps, eps_nhwc_ldc, channels, dz, gg, lam, inv_s, t, sqrt_ac, sqrt_1mac, out, per_sample, numel);
+  return check_launch("guided_eps_kernel");
 }
 
 extern "C" int mri_repaint_undo(float* x, const float* noise, const uint64_t* rng, uint64_t rng_skip,

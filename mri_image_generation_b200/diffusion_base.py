@@ -8,6 +8,9 @@ model arguments (z_pos, context) and the loss; everything that touches the GPU i
     inpainting (not in the reference): mri_inpaint_merge after each update of either sampler;
     undersampled k-space reconstruction (not in the reference): mri_kspace_merge in the same slot;
     RePaint's resampling (not in the reference): mri_repaint_undo between the inpainting steps;
+    measurement-guided sampling of the 3D LDM (not in the reference): mri_guided_x0, the VAE
+    decoder forward, mri_dc_project3d / mri_dc_mask, the decoder's input gradient and
+    mri_guided_eps before each unfused update;
     the variational bound in bits per dimension (not in the reference): mri_vb_terms after each
     evaluation step, on a step graph of its own;
   - the reverse loop: when the denoiser is one of this package's UNets, one CUDA graph holds a
@@ -38,16 +41,17 @@ def _require_cuda(x: torch.Tensor, what: str) -> None:
                             "this framework has no CPU fallback")
 
 
-def kspace_completion(y: torch.Tensor, m: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+def kspace_completion(y: torch.Tensor, m: torch.Tensor,
+                      dims: Tuple[int, ...] = (-2, -1)) -> Tuple[torch.Tensor, torch.Tensor]:
     """Hermitian completion of a measured k-space, on y's device: (x_zf, M) with M = m | m(-k),
-    y(k) = conj(y(-k)) where k is measured only at its mirror, and x_zf = Re ifft2(M y) in fp64
-    (orthonormal, unshifted).  y: complex (..., H, W); m: bool of y's shape.  Values of y outside
-    m are never read."""
-    mir = lambda a: torch.roll(torch.flip(a, (-2, -1)), (1, 1), (-2, -1))   # a(-k)
+    y(k) = conj(y(-k)) where k is measured only at its mirror, and x_zf = Re ifftn(M y) over `dims`
+    in fp64 (orthonormal, unshifted).  y: complex (..., H, W), or (..., D, H, W) with
+    dims = (-3, -2, -1); m: bool of y's shape.  Values of y outside m are never read."""
+    mir = lambda a: torch.roll(torch.flip(a, dims), (1,) * len(dims), dims)   # a(-k)
     full = m | mir(m)
     y = y.to(torch.complex128)
     y = torch.where(m, y, torch.where(full, mir(y).conj(), torch.zeros_like(y)))
-    return torch.fft.ifft2(y, norm="ortho").real, full
+    return torch.fft.ifftn(y, dim=dims, norm="ortho").real, full
 
 
 class _LossFn(torch.autograd.Function):
@@ -367,9 +371,100 @@ class DiffusionBase(nn.Module):
                         k=torch.zeros(1, dtype=torch.int64, device=dev),
                         x0_prev=torch.zeros_like(prog.x_in))
             prog.__dict__["_dpmpp_bufs"] = bufs
-            for key in ("dpmpp", "dpmpp+inpaint", "dpmpp+kspace"):   # captured on the old buffers
-                prog.__dict__.get("_step_graphs", {}).pop(key, None)
+            graphs = prog.__dict__.get("_step_graphs", {})
+            for key in [k for k in graphs if k.startswith("dpmpp")]:   # captured on the old buffers
+                graphs.pop(key)
         return bufs
+
+    # ------------------------------------------------------------------ measurement-guided sampling
+    def _guided_buffers(self, owner, dec, kspace: bool) -> Dict[str, torch.Tensor]:
+        """The guided step's state on `owner` (the UNet program, or a dict for the eager loop): the
+        data-gradient-only decoder program `dec` and the buffers the step reads through device
+        pointers -- zf (x_zf, or x_known for the image mask), mask, lam and inv_s (copied into on
+        every call, so one captured graph serves every measurement), gg, the data term's work and
+        eps (the guided eps, fp32 in the latent's layout).  A new decoder program drops the guided
+        graphs captured on the old one."""
+        d = owner if isinstance(owner, dict) else owner.__dict__
+        bufs = d.setdefault("_guided_bufs", {})
+        if bufs.get("dec") is not dec:
+            bufs.clear()
+            graphs = d.get("_step_graphs", {})
+            for key in [k for k in graphs if "+guided" in k]:
+                graphs.pop(key)
+            dev, B = dec.device, dec.B
+            img = dec.out
+            bufs.update(dec=dec, zf=torch.zeros_like(img), mask=torch.zeros(img.shape, dtype=torch.uint8, device=dev),
+                        gg=torch.zeros(B, dtype=torch.float32, device=dev),
+                        lam=torch.zeros(1, dtype=torch.float32, device=dev),
+                        inv_s=torch.ones(1, dtype=torch.float32, device=dev),
+                        eps=torch.zeros_like(dec.x_in))
+        key = "work_k" if kspace else "work_m"
+        if key not in bufs:
+            img = dec.out
+            n = ops.kspace3d_work_bytes(*img.shape) if kspace else img.shape[0] * ops.DC_MASK_WORK_PER_SAMPLE
+            bufs[key] = torch.zeros(n, dtype=torch.uint8, device=img.device)
+        bufs["work"], bufs["kspace"] = bufs[key], kspace
+        return bufs
+
+    def _guided_stage(self, z, eps, ldc: int, C: int, t, b) -> None:
+        """Steps 2-7 of the guided step (DESIGN.md §4) up to the guided eps, written to b['eps']:
+        x0 / s into the decoder's input, u = D(x0 / s), g and ||g||^2 of the data term into the
+        decoder's output gradient, dz = D^T g, then eps' = eps - (sac / s1m) * delta."""
+        dec = b["dec"]
+        sa, s1m = self.sqrt_alphas_cumprod, self.sqrt_one_minus_alphas_cumprod
+        ops.guided_x0(z, eps, t, sa, s1m, b["inv_s"], dec.x_in, eps_nhwc_ldc=ldc, channels=C)
+        dec.run()
+        dec.finish_output()
+        if b["kspace"]:
+            ops.dc_project3d(dec.out, b["zf"], b["mask"], dec.dout_in, b["gg"], b["work"])
+        else:
+            ops.dc_mask(dec.out, b["zf"], b["mask"], dec.dout_in, b["gg"], b["work"])
+        dec.run_input_backward()
+        ops.guided_eps(eps, dec.dz_out, b["gg"], b["lam"], b["inv_s"], t, sa, s1m, b["eps"],
+                       eps_nhwc_ldc=ldc, channels=C)
+
+    def _guided_sample(self, img, table, prog, eps_fn: Callable, dec, data, kspace: bool,
+                       lam: float, inv_s: float) -> torch.Tensor:
+        """Measurement-guided sampling from the latent x_T = img: DDPM over every timestep (table
+        None) or DPM-Solver++ over `table`, with the guided eps of _guided_stage in every update.
+        data: (zf, mask) on the image grid; dec: the VAE's data-gradient-only decoder program.
+        prog: the UNet program (step graphs 'ddpm+guided:kspace' etc.) or None: eager with
+        eps = eps_fn(x, t).  Draws what sample() / sample_dpmpp() draw.  Returns the latent z_0."""
+        _require_cuda(img, "guided sampling")
+        if dec.params_changed():
+            dec.do_refresh()
+        b = self._guided_buffers(prog if prog is not None else self.__dict__.setdefault("_guided_eager", {}),
+                                 dec, kspace)
+        b["zf"].copy_(data[0])
+        b["mask"].copy_(data[1])
+        b["lam"].fill_(lam)
+        b["inv_s"].fill_(inv_s)
+        mode = "ddpm" if table is None else "dpmpp"
+        T = self.timesteps
+        if prog is not None:
+            if table is None:
+                return self._reverse_loop(prog, img.float(), T - 1, T, mode, guided=b)
+            return self._reverse_loop(prog, img.float(), int(table[0][0]), table[0].numel(), mode,
+                                      table=table, guided=b)
+        dev = img.device
+        x = img.float().contiguous().clone()
+        with torch.cuda.device(dev):
+            if table is None:
+                for i in reversed(range(T)):
+                    t = torch.full((x.shape[0],), i, device=dev, dtype=torch.long)
+                    eps = eps_fn(x, t).float().contiguous()
+                    self._guided_stage(x, eps, 0, 0, t, b)
+                    x = self._p_update(x, t, b["eps"])
+                return x
+            ts, coef = table
+            coef = coef.to(dev)
+            x0_prev = torch.empty_like(x)
+            for i, t in enumerate(ts.tolist()):
+                tt = torch.full((x.shape[0],), t, device=dev, dtype=torch.long)
+                eps = eps_fn(x, tt).float().contiguous()
+                self._guided_stage(x, eps, 0, 0, tt, b)
+                ops.dpmpp_step(x, b["eps"], x0_prev, coef[i], None, x)
+        return x
 
     # ------------------------------------------------------------------ variational bound
     def _vb_input(self, x_start, rank: int) -> torch.Tensor:
@@ -506,7 +601,7 @@ class DiffusionBase(nn.Module):
     def _reverse_loop(self, prog, img: torch.Tensor, start_t: int, n_steps: int, mode: str,
                       use_graph: bool = True, t_vec: Optional[torch.Tensor] = None,
                       stride: int = 1, table=None, inpaint=None, levels=None,
-                      kspace: bool = False) -> torch.Tensor:
+                      kspace: bool = False, guided=None) -> torch.Tensor:
         """Run n_steps reverse steps (i = start_t, start_t - stride, ...) on `prog` (a UNetProgram
         whose x_in is the sampler state).  mode: 'ddpm' | 'ddim' (t_prev = max(t - stride, 0)) |
         'dpmpp' (table = (ts, coef) of schedules.dpmpp_2m_table, n_steps = its rows).
@@ -516,14 +611,17 @@ class DiffusionBase(nn.Module):
         the same z, on 'ddpm+kspace' / 'dpmpp+kspace'.
         levels: RePaint's walk (schedules.repaint_levels), 'ddpm' with inpaint only: its n_steps
         reverse steps replay 'ddpm+inpaint', its undo steps a graph of their own
-        ('repaint-undo': mri_repaint_undo at t, then t += 1), in the walk's order."""
+        ('repaint-undo': mri_repaint_undo at t, then t += 1), in the walk's order.
+        guided: the buffers of _guided_buffers, 'ddpm' or 'dpmpp' only: the unfused step with the
+        guided eps of _guided_stage in the update, on 'ddpm+guided:kspace' / 'dpmpp+guided:mask'
+        etc."""
         dev = img.device
         with torch.cuda.device(dev):
             return self._reverse_loop_on(prog, img, start_t, n_steps, mode, use_graph, t_vec, stride,
-                                         table, inpaint, levels, kspace)
+                                         table, inpaint, levels, kspace, guided)
 
     def _reverse_loop_on(self, prog, img, start_t, n_steps, mode, use_graph, t_vec, stride,
-                         table=None, inpaint=None, levels=None, kspace=False):
+                         table=None, inpaint=None, levels=None, kspace=False, guided=None):
         dev = img.device
         if prog.params_changed():
             prog.do_refresh()
@@ -545,11 +643,16 @@ class DiffusionBase(nn.Module):
             gkey += "+kspace" if kspace else "+inpaint"
         if levels is not None and (inp is None or mode != "ddpm" or kspace):
             raise _lib.MriError("RePaint resampling runs on the DDPM inpainting loop")
+        if guided is not None:
+            if mode not in ("ddpm", "dpmpp") or stride != 1 or t_vec is not None or inp is not None:
+                raise _lib.MriError("guided sampling runs on the full DDPM or the DPM-Solver++ loop")
+            gkey += "+guided:" + ("kspace" if guided["kspace"] else "mask")
         # DDPM inpainting draws a second randn_like(x) per step (the merge's noise)
         adv = 2 * inc if inp is not None else inc
 
+        # the guided step needs eps in HBM: it runs unfused
         fused = (getattr(prog, "fused_head", None) is not None and not prog.training
-                 and os.environ.get("MRI_FUSED_STEP", "1") != "0")
+                 and os.environ.get("MRI_FUSED_STEP", "1") != "0" and guided is None)
         if mode == "dpmpp":
             # the graph reads its row of the table through the device index k: it bakes in no
             # timestep, so changing num_steps or start_t only rewrites the table
@@ -584,16 +687,20 @@ class DiffusionBase(nn.Module):
                     ops.step_advance(prog.t_in, -stride, t_prev=tprev)
                 return
             prog.run()
+            eps, e_ldc, e_c = prog.eps_nhwc, ldc, C
+            if guided is not None:
+                self._guided_stage(prog.x_in, eps, ldc, C, prog.t_in, guided)
+                eps, e_ldc, e_c = guided["eps"], 0, 0
             if mode == "ddpm":
-                ops.ddpm_step_rng(prog.x_in, prog.eps_nhwc, rng, prog.t_in, self.betas,
+                ops.ddpm_step_rng(prog.x_in, eps, rng, prog.t_in, self.betas,
                                   self.sqrt_one_minus_alphas_cumprod, self.sqrt_recip_alphas,
-                                  self.posterior_variance, prog.x_in, eps_nhwc_ldc=ldc, channels=C)
+                                  self.posterior_variance, prog.x_in, eps_nhwc_ldc=e_ldc, channels=e_c)
                 if inp is not None:
                     merge()
                 ops.step_advance(prog.t_in, -1, rng=rng, rng_increment=adv)
             elif mode == "dpmpp":
-                ops.dpmpp_step(prog.x_in, prog.eps_nhwc, xp, dpm["coef"], kbuf, prog.x_in,
-                               eps_nhwc_ldc=ldc, channels=C)
+                ops.dpmpp_step(prog.x_in, eps, xp, dpm["coef"], kbuf, prog.x_in,
+                               eps_nhwc_ldc=e_ldc, channels=e_c)
                 ops.step_table_advance(prog.t_in, kbuf, dpm["ts"], rows)
                 if inp is not None:
                     merge()

@@ -4,10 +4,13 @@ Same constructor, buffers (names, order, bit-identical values), methods and sign
 arithmetic runs in fused sm_100a kernels and the reverse loop is a replayed CUDA graph when the
 denoiser is one of this package's UNets.
 """
+import math
+
 import torch
 
-from ... import ops, schedules
-from ...diffusion_base import DiffusionBase, _require_cuda
+from ... import _lib, ops, schedules
+from ...diffusion_base import DiffusionBase, _require_cuda, kspace_completion
+from .vae import VAE3D
 
 
 class GaussianDiffusionLatent3D(DiffusionBase):
@@ -164,8 +167,7 @@ class GaussianDiffusionLatent3D(DiffusionBase):
         (B, channels, D, H, W) latents; mask broadcasts to it, True / 1 = regenerate, False / 0 =
         keep.  x_T is drawn as sample() draws it; after the update at every step i the kept region
         is set to q_sample(x_known, i - 1, noise=randn_like(x)) (x_known itself after i = 0).  The
-        mask is at latent resolution: mapping an image-space mask to it (e.g. max-pooling by the
-        VAE's downsampling factor) is the caller's job.
+        mask is at latent resolution; for a mask at image resolution use inpaint_image().
 
         jump_n_sample > 1 adds RePaint's resampling: after the step at every multiple j of
         jump_length below T - jump_length, the state is re-noised jump_length steps
@@ -201,3 +203,102 @@ class GaussianDiffusionLatent3D(DiffusionBase):
         table = self._dpmpp_table(self.timesteps - 1, num_steps)
         img = self._randn(known.shape, self.betas.device)
         return self._dpmpp_from(img, table, cond, inpaint=(known.to(img.device), m.to(img.device)))
+
+    # ------------------------------------------------------------------ measurement-guided sampling
+    @torch.no_grad()
+    def reconstruct(self, kspace, kmask, vae, guidance_scale=1.0, latent_scale=1.0, cond=None):
+        """Undersampled 3-D k-space reconstruction through the VAE decoder (not in the reference;
+        DESIGN.md §4).  kspace: complex (B, C, D, H, W), torch.fft.fftn(x, dim=(-3, -2, -1),
+        norm="ortho") of the image x; kmask broadcasts to it, True / 1 = measured (e.g. a
+        phase-encode-plane mask (1, 1, D, H, 1), or one per modality with T1 / T2 fully sampled).
+        The latent is (B, channels, D/f, H/f, W/f) with f = 2^(vae.encoder.num_down - 1).
+
+        The full DDPM sampler, x_T drawn as sample() draws it.  At every step the clean estimate
+        x0 = (z_t - s1m eps) / sac is decoded, u = D(x0 / s), and moved by
+        delta = -guidance_scale * D^T g / (s ||g||), g = P u - x_zf with P u = Re F^-1(M F u)
+        (M the Hermitian completion of kmask, x_zf = Re F^-1(M y)); the update then uses the eps
+        that gives x0 + delta.  No gradient flows through the UNet (MPGD, He et al. ICLR 2024, with
+        DPS's step normalisation).  latent_scale s: the factor the LDM's training latents were
+        multiplied by, z_train = s * vae.encode_to_latent(x) (train.py:540-553).  Returns the fp32
+        image vae.decode_from_latent(z_0 / s), (B, C, D, H, W).  guidance_scale = 1.0 is untuned,
+        and the reconstruction quality on real volumes is unverified.
+
+        ValueError (before anything is drawn): bad shapes or mask, guidance_scale < 0 or not finite,
+        latent_scale <= 0.  MriError: vae not this package's VAE3D, 'split' precision of the VAE or
+        the UNet, CPU tensors, D, H or W over 512."""
+        return self._guided("kspace", kspace, kmask, vae, None, guidance_scale, latent_scale, cond)
+
+    @torch.no_grad()
+    def reconstruct_dpmpp(self, kspace, kmask, vae, num_steps=20, guidance_scale=1.0, latent_scale=1.0,
+                          cond=None):
+        """reconstruct() with DPM-Solver++(2M) in `num_steps` UNet calls (not in the reference): x_T
+        drawn as sample_dpmpp() draws it, the same guided eps in every solver update."""
+        return self._guided("kspace", kspace, kmask, vae, num_steps, guidance_scale, latent_scale, cond)
+
+    @torch.no_grad()
+    def inpaint_image(self, x_known, mask, vae, guidance_scale=1.0, latent_scale=1.0, cond=None):
+        """Inpainting with an image-space mask through the VAE decoder (not in the reference):
+        reconstruct() with the data term g = (1 - mask) (u - x_known).  x_known: (B, C, D, H, W)
+        image; mask broadcasts to it, True / 1 = regenerate, False / 0 = keep, at image resolution:
+        it can keep an acquired modality and regenerate a missing one inside the same latent
+        voxel.  Returns the fp32 image; the kept region is pulled toward x_known, not replaced."""
+        return self._guided("mask", x_known, mask, vae, None, guidance_scale, latent_scale, cond)
+
+    @torch.no_grad()
+    def inpaint_image_dpmpp(self, x_known, mask, vae, num_steps=20, guidance_scale=1.0, latent_scale=1.0,
+                            cond=None):
+        """inpaint_image() with DPM-Solver++(2M) in `num_steps` UNet calls (not in the reference)."""
+        return self._guided("mask", x_known, mask, vae, num_steps, guidance_scale, latent_scale, cond)
+
+    def _guided(self, kind, meas, mask, vae, num_steps, guidance_scale, latent_scale, cond):
+        lam, s = float(guidance_scale), float(latent_scale)
+        if not math.isfinite(lam) or lam < 0:
+            raise ValueError(f"guidance_scale must be finite and >= 0 (got {guidance_scale})")
+        if not math.isfinite(s) or s <= 0:
+            raise ValueError(f"latent_scale must be finite and > 0 (got {latent_scale})")
+        if not isinstance(vae, VAE3D):
+            raise _lib.MriError(f"vae must be this package's VAE3D (got {type(vae).__name__})")
+        name = "kspace" if kind == "kspace" else "x_known"
+        cout = vae.decoder.out_conv.weight.shape[0]
+        ok = torch.is_tensor(meas) and meas.dim() == 5 and meas.shape[1] == cout and meas.numel() > 0 \
+            and meas.is_complex() == (kind == "kspace")
+        if not ok:
+            got = (tuple(meas.shape), meas.dtype) if torch.is_tensor(meas) else type(meas)
+            want = "complex" if kind == "kspace" else "real"
+            raise ValueError(f"{name} must be a non-empty {want} (B, {cout}, D, H, W) tensor (got {got})")
+        if vae.decoder.from_latent.weight.shape[1] != self.channels:
+            raise ValueError(f"the VAE's latent has {vae.decoder.from_latent.weight.shape[1]} channels, "
+                             f"the diffusion model {self.channels}")
+        f = 2 ** (vae.encoder.num_down - 1)
+        if any(n % f for n in meas.shape[2:]):
+            raise ValueError(f"volume size {tuple(meas.shape[2:])} must be divisible by {f}")
+        m = torch.as_tensor(mask)
+        try:
+            ok = torch.broadcast_shapes(m.shape, meas.shape) == meas.shape
+        except RuntimeError:
+            ok = False
+        if not ok:
+            raise ValueError(f"mask of shape {tuple(m.shape)} does not broadcast to {name}'s {tuple(meas.shape)}")
+        if m.dtype != torch.bool and not bool(((m == 0) | (m == 1)).all()):
+            raise ValueError("mask must be bool or hold only 0 / 1")
+        table = self._dpmpp_table(self.timesteps - 1, num_steps) if num_steps is not None else None
+        _require_cuda(meas, "guided sampling")
+        ops.kspace3d_work_bytes(*meas.shape)      # MriError when D, H or W is over 512
+        eng = self._engine_model()
+        if vae.precision == "split" or getattr(eng if eng is not None else self.model, "precision", "bf16") == "split":
+            raise _lib.MriError("guided sampling runs in bf16 precision ('split' is not supported)")
+        dev = self.betas.device
+        B = meas.shape[0]
+        with torch.cuda.device(dev):
+            meas, m = meas.to(dev), m.to(dev).expand(meas.shape).bool()
+            if kind == "kspace":
+                zf, full = kspace_completion(meas, m, dims=(-3, -2, -1))
+                data = (zf.float().contiguous(), full.to(torch.uint8).contiguous())
+            else:
+                data = (meas.float().contiguous(), m.to(torch.uint8).contiguous())
+            lat = torch.empty(B, self.channels, *(n // f for n in meas.shape[2:]), device=dev)
+            dec = vae._program("decode", lat, training=True, wgrad=False)
+            img = self._randn(lat.shape, dev)
+            z0 = self._guided_sample(img, table, self._program_for(img, cond), self._eps_fn(cond), dec, data,
+                                     kind == "kspace", lam, 1.0 / s)
+            return vae.decode_from_latent(z0 / latent_scale)

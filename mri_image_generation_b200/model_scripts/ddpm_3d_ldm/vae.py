@@ -90,7 +90,10 @@ class VAE3D(EngineModule):
                                  enc_out_channels=self.encoder.out_channels, groups=groups)
 
     # ------------------------------------------------------------------ engine plumbing
-    def _program(self, mode: str, x: torch.Tensor, training: bool = False) -> VAE3DProgram:
+    def _program(self, mode: str, x: torch.Tensor, training: bool = False,
+                 wgrad: bool = True) -> VAE3DProgram:
+        """The cached engine program for (mode, shape).  training=True, wgrad=False: the training
+        program without parameter gradients (decoder input gradients for guided sampling)."""
         self._check_input(x)
         if x.dim() != 5:
             raise _lib.MriError(f"VAE3D expects (B, C, D, H, W), got {tuple(x.shape)}")
@@ -102,7 +105,10 @@ class VAE3D(EngineModule):
         if self.precision != "bf16":
             raise _lib.MriError(f"unknown precision {self.precision!r}: 'bf16' or 'split'")
         key = (mode, int(x.shape[0]), tuple(int(s) for s in x.shape[2:]), bool(training))
-        return self.get_program(key, lambda: VAE3DProgram(self, mode, key[1], key[2], training=key[3]))
+        if not wgrad:
+            key += ("dgrad",)
+        return self.get_program(key, lambda: VAE3DProgram(self, mode, key[1], key[2], training=key[3],
+                                                          wgrad=wgrad))
 
     def _run(self, mode: str, x: torch.Tensor, part: nn.Module) -> torch.Tensor:
         xf = x.float().contiguous()

@@ -301,6 +301,78 @@ def kspace_merge(x, x_zf, kmask, t, t_delta: int, sqrt_ac, sqrt_1mac, work=None,
                "mri_kspace_merge")
 
 
+def kspace3d_work_bytes(samples: int, channels: int, D: int, H: int, W: int) -> int:
+    """Bytes of dc_project3d's work buffer; MriError when D, H or W is over 512."""
+    import ctypes as C
+    out = C.c_size_t(0)
+    _lib.check(_lib.load().mri_kspace3d_work_bytes(int(samples), int(channels), int(D), int(H), int(W),
+                                                   C.byref(out)), "mri_kspace3d_work_bytes")
+    return int(out.value)
+
+
+def dc_project3d(u, x_zf, kmask, g, gg, work=None) -> None:
+    """k-space data term of guided sampling: g = Re ifftn(M fftn(u)) - x_zf over (D, H, W) in the
+    orthonormal convention and gg[n] = sum of g^2 over sample n.  u, x_zf, g: (B, C, D, H, W)
+    fp32; kmask: uint8, one byte per element, Hermitian-symmetric; gg: (B,) fp32.  work: a uint8
+    buffer of at least kspace3d_work_bytes (None: allocated here)."""
+    _chk_contig(u, x_zf, kmask, g, gg, work)
+    assert u.dim() == 5 and u.dtype == x_zf.dtype == g.dtype == gg.dtype == torch.float32
+    assert kmask.dtype == torch.uint8 and x_zf.numel() == kmask.numel() == g.numel() == u.numel()
+    B, C, D, H, W = u.shape
+    assert gg.numel() == B
+    if work is None:
+        work = torch.empty(kspace3d_work_bytes(B, C, D, H, W), dtype=torch.uint8, device=u.device)
+    _lib.check(_lib.load().mri_dc_project3d(_p(u), _p(x_zf), _p(kmask), _p(g), _p(gg), _p(work),
+                                            work.numel() * work.element_size(), B, C, D, H, W, _s()),
+               "mri_dc_project3d")
+
+
+DC_MASK_WORK_PER_SAMPLE = 1024
+
+
+def dc_mask(u, known, mask, g, gg, work=None) -> None:
+    """Image-space data term of guided sampling: g = where(mask, 0, u - known) and gg[n] = sum of
+    g^2 over sample n.  mask: uint8, one byte per element (1 = regenerate, 0 = keep).  work: a
+    buffer of at least DC_MASK_WORK_PER_SAMPLE bytes per sample (None: allocated here)."""
+    _chk_contig(u, known, mask, g, gg, work)
+    assert u.dtype == known.dtype == g.dtype == gg.dtype == torch.float32 and mask.dtype == torch.uint8
+    assert known.numel() == mask.numel() == g.numel() == u.numel()
+    B = u.shape[0]
+    assert gg.numel() == B
+    if work is None:
+        work = torch.empty(B * DC_MASK_WORK_PER_SAMPLE, dtype=torch.uint8, device=u.device)
+    _lib.check(_lib.load().mri_dc_mask(_p(u), _p(known), _p(mask), _p(g), _p(gg), _p(work),
+                                       work.numel() * work.element_size(), B, u.numel() // B, _s()),
+               "mri_dc_mask")
+
+
+def guided_x0(z, eps, t, sqrt_ac, sqrt_1mac, inv_s, out, eps_nhwc_ldc: int = 0, channels: int = 0) -> None:
+    """out = (z - sqrt_1mac[t] eps) / sqrt_ac[t] * inv_s per sample (fp32).  eps: fp32 in z's layout,
+    or the bf16 channels-last UNet output with eps_nhwc_ldc / channels; inv_s: a one-element fp32
+    device tensor."""
+    _chk_contig(z, eps, out)
+    assert z.dtype == out.dtype == inv_s.dtype == torch.float32 and out.numel() == z.numel()
+    assert t.dtype == torch.int64
+    n = z.shape[0]
+    _lib.check(_lib.load().mri_guided_x0(_p(z), _p(eps), eps_nhwc_ldc, channels, _p(t), _p(sqrt_ac),
+                                         _p(sqrt_1mac), _p(inv_s), _p(out), n, z.numel() // n, _s()),
+               "mri_guided_x0")
+
+
+def guided_eps(eps, dz, gg, lam, inv_s, t, sqrt_ac, sqrt_1mac, out, eps_nhwc_ldc: int = 0,
+               channels: int = 0) -> None:
+    """out = eps - (sqrt_ac[t] / sqrt_1mac[t]) * delta, delta = -(lam / sqrt(gg)) * dz * inv_s per
+    sample (out = eps where lam / sqrt(gg) is 0), fp32 in dz's layout.  lam, inv_s: one-element
+    fp32 device tensors; gg: (B,) fp32."""
+    _chk_contig(eps, dz, gg, out)
+    assert dz.dtype == gg.dtype == lam.dtype == inv_s.dtype == out.dtype == torch.float32
+    assert out.numel() == dz.numel() and t.dtype == torch.int64
+    n = out.shape[0]
+    _lib.check(_lib.load().mri_guided_eps(_p(eps), eps_nhwc_ldc, channels, _p(dz), _p(gg), _p(lam),
+                                          _p(inv_s), _p(t), _p(sqrt_ac), _p(sqrt_1mac), _p(out), n,
+                                          out.numel() // n, _s()), "mri_guided_eps")
+
+
 def repaint_undo(x, t, alphas, betas, noise=None, rng: Optional[DeviceRng] = None,
                  rng_skip: int = 0) -> None:
     """RePaint's undo step in place: x = sqrt(alphas[l + 1]) * x + sqrt(betas[l + 1]) * z with

@@ -57,14 +57,22 @@ class VAE3DProgram(UNetProgram):
     """mode 'encode': x (B, Cin, D, H, W) fp32 -> [mu | logvar] (B, 2*latent, d, h, w) fp32
     (Encoder3D.forward, vae.py:49-55);
     mode 'decode': z (B, latent, d, h, w) fp32 -> reconstruction (B, Cout, D, H, W) fp32
-    (Decoder3D.forward, vae.py:82-87)."""
+    (Decoder3D.forward, vae.py:82-87).
 
-    def __init__(self, vae, mode: str, batch: int, spatial: Sequence[int], training: bool = False):
+    wgrad=False (training programs only): the backward computes data gradients alone -- for the
+    decoder, dz_out = D^T dout without any parameter gradient, as measurement-guided sampling needs
+    (diffusion_base._guided_loop).  Its forward and dz_out are the training program's, bit for bit."""
+
+    def __init__(self, vae, mode: str, batch: int, spatial: Sequence[int], training: bool = False,
+                 wgrad: bool = True):
         dev = next(vae.parameters()).device
         enc, dec = vae.encoder, vae.decoder
         first_block = enc.downs[0] if mode == "encode" else dec.ups[0]
         self.gn_groups = first_block.norm1.num_groups
         super().__init__(dev, batch, spatial, groups=self.gn_groups, training=training)
+        if not wgrad and not training:
+            raise _lib.MriError("VAE3DProgram: wgrad=False applies to training programs")
+        self.wgrad = wgrad
         self.dz_out: Optional[torch.Tensor] = None
         self.mode = mode
         if len(self.sp) != 3:
@@ -351,11 +359,22 @@ class VAE3DProgram(UNetProgram):
             S = self.sp[0] * self.sp[1] * self.sp[2]
             ops.nhwc_to_nchw(self.dz64, self.dz_out, self.B, S, self.dz_out.shape[1], 64)
 
+    def finish_output(self) -> None:
+        """self.out (fp32 NCDHW) from the last run()'s channels-last output."""
+        S = self.sp_out[0] * self.sp_out[1] * self.sp_out[2]
+        ops.nhwc_to_nchw(self.eps_nhwc, self.out, self.B, S, self.cout, self.cout_pad)
+
+    def run_input_backward(self) -> None:
+        """The backward launches on what dout_in holds, enqueued without a graph of their own (a
+        caller's step graph captures them): dz_out = D^T dout_in after the last run()."""
+        self._bwd_head(self.sp_out[0] * self.sp_out[1] * self.sp_out[2])
+        self.run_backward()
+        self._bwd_tail()
+
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         if self.params_changed():
             self.do_refresh()
         self.x_in.copy_(x)
         self.run()
-        S = self.sp_out[0] * self.sp_out[1] * self.sp_out[2]
-        ops.nhwc_to_nchw(self.eps_nhwc, self.out, self.B, S, self.cout, self.cout_pad)
+        self.finish_output()
         return self.out
