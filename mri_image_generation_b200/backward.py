@@ -154,6 +154,7 @@ class BackwardMixin:
         self._g_last_op: Dict[int, int] = {}              # id(param) -> index of the last op of
         self._g_touched: List[int] = []                   # ... the last tape record touching it
         self.bwd_segments: List[Tuple[int, int, int, int]] = []  # (op_lo, op_hi, arena_lo, arena_hi)
+        self.bwd_ranges: List[Tuple[int, int]] = []   # ops [lo, hi) of each tape record, in tape order
         # deferred parameter-gradient finalisers: (op index, dst, src, idx or None, batch, ld);
         # all finalisers of a launch range run as ONE mri_grad_finalize launch at its end
         self._final: List[Tuple[int, torch.Tensor, torch.Tensor, Optional[torch.Tensor], int, int]] = []
@@ -568,6 +569,7 @@ class BackwardMixin:
         hn = r.hn
         self.emit_grad(hn, lambda out, add: self.bgemm(
             P.conv_plan([P.ConvSource(dqkv)], wqT, out, 1, residual=add, name=f"dgrad:{r.name}.qkv")))
+        r.dO, r.dP, r.dS, r.dqkv = dO, dP, dS, dqkv   # kept for stage-by-stage checks
 
     def bwd_time(self, r: TimeRec) -> None:
         B = self.B
@@ -609,6 +611,7 @@ class BackwardMixin:
         self.grads.update(dy_seed)
         for rec in reversed(self.tape):
             self._g_touched = []
+            lo = len(self.bwd_ops)
             if isinstance(rec, ConvRec):
                 self.bwd_conv(rec)
             elif isinstance(rec, GnRec):
@@ -624,6 +627,7 @@ class BackwardMixin:
             else:  # pragma: no cover
                 raise _lib.MriError(f"unknown tape record {type(rec)}")
             self._close_record()
+            self.bwd_ranges.insert(0, (lo, len(self.bwd_ops)))
         self.bwd_segments = []
 
     def _close_record(self) -> None:
